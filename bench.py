@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the PARESIS image-formation hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Metric (BASELINE.json): speckle image-sets/s.  One image-set = everything PARESIS's main.py
 produces for one membrane position (main.py:63-110): a fresh membrane thickness map, the
@@ -32,6 +32,10 @@ At N = 1 the line also carries `splat`: BASELINE.json's second figure, the stand
 
 `--impl reference` times the CPU oracle port of the same path (oracle/, fp64 numpy + C) on the
 host cores, one process per core, on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last job of the last timed step returned on rank 0
+(ImageFormation.compute_rt_positions: thickness, sample, reference, propag, white, sums) as DIR/<name>.npy, so that two
+builds run with the same arguments can be compared output for output (the inputs depend only on the arguments).
 """
 import argparse
 import json
@@ -64,6 +68,25 @@ ALG_BYTES = {
 }
 SLOTS = 5               # membrane positions in flight (same-box A/B: 3 -> 5 is +1.2 %, 6 no better)
 PER_LAUNCH = 0   # > 1: that many positions share each kernel launch (blockIdx.z) instead; measured no faster (DESIGN.md)
+
+
+DUMP_OUTPUTS = ("thickness", "sample", "reference", "propag", "white", "sums")
+DUMP_MAX_ELEMENTS = 1 << 22     # per output: 16 MiB of float32; the six outputs of a job stay under 64 MB in all
+
+
+def dump_outputs(directory, res, torch):
+    """Write each output of one compute_rt_positions call as <directory>/<name>.npy, float32 or float64 as computed.
+    An output of at most DUMP_MAX_ELEMENTS values is written whole, in its shape.  A larger one (the thickness maps and
+    the sample / reference images of 20 positions) is written as a 1-D sample of its flattened values: DUMP_MAX_ELEMENTS
+    indices drawn without replacement by numpy's default_rng(0), in increasing order -- the same indices on every run."""
+    os.makedirs(directory, exist_ok=True)
+    for name in DUMP_OUTPUTS:
+        t = res[name]
+        assert t.dtype in (torch.float32, torch.float64), (name, t.dtype)
+        if t.numel() > DUMP_MAX_ELEMENTS:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_MAX_ELEMENTS, replace=False))
+            t = t.reshape(-1).index_select(0, torch.as_tensor(idx, device=t.device))
+        np.save(os.path.join(directory, name + ".npy"), t.cpu().numpy())
 
 
 def config_dict(**extra):
@@ -190,9 +213,7 @@ def run_reference(args):
     import multiprocessing as mp
     cores = os.cpu_count() or 1
     workers = max(1, min(cores, 32))
-    per_step = workers                      # bounded sample: one position per worker per step
-    # a step of the CPU arm takes ~10-15 s: cap the run to a few minutes whatever K / W were asked for
-    args.steps, args.warmup = min(args.steps, 5), min(args.warmup, 1)
+    per_step = workers                      # bounded sample: one position per worker per step (a step takes ~10-15 s)
     with mp.get_context("fork").Pool(workers, initializer=_worker_init) as pool:
         for w in range(args.warmup):
             pool.map(_worker_run, [(1, 5000 + w * per_step + i) for i in range(per_step)])
@@ -322,9 +343,9 @@ def run_gpu(args):
         e0.record()
         for jb in range(jobs):                              # one probed position per step, in its first job
             if jb == 0:
-                device_job(s * jobs, dominant, k_events)
+                last = device_job(s * jobs, dominant, k_events)
             else:
-                device_job(s * jobs + jb)
+                last = device_job(s * jobs + jb)
         e1.record()
         step_events.append((e0, e1))
         if s % 8 == 7:
@@ -335,6 +356,8 @@ def run_gpu(args):
     launches = abi.launches - launches0
     dev_s = sum(a.elapsed_time(b) for a, b in step_events) * 1e-3
     eng.check_flag()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last, torch)
     k_ms = [a.elapsed_time(b) for a, b in k_events]
     t = torch.tensor([dev_s], device="cuda", dtype=torch.float64)
     if world > 1:
@@ -692,7 +715,12 @@ def main():
     ap.add_argument("--jobs-per-step", type=int, default=JOBS_PER_STEP, help="20-position jobs per timed step")
     ap.add_argument("--skip-extras", action="store_true", help="headline only: no splat / 8192^2 / energy-sharded sections")
     ap.add_argument("--per-launch", type=int, default=PER_LAUNCH, help="membrane positions per kernel launch (0: one launch per position, on --slots streams)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed job as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.steps < 1):
+        ap.error("--dump-outputs needs the GPU path (--impl b200) and at least one timed step")
+    if args.dump_outputs:
+        args.dump_outputs = os.path.abspath(args.dump_outputs)     # the run changes into a temporary workspace
     if args.impl == "reference":
         run_reference(args)
     else:

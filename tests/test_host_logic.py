@@ -69,21 +69,6 @@ def test_delta_beta_tables_match_reference_values(golden):
     assert tables.interpolate("CuSn", [1.0]) == [(0, 1)]      # below the table: Sample.py:124-128
 
 
-def test_biff8_reader_against_export(tmp_path):
-    """The BIFF8 reader is exercised on the reference workbook where it is mounted."""
-    xls = "/root/reference/CodePython/Samples/DeltaBeta/TablesDeltaBeta.xls"
-    if not os.path.exists(xls):
-        pytest.skip("reference data file not mounted")
-    from paresis_b200.hostio import biff8
-    sh = biff8.open_workbook(xls).sheets()[0]
-    names = {sh.cell(0, c).value: c for c in range(sh.ncols) if isinstance(sh.cell(0, c).value, str) and sh.cell(0, c).value}
-    assert {"CuSn", "PMMA", "Nylon", "Air", "CsI"} <= set(names)
-    c = names["Nylon"]
-    assert sh.cell(2, c).value == "Energy(eV)" and sh.cell(3, c).value == 5000.0
-    z = np.load(os.path.join(ROOT, "paresis_b200/CodePython/Samples/DeltaBeta/delta_beta_tables.npz"))
-    assert z["Nylon"][0, 0] == 5000.0 and z["Nylon"][0, 1] == sh.cell(3, c + 1).value
-
-
 def test_image_io_round_trip(tmp_path):
     from paresis_b200.hostio import imageio
     a = np.random.default_rng(0).random((37, 53)).astype(np.float32)
