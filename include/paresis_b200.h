@@ -202,6 +202,13 @@ int paresis_transmit_rt(const float* intensity_in, const double* phi_in,
                         const double* phase_host, int n_layers,
                         float* intensity_out, double* phi_out, size_t n, paresis_stream stream);
 
+/* out[k][p] = bias[k] + sum_m weights[k][m] * maps[m][p], k < n_out (1..2), m < n_maps (>= 1, no upper limit);
+ * fp64 accumulation, one rounding to fp32.  The per-energy phase / attenuation maps of a sample with more
+ * materials than a hop takes (Sample.py:279, :347-348).  weights_host is row-major [n_out][n_maps]; bias_host
+ * may be NULL (0).  n = pixels of every map. */
+int paresis_mix_maps(const float* const* maps_host, int n_maps, const double* weights_host, const double* bias_host,
+                     int n_out, float* const* out_host, size_t n, paresis_stream stream);
+
 /* Experiment.computeSampleAndReferenceImages_RT for one membrane position in ONE call
  * (Experiment.py:407-526).  The host prepares, per spectrum energy, the scalars of the three
  * refraction hops; the library runs the whole launch sequence on `stream`. */

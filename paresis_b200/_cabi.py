@@ -24,7 +24,7 @@ REFRACTION_MARGIN_V1 = 10  # refractionFileNumba.py:36
 
 EXPORTS = (
     "paresis_version", "paresis_last_error", "paresis_set_tuning", "paresis_trim", "paresis_splat", "paresis_refract_phi", "paresis_refract_layers",
-    "paresis_transmit_rt", "paresis_transmit_wave", "paresis_fresnel_plan_create", "paresis_fresnel_plan_destroy",
+    "paresis_transmit_rt", "paresis_transmit_wave", "paresis_mix_maps", "paresis_fresnel_plan_create", "paresis_fresnel_plan_destroy",
     "paresis_fresnel_plan_bytes", "paresis_fresnel_propagate", "paresis_fresnel_kernel_create", "paresis_fresnel_kernel_destroy",
     "paresis_fresnel_convolve", "paresis_fresnel_spectrum", "paresis_fresnel_from_spectrum", "paresis_detect_work_floats", "paresis_detect",
     "paresis_detect_counts", "paresis_detect_counts_multi",
@@ -127,6 +127,7 @@ def _load():
         "paresis_refract_layers": [vp, cf, ctypes.POINTER(Layer), ci, vp, vp, vp, vp, ci, ci, ci, vp, vp],
         "paresis_transmit_rt": [vp, vp, ctypes.POINTER(vp), ctypes.POINTER(cd), ctypes.POINTER(cd), ci, vp, vp, sz, vp],
         "paresis_transmit_wave": [vp, cf, ctypes.POINTER(vp), ctypes.POINTER(cd), ctypes.POINTER(cd), ci, vp, sz, vp],
+        "paresis_mix_maps": [ctypes.POINTER(vp), ci, ctypes.POINTER(cd), ctypes.POINTER(cd), ci, ctypes.POINTER(vp), sz, vp],
         "paresis_fresnel_plan_create": [ci, ci, ci, ctypes.POINTER(vp)],
         "paresis_fresnel_plan_destroy": [vp],
         "paresis_fresnel_propagate": [vp, vp, vp, vp, C32, vp, vp, vp],
@@ -393,20 +394,47 @@ def _layer_arrays(thickness, atten, phase):
     return n, tp, at, ph
 
 
+def _groups(n):
+    """Transmission is multiplicative: more than MAX_LAYERS materials are applied MAX_LAYERS at a time, each call after the
+    first working in place on the outputs of the one before (Sample.py:279, :347-348 loop over any number of materials)."""
+    return [slice(g, g + MAX_LAYERS) for g in range(0, max(n, 1), MAX_LAYERS)]
+
+
 def transmit_rt(intensity_in, phi_in, thickness, atten, phase, intensity_out, phi_out):
-    n, tp, at, ph = _layer_arrays(thickness, atten, phase)
     count = (intensity_out if intensity_out is not None else phi_out).numel()
-    _check(lib.paresis_transmit_rt(_ptr(intensity_in, torch.float32), _ptr(phi_in, torch.float64), tp, at, ph, n,
-                                   _ptr(intensity_out, torch.float32), _ptr(phi_out, torch.float64), count, _stream()),
-           "paresis_transmit_rt")
-    _count()
+    for k, sl in enumerate(_groups(len(thickness))):
+        n, tp, at, ph = _layer_arrays(thickness[sl], atten[sl], phase[sl])
+        i_in, p_in = (intensity_in, phi_in) if k == 0 else (intensity_out, phi_out)
+        _check(lib.paresis_transmit_rt(_ptr(i_in, torch.float32), _ptr(p_in, torch.float64), tp, at, ph, n,
+                                       _ptr(intensity_out, torch.float32), _ptr(phi_out, torch.float64), count, _stream()),
+               "paresis_transmit_rt")
+        _count()
 
 
 def transmit_wave(wave_in, amplitude_uniform, thickness, atten, phase, wave_out):
-    n, tp, at, ph = _layer_arrays(thickness, atten, phase)
-    _check(lib.paresis_transmit_wave(_ptr(wave_in, torch.complex64), float(amplitude_uniform), tp, at, ph, n,
-                                     _ptr(wave_out, torch.complex64), wave_out.numel(), _stream()),
-           "paresis_transmit_wave")
+    for k, sl in enumerate(_groups(len(thickness))):
+        n, tp, at, ph = _layer_arrays(thickness[sl], atten[sl], phase[sl])
+        w_in = wave_in if k == 0 else wave_out
+        _check(lib.paresis_transmit_wave(_ptr(w_in, torch.complex64), float(amplitude_uniform), tp, at, ph, n,
+                                         _ptr(wave_out, torch.complex64), wave_out.numel(), _stream()),
+               "paresis_transmit_wave")
+        _count()
+
+
+def mix_maps(maps, weights, bias, outs):
+    """paresis_mix_maps: outs[k] = bias[k] + sum_m weights[k][m] * maps[m] (fp64 accumulation, one fp32 rounding).
+    ``weights``: n_out rows of len(maps) values; ``bias``: n_out values or None (0)."""
+    n_out, n_maps = len(outs), len(maps)
+    for t in list(maps) + list(outs):
+        _ptr(t, torch.float32)
+    mp = (ctypes.c_void_p * max(n_maps, 1))(*[t.data_ptr() for t in maps])
+    op = (ctypes.c_void_p * max(n_out, 1))(*[t.data_ptr() for t in outs])
+    w = (ctypes.c_double * max(n_out * n_maps, 1))(*[float(v) for row in weights for v in row])
+    b = (ctypes.c_double * n_out)(*[float(v) for v in bias]) if bias is not None else None
+    count = outs[0].numel() if outs else 0
+    if any(t.numel() != count for t in list(maps) + list(outs)):
+        raise ParesisError("paresis_mix_maps: every map and output must have %d pixels" % count)
+    _check(lib.paresis_mix_maps(mp, n_maps, w, b, n_out, op, count, _stream()), "paresis_mix_maps")
     _count()
 
 

@@ -117,6 +117,7 @@ def compute_rt(exp, point_num):
     to_px = s.d3 / (s.study_pixel_um * 1e-6 * s.magnification)
     sums, energies, ibin, white = [], [], 0, 0.0
     fwhm = s.effective_source_fwhm()
+    fits = eng.sample_fits(s, with_membrane=True)
     for ie, (energy, flux) in enumerate(s.spectrum):
         print("Current Energy: %gkev" % energy)
         k = hm.wavenumber(energy * 1000)
@@ -125,7 +126,7 @@ def compute_rt(exp, point_num):
         mem_maps, mem_ub, _ = eng._split(s.membrane, energy)
         smp_maps, _, _ = eng._split(s.sample, energy)
         # sample layers: the scattering material's thickness counts with its volume fraction; its angle map in pixels
-        smp_layers, have_df = [], False
+        smp_layers, fractions, have_df = [], [], False
         for imat, (t, d, b) in enumerate(smp_maps):
             model = model_of(smp, imat)
             fraction = 1.0
@@ -134,8 +135,12 @@ def compute_rt(exp, point_num):
                 abi.df_angle(t, coeff * to_px, df_px)
                 have_df = True
             smp_layers.append((t, d * fraction, b * fraction))
+            fractions.append(fraction)
         if not have_df:
             df_px.zero_()
+        if not fits:
+            # more materials than a hop takes: the hops see the two mixed maps, the angle map stays the material's own
+            smp_layers = eng.mixed_sample(s.sample, energy, fractions)
         # membrane -> object plane (Experiment.py:463-466)
         eng.i_bs.zero_()
         abi.refract_layers(None, i0 * np.exp(-2 * k * mem_ub) * plate, [(t, d * g2, 0.0, 2 * k * b) for t, d, b in mem_maps],

@@ -48,7 +48,8 @@ class Scene:
     """Everything the per-energy loop reads (products of Experiment.__init__, Experiment.py:81-100).
 
     ``membrane`` may mix mapped and uniform layers (the support plate is uniform: it only
-    attenuates); ``sample`` layers must all be maps."""
+    attenuates).  ``sample`` may hold any number of mapped and uniform layers: when they do not fit
+    a hop, they reach it as two mixed maps per energy (ImageFormation.mixed_sample)."""
 
     def __init__(self, study_dims, study_pixel_um, oversampling, det_dims, det_pixel_um, psf_sigma,
                  d_source_membrane, d_membrane_object, d_object_detector, mean_shot_count,
@@ -123,6 +124,8 @@ class ImageFormation:
         self._plan = None
         self._vectors = {}
         self._waves = None
+        self._mixed = {}         # (material maps, weights) -> the mixed maps of one energy (mixed_sample)
+        self._mixed_of = None    # the material maps the cached mixed maps were made from
 
     # ------------------------------------------------------------------ helpers
     def _gauss(self, sigma):
@@ -159,6 +162,70 @@ class ImageFormation:
                 ub += b * L.uniform
                 ud += d * L.uniform
         return maps, ub, ud
+
+    # ------------------------------------------------------------------ samples with many materials
+    @staticmethod
+    def sample_fits(scene, with_membrane):
+        """Whether the sample's layers go to the hops as they are: all mapped, and at most MAX_LAYERS maps per hop
+        (``with_membrane``: the membrane maps share the hop, as in ray tracing)."""
+        if any(L.map is None for L in scene.sample):
+            return False
+        used = len(scene.sample) + (sum(L.map is not None for L in scene.membrane) if with_membrane else 0)
+        return used <= abi.MAX_LAYERS
+
+    def mixed_sample(self, layers, energy, fractions=None):
+        """The sample at ``energy`` as two layers [(P, delta*, 0), (B, 0, beta*)] (DESIGN.md, "Samples of any number
+        of materials"): P = sum_m (delta_m / delta*) t_m, B = sum_m (beta_m / beta*) t_m + (sum of uniform beta t) / beta*,
+        delta* / beta* the largest coefficients of that energy.  Everything a hop does with the sample is linear in
+        thickness, so these two maps stand for all of them; a uniform layer's constant phase has no gradient and is a
+        global phase of a wave, so uniform layers only enter B.  ``fractions``: per-layer factors on the thickness (the
+        volume fraction of a dark-field material, Sample.py:333, :344).
+
+        The maps depend on (sample, energy) only: they are made once and kept while the sample's maps stay the same."""
+        fractions = fractions if fractions is not None else [1.0] * len(layers)
+        maps, d, b, uniform, bias = [], [], [], [], 0.0
+        for L, f in zip(layers, fractions):
+            dl, bl = L.delta.get(energy, 0.0) * f, L.beta.get(energy, 0.0) * f   # a missing energy leaves 0 (Sample.py:303-319)
+            if L.map is None:
+                uniform.append(bl)
+                bias += bl * L.uniform
+            else:
+                maps.append(L.map)
+                d.append(dl)
+                b.append(bl)
+        if not maps and not uniform:
+            raise NotImplementedError("the sample has no layer")
+        d_star = max((abs(v) for v in d), default=0.0) or 1.0
+        b_star = max((abs(v) for v in b + uniform), default=0.0) or 1.0
+        w_p, w_b, bias_b = [v / d_star for v in d], [v / b_star for v in b], bias / b_star
+        source = tuple(t.data_ptr() for t in maps)
+        if source != self._mixed_of:
+            self._mixed.clear()
+            self._mixed_of = source
+        key = (tuple(w_p), tuple(w_b), bias_b)
+        if key not in self._mixed:
+            try:
+                p_map = torch.empty((self.nx, self.ny), device=self.device, dtype=torch.float32)
+                b_map = torch.empty_like(p_map)
+            except torch.cuda.OutOfMemoryError as exc:
+                raise MemoryError("a sample of %d materials needs %d bytes of device memory per energy for its mixed "
+                                  "phase and attenuation maps (2 x %d x %d float32); %d energies are held already"
+                                  % (len(layers), 8 * self.nx * self.ny, self.nx, self.ny, len(self._mixed))) from exc
+            if maps:
+                abi.mix_maps(maps, [w_p, w_b], [0.0, bias_b], [p_map, b_map])
+            else:
+                abi.fill(p_map, 0.0)
+                abi.fill(b_map, bias_b)
+            # the material maps are held with their mix: their addresses identify it
+            self._mixed[key] = (p_map, b_map, tuple(maps))
+        p_map, b_map, _ = self._mixed[key]
+        return [(p_map, d_star, 0.0), (b_map, 0.0, b_star)]
+
+    def _sample_layers(self, scene, energy, fits):
+        """-> [(map, delta, beta)] the hops take for the sample at ``energy``."""
+        if fits:
+            return self._split(scene.sample, energy)[0]
+        return self.mixed_sample(scene.sample, energy)
 
     def _new_outputs(self, nbins, first):
         """Detector images of one position, stacked [image][bin][x][y] in ONE device buffer
@@ -204,15 +271,16 @@ class ImageFormation:
         g3 = hm.refraction_gradient_scale(s.d3, s.magnification, s.study_pixel_um)
         energies = (abi.RtEnergy * len(indices))()
         keep = []
+        fits = self.sample_fits(s, with_membrane=True)
         for slot, ie in enumerate(indices):
             energy, flux = s.spectrum[ie]
             k = hm.wavenumber(energy * 1000)
             i0 = s.mean_shot_count / s.os ** 2 * flux * s.common_factor(energy)      # :438, :451-459
             plate = s.plate_factor(energy)
             mem_maps, mem_ub, _ = self._split(s.membrane, energy)
-            smp_maps, smp_ub, _ = self._split(s.sample, energy)
-            if smp_ub != 0.0 or not mem_maps or not smp_maps or len(mem_maps) + len(smp_maps) > abi.MAX_LAYERS:
-                raise NotImplementedError("scene needs 1+ membrane maps, sample maps only, at most %d maps per hop"
+            smp_maps = self._sample_layers(s, energy, fits)
+            if not mem_maps or not smp_maps or len(mem_maps) + len(smp_maps) > abi.MAX_LAYERS:
+                raise NotImplementedError("scene needs 1+ membrane maps and a sample, at most %d maps per hop"
                                           % abi.MAX_LAYERS)
             en = energies[slot]
             # uniform layers and the plate only scale the beam (:463, :478-480)
@@ -482,15 +550,16 @@ class ImageFormation:
         w_a, w_b = self._waves
         mag_mem_obj = (s.d1 + s.d2) / s.d1                                            # :340
         ibin, white_sum, bin_starts = 0, 0.0, {0}
+        fits = self.sample_fits(s, with_membrane=False)
         for ie, (energy, flux) in enumerate(s.spectrum):
             k = hm.wavenumber(energy * 1000)
             i0 = s.mean_shot_count / s.os ** 2 * flux * s.common_factor(energy)       # :308, :320-333
             plate = s.plate_factor(energy)
             amp = float(np.sqrt(i0 * plate))   # the plate scales every intensity linearly (:352-356)
             mem_maps, mem_ub, _ = self._split(s.membrane, energy)
-            smp_maps, smp_ub, _ = self._split(s.sample, energy)
-            if smp_ub != 0.0 or not mem_maps or not smp_maps:
-                raise NotImplementedError("scene needs 1+ membrane maps and sample maps only")
+            smp_maps = self._sample_layers(s, energy, fits)
+            if not mem_maps or not smp_maps:
+                raise NotImplementedError("scene needs 1+ membrane maps and a sample")
             # after the membrane (:338); uniform layers: attenuation folded in, constant phase dropped
             abi.transmit_wave(None, amp * np.exp(-k * mem_ub), [t for t, _, _ in mem_maps],
                               [k * b for _, _, b in mem_maps], [k * d for _, d, _ in mem_maps], w_a)

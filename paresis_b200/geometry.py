@@ -29,6 +29,7 @@ class DeviceGeometry:
         self.map_shape = (int(shape[0]), int(shape[1]))
         self._pending = {}
         self._host = {}
+        self._full = {}       # materialised uniform entries: the same tensor every call (engine.mixed_sample keys on it)
 
     def prefetch(self, m=0):
         """Start copying map ``m`` to pinned host memory; overlaps whatever the GPU does next."""
@@ -57,9 +58,12 @@ class DeviceGeometry:
 
     def device_entries(self, materialise=False):
         out = []
-        for e in self.entries:
+        for m, e in enumerate(self.entries):
             if materialise and not isinstance(e, torch.Tensor):
-                e = torch.full(self.map_shape, float(e), device=device(), dtype=torch.float32)
+                key = (m, str(device()))
+                if key not in self._full:
+                    self._full[key] = torch.full(self.map_shape, float(e), device=device(), dtype=torch.float32)
+                e = self._full[key]
             out.append(e)
         return out
 
