@@ -537,11 +537,14 @@ def detect_counts(image, oversampling, det_x, det_y, src_kernel, psf_kernel, wor
 
 
 def detect_counts_multi(images, oversampling, det_x, det_y, src_kernel, psf_kernel, work, outs, noise, seed, sequences):
-    """Up to 4 images of one detector in a single launch (paresis_detect_counts_multi)."""
+    """Up to 8 images of one detector in a single launch (paresis_detect_counts_multi); one output and one Poisson
+    sequence per image."""
+    n = len(images)
+    if len(outs) != n or len(sequences) != n:
+        raise ValueError("detect_counts_multi: %d images, %d outputs and %d sequences" % (n, len(outs), len(sequences)))
     nx, ny = images[0].shape
     sh = 0 if src_kernel is None else (src_kernel.numel() - 1) // 2
     ph = 0 if psf_kernel is None else (psf_kernel.numel() - 1) // 2
-    n = len(images)
     ip = (ctypes.c_void_p * n)(*[_ptr(t, torch.float32) for t in images])
     op = (ctypes.c_void_p * n)(*[_ptr(t, torch.float32) for t in outs])
     sq = (ctypes.c_uint64 * n)(*[int(q) & (2 ** 64 - 1) for q in sequences])

@@ -283,10 +283,13 @@ detect_fused_kernel(const float* __restrict__ img, FusedShape s, const float* __
 template <bool NOISE, int TAPS>
 static int launch_fused(const float* image, const FusedShape& s, const float* gs, const float* gp, float* out,
                         uint64_t seed, uint64_t seq, size_t smem, cudaStream_t st) {
-    static size_t configured = 0;
-    if (smem > configured) {
+    static size_t configured[32] = {0};    // per device: the attribute belongs to the device's copy of the kernel
+    int dev = 0;
+    PARESIS_CUDA(cudaGetDevice(&dev));
+    if (dev < 0 || dev >= 32) dev = 0;
+    if (smem > configured[dev]) {
         PARESIS_CUDA(cudaFuncSetAttribute(detect_fused_kernel<NOISE, TAPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        configured = smem;
+        configured[dev] = smem;
     }
     const dim3 grid(div_up(s.det_y, TB), div_up(s.det_x, TB)), block(FUSED_TX, FUSED_TY);
     detect_fused_kernel<NOISE, TAPS><<<grid, block, smem, st>>>(image, s, gs, gp, out, seed, seq);
