@@ -350,6 +350,60 @@ int paresis_fresnel_spectrum(paresis_fresnel_plan* plan, const paresis_c32* wave
 int paresis_fresnel_from_spectrum(paresis_fresnel_plan* plan, const paresis_c32* hx, const paresis_c32* hy, paresis_c32 phase,
                                   paresis_c32* wave_out, float* intensity_acc, paresis_stream stream);
 
+/* Experiment.computeSampleAndReferenceImages_Fresnel for one membrane position in ONE call (Experiment.py:279-405).
+ * The host prepares, per spectrum energy, the transmission coefficients (fp64) and the three transfer kernels with
+ * their global phases exp(ikz/M) (:250); the library runs the whole launch sequence on `stream`. */
+typedef struct {
+    const float* thickness;
+    double atten;              /* k beta, 1/m */
+    double phase;              /* k delta, 1/m */
+} paresis_wave_layer;
+
+typedef struct {
+    float amplitude_membrane;  /* sqrt(I0*flux*air*efficiency*plate) * exp(-k sum(beta u)) of the uniform membrane layers
+                                  (:308-338; the plate scales every intensity linearly, :352-356) */
+    float amplitude_propag;    /* sqrt(I0*flux*air*efficiency*plate): the sample-only beam (:365) */
+    double white;              /* added to the white field of the bin (:372-375): amplitude_propag^2 in fp64 */
+    const paresis_wave_layer* membrane_host;   /* the membrane's maps (:338), any number >= 1 */
+    int n_membrane;
+    paresis_wave_layer sample[PARESIS_MAX_LAYERS];   /* the sample's maps (:344, :365) */
+    int n_sample;
+    const paresis_fresnel_kernel* reference;   /* membrane -> detector, d2 + d3, magnification (:349) */
+    paresis_c32 phase_reference;
+    const paresis_fresnel_kernel* to_object;   /* membrane -> object, d2, magMemObj = (d1 + d2) / d1 (:340-341) */
+    paresis_c32 phase_to_object;
+    const paresis_fresnel_kernel* to_detector; /* object -> detector, d3, magnification (:348, :365) */
+    paresis_c32 phase_to_detector;
+    int close_bin;             /* run the detector after this energy (:378) */
+} paresis_fresnel_energy;
+
+typedef struct {
+    paresis_fresnel_plan* plan;          /* nx x ny, the size of every map, wave and accumulator below */
+    int oversampling, det_x, det_y;
+    int first_point;                     /* membrane position 0: propagation and white images too (:359-375) */
+    int n_energies;
+    const paresis_fresnel_energy* energies_host;
+    paresis_c32* wave_a; paresis_c32* wave_b;   /* [nx][ny] scratch */
+    float* acc_sample; float* acc_ref; float* acc_propag; float* acc_white;   /* [nx][ny] accumulators (any content);
+                                                                                 acc_propag: first_point only, acc_white:
+                                                                                 first_point with outputs only */
+    double* means;             /* [n_energies]: SUM over the image of |reference beam|^2 of each energy alone, formed
+                                  while it is accumulated; divide by nx*ny for the per-energy mean (:351-358).  May be NULL. */
+    float* detect_work;        /* see paresis_detect_counts; may be NULL for ordinary kernel sizes */
+    const float* src_kernel; int src_half;
+    const float* psf_kernel; int psf_half;
+    int noise; uint64_t seed; uint64_t sequence;   /* Poisson stream: image k of bin b uses sequence + 4b + k */
+    float* out_sample; float* out_ref; float* out_propag; float* out_white;   /* [n_bins][det_x][det_y].  All NULL: the
+                                  energies are accumulated only and close_bin is ignored (the caller runs the detector,
+                                  as the energy-sharded path does) */
+} paresis_fresnel_job;
+
+/* Per energy: transmission through the membrane -> wave_a; wave_a -> detector into acc_ref (+ means[e]); wave_a ->
+ * object -> wave_b; transmission through the sample; wave_b -> detector into acc_sample; at position 0 the sample-only
+ * beam into acc_propag.  Accumulators start from zero and are zeroed again after each detector run.  Every argument is
+ * checked before the first CUDA call (PARESIS_ERR_ARG). */
+int paresis_fresnel_run(const paresis_fresnel_job* job_host, paresis_stream stream);
+
 /* ---------------------------------------------------------------------------------------
  * Detector
  * ------------------------------------------------------------------------------------- */

@@ -26,7 +26,7 @@ EXPORTS = (
     "paresis_version", "paresis_last_error", "paresis_set_tuning", "paresis_trim", "paresis_splat", "paresis_refract_phi", "paresis_refract_layers",
     "paresis_transmit_rt", "paresis_transmit_wave", "paresis_mix_maps", "paresis_fresnel_plan_create", "paresis_fresnel_plan_destroy",
     "paresis_fresnel_plan_bytes", "paresis_fresnel_propagate", "paresis_fresnel_kernel_create", "paresis_fresnel_kernel_destroy",
-    "paresis_fresnel_convolve", "paresis_fresnel_spectrum", "paresis_fresnel_from_spectrum", "paresis_detect_work_floats", "paresis_detect",
+    "paresis_fresnel_convolve", "paresis_fresnel_spectrum", "paresis_fresnel_from_spectrum", "paresis_fresnel_run", "paresis_detect_work_floats", "paresis_detect",
     "paresis_detect_counts", "paresis_detect_counts_multi",
     "paresis_poisson", "paresis_bin_sum", "paresis_raster_work_bytes", "paresis_raster_spheres", "paresis_sphere_map", "paresis_cylinder_map",
     "paresis_fill", "paresis_axpy", "paresis_mean", "paresis_sum_scaled", "paresis_rt_run", "paresis_rt_run_positions",
@@ -108,6 +108,32 @@ class C32(ctypes.Structure):
     _fields_ = [("re", ctypes.c_float), ("im", ctypes.c_float)]
 
 
+class WaveLayer(ctypes.Structure):
+    _fields_ = [("thickness", ctypes.c_void_p), ("atten", ctypes.c_double), ("phase", ctypes.c_double)]
+
+
+class FresnelEnergy(ctypes.Structure):
+    _fields_ = [("amplitude_membrane", ctypes.c_float), ("amplitude_propag", ctypes.c_float), ("white", ctypes.c_double),
+                ("membrane_host", ctypes.POINTER(WaveLayer)), ("n_membrane", ctypes.c_int),
+                ("sample", WaveLayer * MAX_LAYERS), ("n_sample", ctypes.c_int),
+                ("reference", ctypes.c_void_p), ("phase_reference", C32),
+                ("to_object", ctypes.c_void_p), ("phase_to_object", C32),
+                ("to_detector", ctypes.c_void_p), ("phase_to_detector", C32),
+                ("close_bin", ctypes.c_int)]
+
+
+class FresnelJob(ctypes.Structure):
+    _fields_ = [("plan", ctypes.c_void_p), ("oversampling", ctypes.c_int), ("det_x", ctypes.c_int), ("det_y", ctypes.c_int),
+                ("first_point", ctypes.c_int), ("n_energies", ctypes.c_int), ("energies_host", ctypes.POINTER(FresnelEnergy)),
+                ("wave_a", ctypes.c_void_p), ("wave_b", ctypes.c_void_p),
+                ("acc_sample", ctypes.c_void_p), ("acc_ref", ctypes.c_void_p), ("acc_propag", ctypes.c_void_p),
+                ("acc_white", ctypes.c_void_p), ("means", ctypes.c_void_p), ("detect_work", ctypes.c_void_p),
+                ("src_kernel", ctypes.c_void_p), ("src_half", ctypes.c_int), ("psf_kernel", ctypes.c_void_p), ("psf_half", ctypes.c_int),
+                ("noise", ctypes.c_int), ("seed", ctypes.c_uint64), ("sequence", ctypes.c_uint64),
+                ("out_sample", ctypes.c_void_p), ("out_ref", ctypes.c_void_p), ("out_propag", ctypes.c_void_p),
+                ("out_white", ctypes.c_void_p)]
+
+
 def _load():
     if not os.path.exists(LIB_PATH):
         raise ImportError(
@@ -136,6 +162,7 @@ def _load():
         "paresis_fresnel_convolve": [vp, vp, vp, C32, vp, vp, vp],
         "paresis_fresnel_spectrum": [vp, vp, vp],
         "paresis_fresnel_from_spectrum": [vp, vp, vp, C32, vp, vp, vp],
+        "paresis_fresnel_run": [ctypes.POINTER(FresnelJob), vp],
         "paresis_detect": [vp, ci, ci, ci, ci, ci, vp, ci, vp, ci, vp, vp, vp],
         "paresis_detect_counts": [vp, ci, ci, ci, ci, ci, vp, ci, vp, ci, vp, vp, ci, u64, u64, vp],
         "paresis_detect_counts_multi": [ctypes.POINTER(vp), ctypes.POINTER(vp), ctypes.POINTER(u64), ci, ci, ci, ci, ci, ci, vp, ci,
@@ -230,6 +257,12 @@ def rt_run(job, launches_in_job, probe=None):
     else:
         job.probe = 0
     _check(lib.paresis_rt_run(ctypes.byref(job), _stream()), "paresis_rt_run")
+    _count(launches_in_job)
+
+
+def fresnel_run(job, launches_in_job):
+    """paresis_fresnel_run: one membrane position of the Fresnel model (a FresnelJob)."""
+    _check(lib.paresis_fresnel_run(ctypes.byref(job), _stream()), "paresis_fresnel_run")
     _count(launches_in_job)
 
 

@@ -26,6 +26,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "fresnel.cuh"
 #include "fresnel_lines.cuh"
 
 struct paresis_fresnel_kernel {
@@ -138,12 +139,13 @@ mul_lines_kernel(float2* __restrict__ work, const float2* __restrict__ G, int M)
 // |.|^2 into acc instead of (or besides) storing the field.  32 lines x 64 samples per block of 32 x 8 threads; a thread
 // owns four lines (8 apart) of two samples (32 apart), so that one term costs two 128-bit broadcast loads of margin
 // samples and two kernel values for 32 FMAs.  MARGIN > 0: compile-time margin (the loop over the 2m terms unrolls, every
-// shared-memory offset is an immediate); MARGIN = 0: run-time margin m.
+// shared-memory offset is an immediate); MARGIN = 0: run-time margin m.  `sum` (nullable): *sum += the fp64 sum of the
+// block's |.|^2 values, the same fp32 values that go into acc (warp shuffle, then one atomicAdd per block).
 constexpr int POST_L = 32, POST_S = 64, POST_MAXM = 16;
 template <int MARGIN>
 __global__ void __launch_bounds__(256)
 post_lines_kernel(const float2* __restrict__ work, const float2* __restrict__ in, const float2* __restrict__ c, int lines, int n, int m_rt,
-                  int pitch, float2 phase, float2* __restrict__ out, float* __restrict__ acc) {
+                  int pitch, float2 phase, float2* __restrict__ out, float* __restrict__ acc, double* __restrict__ sum) {
     __shared__ float2 tile[POST_L][POST_S + 1];
     __shared__ __align__(16) float2 edge[2 * POST_MAXM][POST_L];   // [term][slot]: lines ty, ty+8 at slots 2ty, 2ty+1; ty+16, ty+24 at 16+2ty, 17+2ty
     __shared__ float2 cwin[POST_S + 2 * POST_MAXM];
@@ -190,6 +192,7 @@ post_lines_kernel(const float2* __restrict__ work, const float2* __restrict__ in
 #pragma unroll
         for (int h = 0; h < 2; ++h) tile[ty + 8 * i][tx + 32 * h] = v[i][h];
     __syncthreads();
+    double part = 0.0;
 #pragma unroll
     for (int i = 0; i < POST_S / 8; ++i) {
         const int so = s0 + ty + 8 * i, lo = l0 + tx;
@@ -197,8 +200,23 @@ post_lines_kernel(const float2* __restrict__ work, const float2* __restrict__ in
             const float2 w = tile[tx][ty + 8 * i];
             const float2 r = make_float2(w.x * phase.x - w.y * phase.y, w.x * phase.y + w.y * phase.x);
             const size_t o = (size_t)so * lines + lo;
+            const float i2 = r.x * r.x + r.y * r.y;
             if (out) out[o] = r;
-            if (acc) acc[o] += r.x * r.x + r.y * r.y;
+            if (acc) acc[o] += i2;
+            part += (double)i2;
+        }
+    }
+    if (sum) {
+        // the tile is no longer read: its first row holds the eight warp sums
+        __syncthreads();
+        for (int o = 16; o > 0; o >>= 1) part += __shfl_down_sync(0xffffffffu, part, o);
+        double* warp_sums = reinterpret_cast<double*>(&tile[0][0]);
+        if (tx == 0) warp_sums[ty] = part;
+        __syncthreads();
+        if (tid == 0) {
+            double s = 0.0;
+            for (int w = 0; w < 8; ++w) s += warp_sums[w];
+            atomicAdd(sum, s);
         }
     }
 }
@@ -309,16 +327,16 @@ static int kernel_fill(paresis_fresnel_plan* p, const float2* hx, const float2* 
 }
 
 static int launch_post(dim3 grid, const float2* work, const float2* in, const float2* c, int lines, int n, int m, int pitch, float2 phase,
-                       float2* out, float* acc, cudaStream_t s) {
-    if (m == 15) post_lines_kernel<15><<<grid, dim3(32, 8), 0, s>>>(work, in, c, lines, n, m, pitch, phase, out, acc);
-    else post_lines_kernel<0><<<grid, dim3(32, 8), 0, s>>>(work, in, c, lines, n, m, pitch, phase, out, acc);
+                       float2* out, float* acc, double* sum, cudaStream_t s) {
+    if (m == 15) post_lines_kernel<15><<<grid, dim3(32, 8), 0, s>>>(work, in, c, lines, n, m, pitch, phase, out, acc, sum);
+    else post_lines_kernel<0><<<grid, dim3(32, 8), 0, s>>>(work, in, c, lines, n, m, pitch, phase, out, acc, sum);
     PARESIS_LAUNCH_CHECK("post_lines_kernel");
     return PARESIS_OK;
 }
 
 // one axis: `lines` lines of n samples (row-major `in`) -> out[s][l]
 static int convolve_axis(paresis_fresnel_plan* p, int ax, const float2* in, int lines, const paresis_fresnel_kernel* k, float2 phase,
-                         float2* out, float* acc, cudaStream_t s) {
+                         float2* out, float* acc, double* sum, cudaStream_t s) {
     const int n = p->len[ax], M = p->fft_len[ax], m = p->margin;
     const dim3 gt((n + POST_S - 1) / POST_S, (lines + POST_L - 1) / POST_L);
     if (p->fused[ax]) {
@@ -332,7 +350,7 @@ static int convolve_axis(paresis_fresnel_plan* p, int ax, const float2* in, int 
             default: rc = launch_line_convolve<14>(in, lines, n, p->tw[ax], k->g_dr[ax], p->work, s); break;
         }
         if (rc != PARESIS_OK) return rc;
-        return launch_post(gt, p->work, in, k->c[ax], lines, n, m, n, phase, out, acc, s);
+        return launch_post(gt, p->work, in, k->c[ax], lines, n, m, n, phase, out, acc, sum, s);
     }
     const dim3 gl((M / 2 + 255) / 256, lines);
     pad_lines_kernel<<<gl, 256, 0, s>>>(in, lines, n, M, p->work);
@@ -344,16 +362,28 @@ static int convolve_axis(paresis_fresnel_plan* p, int ax, const float2* in, int 
     PARESIS_LAUNCH_CHECK("mul_lines_kernel");
     r = cufftExecC2C(p->lines[ax], p->work, p->work, CUFFT_INVERSE);
     if (r != CUFFT_SUCCESS) return fft_error(r, "cufftExecC2C inverse (lines)");
-    return launch_post(gt, p->work, in, k->c[ax], lines, n, m, M, phase, out, acc, s);
+    return launch_post(gt, p->work, in, k->c[ax], lines, n, m, M, phase, out, acc, sum, s);
 }
 
-static int convolve(paresis_fresnel_plan* p, const float2* wave_in, const paresis_fresnel_kernel* k, float2 phase, float2* wave_out,
-                    float* acc, cudaStream_t s) {
-    // along y: the nx rows of the wave -> mid[ny][nx]; along x: the ny rows of mid -> out[nx][ny]
-    const int rc = convolve_axis(p, 1, wave_in, p->nx, k, make_float2(1.f, 0.f), p->mid, nullptr, s);
+}  // namespace paresis
+
+// along y: the nx rows of the wave -> mid[ny][nx]; along x: the ny rows of mid -> out[nx][ny] (+ acc, + *sum)
+int paresis::fresnel_convolve(paresis_fresnel_plan* p, const float2* wave_in, const paresis_fresnel_kernel* k, float2 phase,
+                              float2* wave_out, float* acc, double* sum, cudaStream_t s) {
+    const int rc = convolve_axis(p, 1, wave_in, p->nx, k, make_float2(1.f, 0.f), p->mid, nullptr, nullptr, s);
     if (rc != PARESIS_OK) return rc;
-    return convolve_axis(p, 0, p->mid, p->ny, k, phase, wave_out, acc, s);
+    return convolve_axis(p, 0, p->mid, p->ny, k, phase, wave_out, acc, sum, s);
 }
+
+bool paresis::fresnel_kernel_fits(const paresis_fresnel_plan* p, const paresis_fresnel_kernel* k) {
+    for (int ax = 0; ax < 2; ++ax)
+        if (k->len[ax] != p->len[ax] || k->fft_len[ax] != p->fft_len[ax]) return false;
+    return true;
+}
+
+void paresis::fresnel_plan_dims(const paresis_fresnel_plan* p, int* nx, int* ny) { *nx = p->nx; *ny = p->ny; }
+
+namespace paresis {
 
 static int ensure_2d(paresis_fresnel_plan* p) {
     if (p->have_2d) return PARESIS_OK;
@@ -487,13 +517,13 @@ extern "C" int paresis_fresnel_convolve(paresis_fresnel_plan* p, const paresis_c
         set_last_error("paresis_fresnel_convolve: null pointer");
         return PARESIS_ERR_ARG;
     }
-    for (int ax = 0; ax < 2; ++ax)
-        if (kernel->len[ax] != p->len[ax] || kernel->fft_len[ax] != p->fft_len[ax]) {
-            set_last_error("paresis_fresnel_convolve: the kernel was prepared for a %d x %d plan, this one is %d x %d", kernel->len[0],
-                           kernel->len[1], p->len[0], p->len[1]);
-            return PARESIS_ERR_ARG;
-        }
-    return convolve(p, (const float2*)wave_in, kernel, make_float2(phase.re, phase.im), (float2*)wave_out, intensity_acc, (cudaStream_t)stream);
+    if (!fresnel_kernel_fits(p, kernel)) {
+        set_last_error("paresis_fresnel_convolve: the kernel was prepared for a %d x %d plan, this one is %d x %d", kernel->len[0],
+                       kernel->len[1], p->len[0], p->len[1]);
+        return PARESIS_ERR_ARG;
+    }
+    return fresnel_convolve(p, (const float2*)wave_in, kernel, make_float2(phase.re, phase.im), (float2*)wave_out, intensity_acc, nullptr,
+                            (cudaStream_t)stream);
 }
 
 extern "C" int paresis_fresnel_propagate(paresis_fresnel_plan* p, const paresis_c32* wave_in,
@@ -506,7 +536,7 @@ extern "C" int paresis_fresnel_propagate(paresis_fresnel_plan* p, const paresis_
     cudaStream_t s = (cudaStream_t)stream;
     const int rc = kernel_fill(p, (const float2*)hx, (const float2*)hy, &p->own, s);
     if (rc != PARESIS_OK) return rc;
-    return convolve(p, (const float2*)wave_in, &p->own, make_float2(phase.re, phase.im), (float2*)wave_out, intensity_acc, s);
+    return fresnel_convolve(p, (const float2*)wave_in, &p->own, make_float2(phase.re, phase.im), (float2*)wave_out, intensity_acc, nullptr, s);
 }
 
 // Two propagations of the SAME field over different distances (Experiment.py:340-341 and :349 both start from the wave

@@ -236,18 +236,10 @@ class ImageFormation:
         out["_stack"] = stack
         return out
 
-    def _mean_energy(self, energies, bin_starts=None, sums=None):
-        """Experiment.py:485-486, :523.  ``sums`` = per-energy sums of the reference beam (ray tracing:
-        formed while it is deposited); otherwise ``self.means`` holds the running means of the
-        reference accumulator within each bin (Fresnel)."""
-        if sums is not None:
-            per = np.asarray(sums, dtype=np.float64) / float(self.nx * self.ny)
-        else:
-            r = self.means[:len(energies)].cpu().numpy()
-            per = r.copy()
-            for i in range(1, len(per)):
-                if i not in bin_starts:
-                    per[i] = r[i] - r[i - 1]
+    def _mean_energy(self, energies, sums):
+        """Experiment.py:485-486, :523 (Fresnel :351-358).  ``sums`` = per-energy sums of the reference beam, formed
+        while it is deposited (ray tracing) or propagated (Fresnel)."""
+        per = np.asarray(sums, dtype=np.float64) / float(self.nx * self.ny)
         return float(np.dot(per, energies)), float(per.sum())
 
     # ------------------------------------------------------------------ ray tracing
@@ -498,22 +490,6 @@ class ImageFormation:
         return self.means[:len(indices)] / float(self.nx * self.ny)
 
     # ------------------------------------------------------------------ Fresnel
-    def _reset(self, n_energies):
-        for a in self.acc.values():
-            a.zero_()
-        if n_energies > self.means.numel():
-            self.means = torch.zeros(n_energies, device=self.device, dtype=torch.float64)
-
-    def _close_bin(self, scene, out, ibin, point_num, first, white_sum, sequence_base):
-        fwhm = scene.effective_source_fwhm()
-        seq = ((sequence_base + point_num) << 16) + ibin * 4
-        self.detect(self.acc["sample"], fwhm, scene.psf_sigma, seq + 0, out["sample"][ibin])
-        self.detect(self.acc["reference"], fwhm, scene.psf_sigma, seq + 1, out["reference"][ibin])
-        if first:
-            self.detect(self.acc["propag"], fwhm, scene.psf_sigma, seq + 2, out["propag"][ibin])
-            abi.fill(self.acc["white"], white_sum)
-            self.detect(self.acc["white"], fwhm, scene.psf_sigma, seq + 3, out["white"][ibin])
-
     def _fresnel_setup(self):
         if self._plan is None:
             self._plan = abi.FresnelPlan(self.nx, self.ny, 15)
@@ -539,50 +515,104 @@ class ImageFormation:
         # |.|^2 ignores the global phase; a returned field carries it (formed in fp64 on the host)
         self._plan.convolve(wave_in, kern, phase if wave_out is not None else 1.0, wave_out, intensity_acc)
 
-    @_on_own_device
-    def compute_fresnel(self, scene, point_num, sequence_base=0):
-        """Experiment.computeSampleAndReferenceImages_Fresnel (Experiment.py:279-405)."""
-        s = scene
+    @staticmethod
+    def fresnel_amplitude(scene, energy, flux):
+        """Amplitude of the incident wave at one energy (Experiment.py:308, :320-333); the plate scales every intensity
+        linearly (:352-356).  Its square is that energy's share of the white field (:372-375)."""
+        i0 = scene.mean_shot_count / scene.os ** 2 * flux * scene.common_factor(energy)
+        return float(np.sqrt(i0 * scene.plate_factor(energy)))
+
+    def _fresnel_energies(self, scene, indices, closing):
+        """ctypes array of paresis_fresnel_energy for the spectrum entries ``indices``; ``closing`` = set of spectrum
+        indices after which the detector runs.  Returns it with what it points to."""
         self._fresnel_setup()
-        first = point_num == 0
-        out = self._new_outputs(len(s.thresholds), first)
-        self._reset(len(s.spectrum))
-        w_a, w_b = self._waves
+        s = scene
         mag_mem_obj = (s.d1 + s.d2) / s.d1                                            # :340
-        ibin, white_sum, bin_starts = 0, 0.0, {0}
+        energies = (abi.FresnelEnergy * len(indices))()
+        keep = []
         fits = self.sample_fits(s, with_membrane=False)
-        for ie, (energy, flux) in enumerate(s.spectrum):
+        for slot, ie in enumerate(indices):
+            energy, flux = s.spectrum[ie]
             k = hm.wavenumber(energy * 1000)
-            i0 = s.mean_shot_count / s.os ** 2 * flux * s.common_factor(energy)       # :308, :320-333
-            plate = s.plate_factor(energy)
-            amp = float(np.sqrt(i0 * plate))   # the plate scales every intensity linearly (:352-356)
+            amp = self.fresnel_amplitude(s, energy, flux)
             mem_maps, mem_ub, _ = self._split(s.membrane, energy)
             smp_maps = self._sample_layers(s, energy, fits)
             if not mem_maps or not smp_maps:
                 raise NotImplementedError("scene needs 1+ membrane maps and a sample")
+            en = energies[slot]
             # after the membrane (:338); uniform layers: attenuation folded in, constant phase dropped
-            abi.transmit_wave(None, amp * np.exp(-k * mem_ub), [t for t, _, _ in mem_maps],
-                              [k * b for _, _, b in mem_maps], [k * d for _, d, _ in mem_maps], w_a)
-            # reference beam: membrane -> detector in one hop (:349, :354)
-            self.propagate(s, w_a, s.d3 + s.d2, energy, s.magnification, intensity_acc=self.acc["reference"])
-            # sample beam: membrane -> object (:340-341), through the sample (:344), -> detector (:348)
-            self.propagate(s, w_a, s.d2, energy, mag_mem_obj, wave_out=w_b)
-            abi.transmit_wave(w_b, 0.0, [t for t, _, _ in smp_maps], [k * b for _, _, b in smp_maps],
-                              [k * d for _, d, _ in smp_maps], w_b)
-            self.propagate(s, w_b, s.d3, energy, s.magnification, intensity_acc=self.acc["sample"])
-            abi.mean(self.acc["reference"], self.means[ie:ie + 1])
-            if first:
-                abi.transmit_wave(None, amp, [t for t, _, _ in smp_maps], [k * b for _, _, b in smp_maps],
-                                  [k * d for _, d, _ in smp_maps], w_b)               # :365
-                self.propagate(s, w_b, s.d3, energy, s.magnification, intensity_acc=self.acc["propag"])
-                white_sum += amp * amp                                                # :372-375
-            if energy > s.thresholds[ibin] - s.energy_sampling / 2:                   # :378
-                self._close_bin(s, out, ibin, point_num, first, white_sum, sequence_base)
-                ibin += 1
-                if ie + 1 < len(s.spectrum):
-                    for a in self.acc.values():
-                        a.zero_()
-                    white_sum = 0.0
-                    bin_starts.add(ie + 1)
-        out["mean_energy"] = self._mean_energy([e for e, _ in s.spectrum], bin_starts=bin_starts)
+            en.amplitude_membrane = amp * np.exp(-k * mem_ub)
+            en.amplitude_propag = amp
+            en.white = amp * amp
+            membrane = (abi.WaveLayer * len(mem_maps))()
+            for dst, (t, d, b) in zip(membrane, mem_maps):
+                dst.thickness, dst.atten, dst.phase = t.data_ptr(), k * b, k * d
+            en.membrane_host, en.n_membrane = membrane, len(mem_maps)
+            for dst, (t, d, b) in zip(en.sample, smp_maps):
+                dst.thickness, dst.atten, dst.phase = t.data_ptr(), k * b, k * d
+            en.n_sample = len(smp_maps)
+            hops = (("reference", s.d3 + s.d2, s.magnification),                      # :349
+                    ("to_object", s.d2, mag_mem_obj),                                 # :340-341
+                    ("to_detector", s.d3, s.magnification))                           # :348, :365
+            for name, distance, magnification in hops:
+                kern, phase = self._transfer(s, distance, energy, magnification)
+                setattr(en, name, kern._h)
+                setattr(en, "phase_" + name, abi.C32(float(np.real(phase)), float(np.imag(phase))))
+            en.close_bin = 1 if ie in closing else 0
+            keep += [membrane] + [t for t, _, _ in mem_maps + smp_maps]
+        return energies, keep
+
+    def _fresnel_job(self, scene, energies, first, sequence):
+        fwhm = scene.effective_source_fwhm()
+        src = self._gauss(fwhm / 2.355) if fwhm != 0 else None
+        psf = self._gauss(scene.psf_sigma) if scene.psf_sigma != 0 else None
+        if len(energies) > self.means.numel():
+            self.means = torch.zeros(len(energies), device=self.device, dtype=torch.float64)
+        job = abi.FresnelJob()
+        job.plan = self._plan._h
+        job.oversampling, job.det_x, job.det_y = self.os, self.det_x, self.det_y
+        job.first_point, job.n_energies, job.energies_host = int(first), len(energies), energies
+        job.wave_a, job.wave_b = self._waves[0].data_ptr(), self._waves[1].data_ptr()
+        job.acc_sample, job.acc_ref = self.acc["sample"].data_ptr(), self.acc["reference"].data_ptr()
+        job.acc_propag, job.acc_white = self.acc["propag"].data_ptr(), self.acc["white"].data_ptr()
+        job.means, job.detect_work = self.means.data_ptr(), self.work.data_ptr()
+        job.src_kernel, job.src_half = (src.data_ptr(), (src.numel() - 1) // 2) if src is not None else (None, 0)
+        job.psf_kernel, job.psf_half = (psf.data_ptr(), (psf.numel() - 1) // 2) if psf is not None else (None, 0)
+        job.noise, job.seed, job.sequence = int(self.poisson), self.seed, sequence
+        return job, (src, psf)
+
+    @staticmethod
+    def _fresnel_launches(n_energies, n_bins, first):
+        # per energy: 2 transmissions + 3 propagations (+ 1 + 1 at position 0), counted as _cabi does; per bin: the
+        # detector (+ the white fill)
+        return n_energies * (20 if not first else 27) + n_bins * (2 if first else 1)
+
+    @_on_own_device
+    def compute_fresnel(self, scene, point_num, sequence_base=0):
+        """Experiment.computeSampleAndReferenceImages_Fresnel (Experiment.py:279-405) as one library call
+        (paresis_fresnel_run).  Returns what compute_rt returns."""
+        s = scene
+        first = point_num == 0
+        bins = self.bins(s)
+        nbins, n_e = len(s.thresholds), len(s.spectrum)
+        out = self._new_outputs(nbins, first)
+        closing = {b[-1] for b in bins[:nbins]}
+        energies, keep = self._fresnel_energies(s, list(range(n_e)), closing)
+        job, keep2 = self._fresnel_job(s, energies, first, self.sequence(point_num, sequence_base))
+        job.out_sample, job.out_ref = out["sample"].data_ptr(), out["reference"].data_ptr()
+        if first:
+            job.out_propag, job.out_white = out["propag"].data_ptr(), out["white"].data_ptr()
+        abi.fresnel_run(job, self._fresnel_launches(n_e, len(closing), first))
+        out["mean_energy"] = self._mean_energy([e for e, _ in s.spectrum], sums=self.means[:n_e].cpu().numpy())
         return out
+
+    @_on_own_device
+    def accumulate_fresnel(self, scene, point_num, indices):
+        """The energies ``indices`` (all of ONE detector bin) of a position, without the detector: leaves the partial
+        sums in ``self.acc`` and returns the per-energy means of the reference beam (device float64 tensor,
+        len(indices)).  The Fresnel counterpart of accumulate_rt (shard.py)."""
+        first = point_num == 0
+        energies, keep = self._fresnel_energies(scene, list(indices), closing=set())
+        job, keep2 = self._fresnel_job(scene, energies, first, 0)
+        abi.fresnel_run(job, self._fresnel_launches(len(indices), 0, first))
+        return self.means[:len(indices)] / float(self.nx * self.ny)

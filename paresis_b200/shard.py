@@ -46,8 +46,8 @@ def combine_means(values, indices, n_total, group=None):
 
 
 class ShardedPosition:
-    """What ``compute_rt_energy_sharded(..., defer=True)`` returns on every rank: the device work of the position is
-    queued, its host-side tail is not done yet.  ``finish()`` waits for the per-energy means and the status flags (one
+    """What ``compute_rt_energy_sharded(..., defer=True)`` and ``compute_fresnel_energy_sharded(..., defer=True)`` return on
+    every rank: the device work of the position is queued, its host-side tail is not done yet.  ``finish()`` waits for the per-energy means and the status flags (one
     all_reduce, already queued), raises ``InsaneValues`` on every rank if any rank saw a non-finite value, and returns what
     the immediate call returns (the result dict on the owner, None elsewhere).  The images must not be used before it."""
 
@@ -79,6 +79,26 @@ def compute_rt_energy_sharded(engine, scene, point_num, owner=0, group=None, seq
     ``defer=True``: return a ``ShardedPosition`` instead, without waiting for the device: the caller queues the next
     position first and calls ``finish()`` on this one afterwards (every rank, same order), so the host's turn-around and
     the device->host read of the means overlap the next position's kernels."""
+    def white(energy, flux):   # Experiment.py:490-497
+        return scene.mean_shot_count / scene.os ** 2 * flux * scene.common_factor(energy) * scene.plate_factor(energy)
+    return _energy_sharded(engine.accumulate_rt, white, engine, scene, point_num, owner, group, sequence_base, reduce_events,
+                           defer)
+
+
+def compute_fresnel_energy_sharded(engine, scene, point_num, owner=0, group=None, sequence_base=0, reduce_events=None,
+                                   defer=False):
+    """The Fresnel model (``ImageFormation.compute_fresnel``) with the spectrum spread over the ranks of ``group``: same
+    arguments and results as ``compute_rt_energy_sharded``."""
+    def white(energy, flux):   # Experiment.py:372-375
+        return engine.fresnel_amplitude(scene, energy, flux) ** 2
+    return _energy_sharded(engine.accumulate_fresnel, white, engine, scene, point_num, owner, group, sequence_base,
+                           reduce_events, defer)
+
+
+def _energy_sharded(accumulate, white_of, engine, scene, point_num, owner, group, sequence_base, reduce_events, defer):
+    """Body of the energy-sharded calls.  ``accumulate(scene, point_num, indices)``: the model's partial sums of some
+    energies of one bin into ``engine.acc``, returning their per-energy reference means; ``white_of(energy, flux)``: one
+    energy's share of the white field."""
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     first = point_num == 0
@@ -95,11 +115,9 @@ def compute_rt_energy_sharded(engine, scene, point_num, owner=0, group=None, seq
         mine = energies_of(indices, rank, world)
         partial.zero_()
         if mine:
-            means[torch.as_tensor(mine, device=engine.device)] = engine.accumulate_rt(scene, point_num, mine)
+            means[torch.as_tensor(mine, device=engine.device)] = accumulate(scene, point_num, mine)
             if first:   # the white field is the incident beam itself: fill it with this rank's share
-                white = sum(scene.mean_shot_count / scene.os ** 2 * scene.spectrum[i][1] *
-                            scene.common_factor(scene.spectrum[i][0]) * scene.plate_factor(scene.spectrum[i][0]) for i in mine)
-                abi.fill(engine.acc["white"], white)
+                abi.fill(engine.acc["white"], sum(white_of(*scene.spectrum[i]) for i in mine))
             for k, name in enumerate(IMAGES[:count]):
                 # the linear part of the detector before the exchange: detector-resolution images travel
                 abi.detect_counts(engine.acc[name], engine.os, engine.det_x, engine.det_y, src, psf, engine.work,
