@@ -524,6 +524,41 @@ int paresis_df_split(const float* intensity, float intensity_uniform, const floa
  * (gaussian_shape, :14-23); df_px == 0 adds the value in place.  out[nx][ny] is accumulated into. */
 int paresis_df_scatter(const float* scattered, const float* df_px, float* out, int nx, int ny, paresis_stream stream);
 
+/* Experiment.computeSampleAndReferenceImages_RT for one membrane position of a scattering sample in ONE call
+ * (Experiment.py:407-526 with fastRefractionDF, refractionFileNumba2.py:88-196).  Per energy, on `stream`:
+ * paresis_df_angle on the scattering material's map -> `angle`; the membrane hop into i_bs; paresis_df_split of i_bs
+ * (limit nx/4) into plain / scattered rays; two dual-beam object hops (hop2 layers): plain -> (acc_sample, acc_ref),
+ * scattered -> (moved, acc_ref); paresis_df_scatter(moved, clean, acc_sample).  Both object hops add to means[e], which
+ * is therefore the sum of the whole reference beam.  At position 0 the sample-only beam goes through the same split, two
+ * single-beam hops (propag layers) and one scatter into acc_propag, and dark_field += dark_field_weight * angle.  At a
+ * bin close the detector runs on 2 or 4 images as in paresis_rt_run.  Every argument is checked before the first CUDA
+ * call (PARESIS_ERR_ARG). */
+typedef struct {
+    const float* scatter_map;  /* thickness map (metres) of the material whose angle applies: with several scattering
+                                  materials, the last one (Sample.py:322-343 overwrites newDf).  Required. */
+    double angle_coeff;        /* df_px = angle_coeff * sqrt(t): 2 delta sqrt(NsphereVol^(1/3) * 1e6) sqrt(ln(2/delta) + 1)
+                                  * d3 / (pixel * M), formed in fp64 on the host (refractionFileNumba2.py:114) */
+    double dark_field_weight;  /* flux * pixel * M / d3: the angle map of this energy back in radians, weighted by the
+                                  spectrum (Experiment.py:491) */
+} paresis_df_energy;
+
+typedef struct {
+    paresis_rt_job rt;         /* as for paresis_rt_run, with these differences: i_bs_group, positions_per_launch, dx_pad,
+                                  dy_pad and probe are ignored; out_* may all be NULL, then the energies are accumulated
+                                  only and close_bin is ignored (the energy-sharded path runs the detector itself);
+                                  acc_white is needed with outputs at position 0 only.  i_bs keeps paresis_rt_run's
+                                  contract: all zero on entry unless i_bs_dirty is set, all zero on exit.  The object
+                                  hops of each energy must fit in PARESIS_MAX_LAYERS maps (mix the sample's maps
+                                  otherwise). */
+    const paresis_df_energy* energies_df_host;   /* [rt.n_energies] */
+    float* angle;              /* [nx][ny] scratch: the angle map in pixels; holds the last energy's when the job has run */
+    float* plain; float* scattered; float* clean; float* moved;   /* [nx][ny] scratch, any content on entry */
+    float* dark_field;         /* optional [nx][ny], position 0 only: += sum over the job's energies of
+                                  dark_field_weight * angle (radians).  The caller zeroes it. */
+} paresis_df_job;
+
+int paresis_df_run(const paresis_df_job* job_host, paresis_stream stream);
+
 /* Result transfers (the reference hands back host arrays: Experiment.py:405, :526, main.py:99): an
  * asynchronous device -> pinned-host copy on the library's copy stream, ordered after `producer`.
  * A lane holds the events of one copy in flight; reuse it once paresis_transfer_wait returned. */

@@ -25,7 +25,7 @@ from refractionFileNumba2 import fastRefraction, fastRefractionDF
 from usefullScripts.getSamplingFactor import is_overSampling_ok
 import torch
 
-from paresis_b200 import engine, geometry, host_api, transfer
+from paresis_b200 import darkfield, engine, geometry, host_api, hostmath, transfer
 from paresis_b200.hostio import xmlparams
 
 
@@ -202,7 +202,9 @@ class Experiment:
     def _layers(self, obj, materialise):
         geom = obj._device_geometry()
         entries = geom.device_entries(materialise=materialise)
-        return [engine.Layer(t, self._lookup(obj.delta[m]), self._lookup(obj.beta[m])) for m, t in enumerate(entries)]
+        models = [darkfield.model_of(obj, m) for m in range(len(entries))]      # Sample.py:322-343
+        return [engine.Layer(t, self._lookup(obj.delta[m]), self._lookup(obj.beta[m]),
+                             hostmath.MODELS[models[m]] if models[m] is not None else None) for m, t in enumerate(entries)]
 
     def _uniform_attenuation(self, obj, energy):
         """exp(-2 k beta t) of an object made of uniform layers (air volume, plate: Sample.py:239-243, :347)."""
@@ -317,9 +319,6 @@ class Experiment:
             Dxreal, Dyreal: displacement maps of the sample-only beam, zero-padded by 15 (from point 0),
             darkFieldPropag: [N, N] dark-field map (zeros unless the sample has a dark-field model).
         """
-        if self.mySampleofInterest._has_dark_field():
-            from paresis_b200 import darkfield
-            return darkfield.compute_rt(self, pointNum)
         thresholds = self._open_bins(pointNum)
         for energy, _ in self.mySource.mySpectrum:
             print("Current Energy: %gkev" % energy)
@@ -334,8 +333,11 @@ class Experiment:
         if want_d:
             self.Dxreal = transfer.fetch(eng.dx_pad, torch.float64)
             self.Dyreal = transfer.fetch(eng.dy_pad, torch.float64)
-        n = self.exp_dict['studyDimensions']
-        self.darkFieldPropag = self._zeros((int(n[0]), int(n[1])))
+        if "dark_field" in res:
+            self.darkFieldPropag = transfer.fetch(res["dark_field"], torch.float64)      # Experiment.py:491, from point 0
+        elif not eng.scatters(scene):
+            n = self.exp_dict['studyDimensions']
+            self.darkFieldPropag = self._zeros((int(n[0]), int(n[1])))
         print("Mean detected energy in reference image", self.exp_dict['meanEnergy'])
         return out[0], out[1], out[2], out[3], self.Dxreal, self.Dyreal, self.darkFieldPropag
 

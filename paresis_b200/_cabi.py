@@ -26,7 +26,7 @@ EXPORTS = (
     "paresis_version", "paresis_last_error", "paresis_set_tuning", "paresis_trim", "paresis_splat", "paresis_refract_phi", "paresis_refract_layers",
     "paresis_transmit_rt", "paresis_transmit_wave", "paresis_mix_maps", "paresis_fresnel_plan_create", "paresis_fresnel_plan_destroy",
     "paresis_fresnel_plan_bytes", "paresis_fresnel_propagate", "paresis_fresnel_kernel_create", "paresis_fresnel_kernel_destroy",
-    "paresis_fresnel_convolve", "paresis_fresnel_spectrum", "paresis_fresnel_from_spectrum", "paresis_fresnel_run", "paresis_detect_work_floats", "paresis_detect",
+    "paresis_fresnel_convolve", "paresis_fresnel_spectrum", "paresis_fresnel_from_spectrum", "paresis_fresnel_run", "paresis_df_run", "paresis_detect_work_floats", "paresis_detect",
     "paresis_detect_counts", "paresis_detect_counts_multi",
     "paresis_poisson", "paresis_bin_sum", "paresis_raster_work_bytes", "paresis_raster_spheres", "paresis_sphere_map", "paresis_cylinder_map",
     "paresis_fill", "paresis_axpy", "paresis_mean", "paresis_sum_scaled", "paresis_rt_run", "paresis_rt_run_positions",
@@ -67,6 +67,16 @@ class RtJob(ctypes.Structure):
                 ("flag", ctypes.c_void_p), ("probe", ctypes.c_int), ("probe_start", ctypes.c_void_p),
                 ("probe_end", ctypes.c_void_p), ("i_bs_dirty", ctypes.c_int), ("i_bs_group", ctypes.c_void_p * (MAX_GROUP - 1)),
                 ("positions_per_launch", ctypes.c_int), ("throughput", ctypes.c_int)]
+
+
+class DfEnergy(ctypes.Structure):
+    _fields_ = [("scatter_map", ctypes.c_void_p), ("angle_coeff", ctypes.c_double), ("dark_field_weight", ctypes.c_double)]
+
+
+class DfJob(ctypes.Structure):
+    _fields_ = [("rt", RtJob), ("energies_df_host", ctypes.POINTER(DfEnergy)), ("angle", ctypes.c_void_p),
+                ("plain", ctypes.c_void_p), ("scattered", ctypes.c_void_p), ("clean", ctypes.c_void_p), ("moved", ctypes.c_void_p),
+                ("dark_field", ctypes.c_void_p)]
 
 
 class GroupEnergy(ctypes.Structure):
@@ -179,6 +189,7 @@ def _load():
         "paresis_mean": [vp, sz, vp, vp],
         "paresis_sum_scaled": [vp, sz, cd, vp, vp],
         "paresis_rt_run": [ctypes.POINTER(RtJob), vp],
+        "paresis_df_run": [ctypes.POINTER(DfJob), vp],
         "paresis_two_sphere_phantom": [ci, ci, ci, cd, vp, vp],
         "paresis_df_angle": [vp, cd, vp, sz, vp],
         "paresis_df_split": [vp, cf, vp, cf, vp, vp, vp, sz, vp],
@@ -263,6 +274,12 @@ def rt_run(job, launches_in_job, probe=None):
 def fresnel_run(job, launches_in_job):
     """paresis_fresnel_run: one membrane position of the Fresnel model (a FresnelJob)."""
     _check(lib.paresis_fresnel_run(ctypes.byref(job), _stream()), "paresis_fresnel_run")
+    _count(launches_in_job)
+
+
+def df_run(job, launches_in_job):
+    """paresis_df_run: one membrane position of the ray-tracing model with a scattering sample (a DfJob)."""
+    _check(lib.paresis_df_run(ctypes.byref(job), _stream()), "paresis_df_run")
     _count(launches_in_job)
 
 

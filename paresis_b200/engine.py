@@ -31,17 +31,22 @@ PER_POSITION = _PerPosition()
 
 
 class Layer:
-    """One material of an object: a device thickness map (metres) or a uniform thickness."""
+    """One material of an object: a device thickness map (metres) or a uniform thickness.
 
-    __slots__ = ("map", "uniform", "delta", "beta")
+    ``scatter``: the dark-field model of a scattering material of the sample, (sphere radius um, volume fraction) as in
+    hostmath.MODELS (Sample.py:322-343), or None.  Ray tracing scales that material's delta and beta by the fraction and
+    spreads the rays by its scattering angle (paresis_df_run); the Fresnel model ignores it, as the reference does."""
 
-    def __init__(self, thickness, delta, beta):
+    __slots__ = ("map", "uniform", "delta", "beta", "scatter")
+
+    def __init__(self, thickness, delta, beta, scatter=None):
         # delta / beta: {energy_keV: value}
         if isinstance(thickness, torch.Tensor) or thickness is PER_POSITION:
             self.map, self.uniform = thickness, None
         else:
             self.map, self.uniform = None, float(thickness)
         self.delta, self.beta = delta, beta
+        self.scatter = scatter
 
 
 class Scene:
@@ -126,6 +131,7 @@ class ImageFormation:
         self._waves = None
         self._mixed = {}         # (material maps, weights) -> the mixed maps of one energy (mixed_sample)
         self._mixed_of = None    # the material maps the cached mixed maps were made from
+        self._df = None          # scratch images of paresis_df_run, made with the first scattering sample
 
     # ------------------------------------------------------------------ helpers
     def _gauss(self, sigma):
@@ -221,11 +227,27 @@ class ImageFormation:
         p_map, b_map, _ = self._mixed[key]
         return [(p_map, d_star, 0.0), (b_map, 0.0, b_star)]
 
-    def _sample_layers(self, scene, energy, fits):
-        """-> [(map, delta, beta)] the hops take for the sample at ``energy``."""
-        if fits:
-            return self._split(scene.sample, energy)[0]
-        return self.mixed_sample(scene.sample, energy)
+    def _sample_layers(self, scene, energy, fits, fractions=None):
+        """-> [(map, delta, beta)] the hops take for the sample at ``energy``; ``fractions``: see mixed_sample."""
+        if not fits:
+            return self.mixed_sample(scene.sample, energy, fractions)
+        maps = self._split(scene.sample, energy)[0]
+        if fractions is None:
+            return maps
+        return [(t, d * f, b * f) for (t, d, b), f in zip(maps, fractions)]
+
+    @staticmethod
+    def scatters(scene):
+        """Whether a material of the sample has a dark-field model (Layer.scatter)."""
+        return any(L.scatter is not None for L in scene.sample)
+
+    @staticmethod
+    def _rt_fractions(scene):
+        """Per sample layer: the volume fraction of a scattering material, 1 otherwise (Sample.py:333, :344); None when
+        nothing scatters."""
+        if not ImageFormation.scatters(scene):
+            return None
+        return [L.scatter[1] if L.scatter is not None else 1.0 for L in scene.sample]
 
     def _new_outputs(self, nbins, first):
         """Detector images of one position, stacked [image][bin][x][y] in ONE device buffer
@@ -264,13 +286,14 @@ class ImageFormation:
         energies = (abi.RtEnergy * len(indices))()
         keep = []
         fits = self.sample_fits(s, with_membrane=True)
+        fractions = self._rt_fractions(s)
         for slot, ie in enumerate(indices):
             energy, flux = s.spectrum[ie]
             k = hm.wavenumber(energy * 1000)
             i0 = s.mean_shot_count / s.os ** 2 * flux * s.common_factor(energy)      # :438, :451-459
             plate = s.plate_factor(energy)
             mem_maps, mem_ub, _ = self._split(s.membrane, energy)
-            smp_maps = self._sample_layers(s, energy, fits)
+            smp_maps = self._sample_layers(s, energy, fits, fractions)
             if not mem_maps or not smp_maps or len(mem_maps) + len(smp_maps) > abi.MAX_LAYERS:
                 raise NotImplementedError("scene needs 1+ membrane maps and a sample, at most %d maps per hop"
                                           % abi.MAX_LAYERS)
@@ -291,7 +314,7 @@ class ImageFormation:
             en.close_bin = 1 if ie in closing else 0
         return energies, keep
 
-    def _rt_job(self, scene, energies, first, sequence):
+    def _rt_job(self, scene, energies, first, sequence, group=True):
         fwhm = scene.effective_source_fwhm()
         src = self._gauss(fwhm / 2.355) if fwhm != 0 else None
         psf = self._gauss(scene.psf_sigma) if scene.psf_sigma != 0 else None
@@ -302,7 +325,7 @@ class ImageFormation:
         job.first_point, job.n_energies, job.energies_host = int(first), len(energies), energies
         job.i_bs = self.i_bs.data_ptr()
         job.i_bs_dirty = 1 if self._i_bs_dirty else 0
-        for k, t in enumerate(self._group_buffers(scene)):
+        for k, t in enumerate(self._group_buffers(scene) if group else ()):
             job.i_bs_group[k] = t.data_ptr()
         job.acc_sample, job.acc_ref = self.acc["sample"].data_ptr(), self.acc["reference"].data_ptr()
         job.acc_propag, job.acc_white = self.acc["propag"].data_ptr(), self.acc["white"].data_ptr()
@@ -321,6 +344,64 @@ class ImageFormation:
             store.append(torch.zeros((self.nx, self.ny), device=self.device, dtype=torch.float32))
         return store[:want]
 
+    # ------------------------------------------------------------------ scattering samples (dark field)
+    def _df_energies(self, scene, indices):
+        """ctypes array of paresis_df_energy for the spectrum entries ``indices``: the angle map comes from the last
+        scattering material's own thickness map (Sample.py:322-343 overwrites newDf), also when the hops see mixed maps."""
+        s = scene
+        to_px = s.d3 / (s.study_pixel_um * 1e-6 * s.magnification)           # refractionFileNumba2.py:114
+        last = [L for L in s.sample if L.scatter is not None][-1]
+        if last.map is None or last.map is PER_POSITION:
+            raise NotImplementedError("a scattering material needs a thickness map of its own")
+        out = (abi.DfEnergy * len(indices))()
+        for slot, ie in enumerate(indices):
+            energy, flux = s.spectrum[ie]
+            out[slot].scatter_map = last.map.data_ptr()
+            out[slot].angle_coeff = hm.angle_coefficient(last.delta.get(energy, 0.0), last.scatter) * to_px
+            out[slot].dark_field_weight = flux / to_px                          # Experiment.py:491, in radians
+        return out, last.map
+
+    def _df_scratch(self):
+        """The scratch images of paresis_df_run: angle, plain, scattered, clean, moved (any content between jobs)."""
+        if self._df is None:
+            self._df = {k: torch.empty((self.nx, self.ny), device=self.device, dtype=torch.float32)
+                        for k in ("angle", "plain", "scattered", "clean", "moved")}
+        return self._df
+
+    def _df_job(self, scene, job, indices, dark_field=None):
+        """Wrap a paresis_rt_job (``job``) into a paresis_df_job for the spectrum entries ``indices``."""
+        df_energies, keep = self._df_energies(scene, indices)
+        scratch = self._df_scratch()
+        dj = abi.DfJob()
+        dj.rt = job
+        dj.energies_df_host = df_energies
+        for k in ("angle", "plain", "scattered", "clean", "moved"):
+            setattr(dj, k, scratch[k].data_ptr())
+        dj.dark_field = dark_field.data_ptr() if dark_field is not None else None
+        return dj, (df_energies, keep)
+
+    @staticmethod
+    def _df_launches(n_energies, n_bins, first):
+        # per energy: angle, membrane hop, split, 2 object hops, scatter (+ split, 2 hops, scatter, dark-field axpy at
+        # position 0); per bin: the detector (+ the white fill)
+        return n_energies * (11 if first else 6) + n_bins * (2 if first else 1)
+
+    def _df_displacement(self, scene):
+        """Dx, Dy of the sample-only beam at the last energy into self.dx_pad / self.dy_pad, zero-padded by
+        margin2 = ceil(6 max(angle)) as fastRefractionDF returns them (refractionFileNumba2.py:115-117, Experiment.py:492);
+        the angle map is the one paresis_df_run left in its scratch."""
+        s = scene
+        scratch = self._df_scratch()
+        margin2 = int(np.ceil(float(scratch["angle"].max().item()) * 6))
+        shape = (self.nx + 2 * margin2, self.ny + 2 * margin2)
+        self.dx_pad = torch.zeros(shape, device=self.device, dtype=torch.float32)
+        self.dy_pad = torch.zeros_like(self.dx_pad)
+        g3 = hm.refraction_gradient_scale(s.d3, s.magnification, s.study_pixel_um)
+        layers = self._sample_layers(s, s.spectrum[-1][0], self.sample_fits(s, with_membrane=True), self._rt_fractions(s))
+        # the image goes to scratch: only the maps are wanted (paresis_df_run clears `moved` before it reads it)
+        abi.refract_layers(None, 1.0, [(t, d * g3, 0.0, 0.0) for t, d, b in layers], scratch["moved"], margin=margin2,
+                           dx_pad=self.dx_pad, dy_pad=self.dy_pad)
+
     @staticmethod
     def sequence(point_num, sequence_base=0):
         """Poisson stream id of a position; image k of bin b draws from sequence + 4b + k."""
@@ -330,30 +411,41 @@ class ImageFormation:
     def compute_rt(self, scene, point_num, want_displacement=False, sequence_base=0, probe=None, want_mean=True,
                    defer=False):
         """Experiment.computeSampleAndReferenceImages_RT (Experiment.py:407-526) as one library
-        call (paresis_rt_run).
+        call (paresis_rt_run; paresis_df_run when a sample material scatters, Layer.scatter).
 
         Returns a dict of device tensors [nbins, det_x, det_y]: sample, reference (+ propag, white
         at position 0; absent keys are all-zero images), plus ``mean_energy`` = (sum E*mean,
-        sum mean) of Experiment.py:485-486."""
+        sum mean) of Experiment.py:485-486.  A scattering sample adds ``dark_field`` at position 0: the
+        [nx, ny] float32 map of Experiment.py:491 (radians, summed over the spectrum).  ``want_displacement``
+        leaves the Dx, Dy maps of the sample-only beam at the last energy in self.dx_pad / self.dy_pad."""
         s = scene
         first = point_num == 0
         bins = self.bins(s)
         nbins, n_e = len(s.thresholds), len(s.spectrum)
         out = self._new_outputs(nbins, first)
+        scatters = self.scatters(s)
         wd = first and want_displacement
-        if wd and self.dx_pad is None:
+        if wd and not scatters and (self.dx_pad is None or self.dx_pad.shape != (self.nx + 30, self.ny + 30)):
             self.dx_pad = torch.empty((self.nx + 30, self.ny + 30), device=self.device, dtype=torch.float32)
             self.dy_pad = torch.empty_like(self.dx_pad)
         closing = {b[-1] for b in bins[:nbins]}
         energies, keep = self._rt_energies(s, list(range(n_e)), closing)
-        job, keep2 = self._rt_job(s, energies, first, self.sequence(point_num, sequence_base))
+        job, keep2 = self._rt_job(s, energies, first, self.sequence(point_num, sequence_base), group=not scatters)
         job.out_sample, job.out_ref = out["sample"].data_ptr(), out["reference"].data_ptr()
         if first:
             job.out_propag, job.out_white = out["propag"].data_ptr(), out["white"].data_ptr()
-        if wd:
-            job.dx_pad, job.dy_pad = self.dx_pad.data_ptr(), self.dy_pad.data_ptr()
-        launches = n_e * (3 if first else 2) + len(closing) * (2 if first else 1)
-        self._run(job, launches, probe)
+        if scatters:
+            if first:
+                out["dark_field"] = torch.zeros((self.nx, self.ny), device=self.device, dtype=torch.float32)
+            dj, keep3 = self._df_job(s, job, list(range(n_e)), out.get("dark_field"))
+            self._run_df(dj, self._df_launches(n_e, len(closing), first))
+            if wd:
+                self._df_displacement(s)
+        else:
+            if wd:
+                job.dx_pad, job.dy_pad = self.dx_pad.data_ptr(), self.dy_pad.data_ptr()
+            launches = n_e * (3 if first else 2) + len(closing) * (2 if first else 1)
+            self._run(job, launches, probe)
         if want_mean and defer:
             # no host synchronisation here: the per-energy sums and the status flag travel with the images
             # (one small device buffer); the caller finishes with finish_deferred() once they are on the host
@@ -376,6 +468,12 @@ class ImageFormation:
         """paresis_rt_run keeps I_bs all-zero between jobs; a failed call may leave it dirty."""
         self._i_bs_dirty = True
         abi.rt_run(job, launches, probe)
+        self._i_bs_dirty = False
+
+    def _run_df(self, dj, launches):
+        """paresis_df_run keeps the same I_bs contract."""
+        self._i_bs_dirty = True
+        abi.df_run(dj, launches)
         self._i_bs_dirty = False
 
     # ------------------------------------------------------------------ many positions, one call
@@ -410,6 +508,9 @@ class ImageFormation:
         propag / white [P0, nbins, dx, dy] for the positions with ``points[p] == 0`` (in order),
         sums [P, n_energies] (float64 sums of the reference beam, see paresis_rt_job.means)."""
         s = scene
+        if self.scatters(s):
+            raise NotImplementedError("scattering (dark-field) samples run position by position: compute_rt, or the "
+                                      "energy-sharded call")
         n_pos = len(offsets)
         bins = self.bins(s)
         nbins, n_e = len(s.thresholds), len(s.spectrum)
@@ -476,13 +577,19 @@ class ImageFormation:
         return out
 
     @_on_own_device
-    def accumulate_rt(self, scene, point_num, indices):
+    def accumulate_rt(self, scene, point_num, indices, dark_field=None):
         """The energies ``indices`` (all of ONE detector bin) of a position, without the detector:
         leaves the partial sums in ``self.acc`` and returns the per-energy means of the reference
         beam (device float64 tensor, len(indices)).  Used when a bin's energies are spread over
-        several GPUs (shard.py)."""
+        several GPUs (shard.py).  ``dark_field``: [nx, ny] float32 tensor that a scattering sample at
+        position 0 adds these energies' share of compute_rt's ``dark_field`` to."""
         first = point_num == 0
         energies, keep = self._rt_energies(scene, list(indices), closing=set())
+        if self.scatters(scene):
+            job, keep2 = self._rt_job(scene, energies, first, 0, group=False)
+            dj, keep3 = self._df_job(scene, job, list(indices), dark_field if first else None)
+            self._run_df(dj, self._df_launches(len(indices), 0, first))
+            return self.means[:len(indices)] / float(self.nx * self.ny)
         job, keep2 = self._rt_job(scene, energies, first, 0)
         dummy = torch.empty(1, device=self.device, dtype=torch.float32)
         job.out_sample = job.out_ref = job.out_propag = job.out_white = dummy.data_ptr()

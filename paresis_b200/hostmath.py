@@ -59,3 +59,15 @@ def refraction_gradient_scale(distance, magnification, pixel_um):
     (Sample.py:348, refractionFileNumba2.py:54-56); k cancels."""
     h = pixel_um * 1e-6
     return -distance / (h * magnification) / (2.0 * h)
+
+
+# dark-field models: sphere radius (um), volume fraction (Sample.py:325-326, :336-337)
+MODELS = {"Lung": (47.0, 0.5), "cylinder_beeds": (15.0, 0.6)}
+
+
+def angle_coefficient(delta, scatter):
+    """newDf = coeff * sqrt(thickness[m]) in radians (Sample.py:328-332, :339-343) for a material of refractive decrement
+    ``delta`` and ``scatter`` = (sphere radius um, volume fraction), a value of MODELS."""
+    radius, fraction = scatter
+    n_vol = fraction * 3 / 4 / np.pi / (radius ** 3)
+    return 2 * delta * np.sqrt(n_vol ** (1 / 3) * 1e6) * np.sqrt(np.log(2 / delta) + 1)

@@ -78,11 +78,19 @@ def compute_rt_energy_sharded(engine, scene, point_num, owner=0, group=None, seq
     ``reduce_events``: a list that receives one (start, end) CUDA event pair per NCCL reduction (bench.py).
     ``defer=True``: return a ``ShardedPosition`` instead, without waiting for the device: the caller queues the next
     position first and calls ``finish()`` on this one afterwards (every rank, same order), so the host's turn-around and
-    the device->host read of the means overlap the next position's kernels."""
+    the device->host read of the means overlap the next position's kernels.
+    A scattering sample at position 0 also gives ``dark_field`` on the owner: each rank adds its energies' share and
+    the shares are summed with one more reduction."""
     def white(energy, flux):   # Experiment.py:490-497
         return scene.mean_shot_count / scene.os ** 2 * flux * scene.common_factor(energy) * scene.plate_factor(energy)
-    return _energy_sharded(engine.accumulate_rt, white, engine, scene, point_num, owner, group, sequence_base, reduce_events,
-                           defer)
+    dark = None
+    if point_num == 0 and engine.scatters(scene):
+        dark = torch.zeros((engine.nx, engine.ny), device=engine.device, dtype=torch.float32)
+
+    def accumulate(sc, point, indices):
+        return engine.accumulate_rt(sc, point, indices, dark_field=dark)
+    return _energy_sharded(accumulate, white, engine, scene, point_num, owner, group, sequence_base, reduce_events,
+                           defer, dark)
 
 
 def compute_fresnel_energy_sharded(engine, scene, point_num, owner=0, group=None, sequence_base=0, reduce_events=None,
@@ -95,10 +103,12 @@ def compute_fresnel_energy_sharded(engine, scene, point_num, owner=0, group=None
                            reduce_events, defer)
 
 
-def _energy_sharded(accumulate, white_of, engine, scene, point_num, owner, group, sequence_base, reduce_events, defer):
+def _energy_sharded(accumulate, white_of, engine, scene, point_num, owner, group, sequence_base, reduce_events, defer,
+                    dark_field=None):
     """Body of the energy-sharded calls.  ``accumulate(scene, point_num, indices)``: the model's partial sums of some
     energies of one bin into ``engine.acc``, returning their per-energy reference means; ``white_of(energy, flux)``: one
-    energy's share of the white field."""
+    energy's share of the white field.  ``dark_field``: this rank's share of the dark-field map, which ``accumulate``
+    adds to; it is summed onto the owner and returned there."""
     rank = dist.get_rank(group) if dist.is_initialized() else 0
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     first = point_num == 0
@@ -137,6 +147,10 @@ def _energy_sharded(accumulate, white_of, engine, scene, point_num, owner, group
                     abi.poisson(partial[k], out[name][b], engine.seed, seq + k)
                 else:
                     out[name][b].copy_(partial[k])
+    if dark_field is not None:
+        reduce_images(dark_field, owner, group)
+        if rank == owner:
+            out["dark_field"] = dark_field
     # the reference's NaN / "insane values" guard (refractionFileNumba2.py:81-82) must fire whichever rank saw the bad
     # value: the status flags travel with the means (one all_reduce), every rank clears its own and every rank raises
     tail = torch.cat((means, engine.flag.to(torch.float64)))
