@@ -404,6 +404,32 @@ typedef struct {
  * checked before the first CUDA call (PARESIS_ERR_ARG). */
 int paresis_fresnel_run(const paresis_fresnel_job* job_host, paresis_stream stream);
 
+/* Many membrane positions of the Fresnel model in ONE call, as paresis_rt_run_positions does for ray tracing: for each
+ * position, its membrane map is cut from the sphere field (paresis_membrane_from_field) or, without a field, rasterised
+ * (paresis_raster_spheres) into position.thickness; then the launch sequence of paresis_fresnel_run runs on the slot's
+ * stream with the slot's plan and buffers and the position's outputs, means and sequence.  Position p goes to slot
+ * p mod n_slots, so that consecutive positions overlap on the GPU.  `stream` is the caller's stream: every slot stream
+ * first waits for it, and it waits for every slot stream at the end.
+ *
+ * `job_host` is the template of paresis_fresnel_run: its plan, wave, accumulator, detect_work, output, means, sequence
+ * and first_point fields are ignored (they come from the slot and the position).  A membrane layer whose `thickness` is
+ * NULL stands for "the membrane map of this position"; a NULL sample map is an error.  Positions take no probe events.
+ * Every argument is checked before the first CUDA call (PARESIS_ERR_ARG); n_positions == 0 does nothing. */
+typedef struct {
+    paresis_fresnel_plan* plan;                 /* this slot's OWN plan (a plan owns its work buffers): the size of every
+                                                   transfer kernel of the job; no two slots may share one */
+    paresis_c32* wave_a; paresis_c32* wave_b;   /* [nx][ny] scratch */
+    float* acc_sample; float* acc_ref; float* acc_propag; float* acc_white;   /* [nx][ny], any content */
+    float* detect_work;                         /* per slot (slots run concurrently); may be NULL as in paresis_fresnel_job */
+    void* raster_work; size_t raster_work_bytes;   /* needed only when the membrane has no sphere field: at least
+                                                      paresis_raster_work_bytes(n_spheres, n_layers, nx, ny) */
+    paresis_stream stream;
+} paresis_fresnel_slot;
+
+int paresis_fresnel_run_positions(const paresis_fresnel_job* job_host, const paresis_membrane* membrane_host,
+                                  const paresis_rt_position* positions_host, int n_positions,
+                                  paresis_fresnel_slot* slots_host, int n_slots, paresis_stream stream);
+
 /* ---------------------------------------------------------------------------------------
  * Detector
  * ------------------------------------------------------------------------------------- */

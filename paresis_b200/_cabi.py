@@ -26,7 +26,7 @@ EXPORTS = (
     "paresis_version", "paresis_last_error", "paresis_set_tuning", "paresis_trim", "paresis_splat", "paresis_refract_phi", "paresis_refract_layers",
     "paresis_transmit_rt", "paresis_transmit_wave", "paresis_mix_maps", "paresis_fresnel_plan_create", "paresis_fresnel_plan_destroy",
     "paresis_fresnel_plan_bytes", "paresis_fresnel_propagate", "paresis_fresnel_kernel_create", "paresis_fresnel_kernel_destroy",
-    "paresis_fresnel_convolve", "paresis_fresnel_spectrum", "paresis_fresnel_from_spectrum", "paresis_fresnel_run", "paresis_df_run", "paresis_detect_work_floats", "paresis_detect",
+    "paresis_fresnel_convolve", "paresis_fresnel_spectrum", "paresis_fresnel_from_spectrum", "paresis_fresnel_run", "paresis_fresnel_run_positions", "paresis_df_run", "paresis_detect_work_floats", "paresis_detect",
     "paresis_detect_counts", "paresis_detect_counts_multi",
     "paresis_poisson", "paresis_bin_sum", "paresis_raster_work_bytes", "paresis_raster_spheres", "paresis_sphere_map", "paresis_cylinder_map",
     "paresis_fill", "paresis_axpy", "paresis_mean", "paresis_sum_scaled", "paresis_rt_run", "paresis_rt_run_positions",
@@ -144,6 +144,13 @@ class FresnelJob(ctypes.Structure):
                 ("out_white", ctypes.c_void_p)]
 
 
+class FresnelSlot(ctypes.Structure):
+    _fields_ = [("plan", ctypes.c_void_p), ("wave_a", ctypes.c_void_p), ("wave_b", ctypes.c_void_p),
+                ("acc_sample", ctypes.c_void_p), ("acc_ref", ctypes.c_void_p), ("acc_propag", ctypes.c_void_p),
+                ("acc_white", ctypes.c_void_p), ("detect_work", ctypes.c_void_p), ("raster_work", ctypes.c_void_p),
+                ("raster_work_bytes", ctypes.c_size_t), ("stream", ctypes.c_void_p)]
+
+
 def _load():
     if not os.path.exists(LIB_PATH):
         raise ImportError(
@@ -173,6 +180,8 @@ def _load():
         "paresis_fresnel_spectrum": [vp, vp, vp],
         "paresis_fresnel_from_spectrum": [vp, vp, vp, C32, vp, vp, vp],
         "paresis_fresnel_run": [ctypes.POINTER(FresnelJob), vp],
+        "paresis_fresnel_run_positions": [ctypes.POINTER(FresnelJob), ctypes.POINTER(Membrane), ctypes.POINTER(RtPosition), ci,
+                                          ctypes.POINTER(FresnelSlot), ci, vp],
         "paresis_detect": [vp, ci, ci, ci, ci, ci, vp, ci, vp, ci, vp, vp, vp],
         "paresis_detect_counts": [vp, ci, ci, ci, ci, ci, vp, ci, vp, ci, vp, vp, ci, u64, u64, vp],
         "paresis_detect_counts_multi": [ctypes.POINTER(vp), ctypes.POINTER(vp), ctypes.POINTER(u64), ci, ci, ci, ci, ci, ci, vp, ci,
@@ -274,6 +283,13 @@ def rt_run(job, launches_in_job, probe=None):
 def fresnel_run(job, launches_in_job):
     """paresis_fresnel_run: one membrane position of the Fresnel model (a FresnelJob)."""
     _check(lib.paresis_fresnel_run(ctypes.byref(job), _stream()), "paresis_fresnel_run")
+    _count(launches_in_job)
+
+
+def fresnel_run_positions(job, membrane, positions, slots, launches_in_job):
+    """paresis_fresnel_run_positions: `positions` / `slots` are ctypes arrays of RtPosition / FresnelSlot."""
+    _check(lib.paresis_fresnel_run_positions(ctypes.byref(job), ctypes.byref(membrane), positions, len(positions), slots,
+                                             len(slots), _stream()), "paresis_fresnel_run_positions")
     _count(launches_in_job)
 
 

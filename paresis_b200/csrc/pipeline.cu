@@ -13,6 +13,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "positions.cuh"
 
 using namespace paresis;
 
@@ -164,24 +165,6 @@ extern "C" int paresis_rt_run(const paresis_rt_job* job, paresis_stream stream) 
     return PARESIS_OK;
 }
 
-namespace {
-// fork / join events of the slot streams, created once per process
-struct SlotEvents {
-    cudaEvent_t fork = nullptr;
-    std::vector<cudaEvent_t> join;
-    int ensure(int n) {
-        if (!fork) PARESIS_CUDA(cudaEventCreateWithFlags(&fork, cudaEventDisableTiming));
-        while ((int)join.size() < n) {
-            cudaEvent_t e;
-            PARESIS_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
-            join.push_back(e);
-        }
-        return PARESIS_OK;
-    }
-};
-SlotEvents g_events_of[32];     // CUDA events belong to a device
-}  // namespace
-
 // ---------------------------------------------------------------------------------------------------------------
 // Several positions per launch.  A position at 2048^2 is 18 pixels per resident thread: ramp, tail and per-block set-up
 // of its kernels cannot be amortised inside one position (DESIGN.md, "What bounds the hops").  Here the membrane cut,
@@ -329,15 +312,14 @@ extern "C" int paresis_rt_run_positions(const paresis_rt_job* job, const paresis
     if (n_positions == 0) return PARESIS_OK;
     if (job->positions_per_launch > 1 && mem->field && !job->i_bs_group[0] && single_energy_bins(job))
         return run_positions_batched(job, mem, positions, n_positions, slots, n_slots, stream);
-    int dev = 0;
-    PARESIS_CUDA(cudaGetDevice(&dev));
-    SlotEvents& g_events = g_events_of[(dev < 0 || dev >= 32) ? 0 : dev];
-    int rc = g_events.ensure(n_slots);
+    SlotEvents* events = nullptr;
+    int rc = slot_events(n_slots, &events);
     if (rc) return rc;
+    SlotEvents& g_events = *events;
     cudaStream_t main_stream = (cudaStream_t)stream;
     const int used = n_slots < n_positions ? n_slots : n_positions;
-    PARESIS_CUDA(cudaEventRecord(g_events.fork, main_stream));
-    for (int k = 0; k < used; ++k) PARESIS_CUDA(cudaStreamWaitEvent((cudaStream_t)slots[k].stream, g_events.fork, 0));
+    rc = fork_slots(g_events, main_stream, slots, used);
+    if (rc) return rc;
 
     std::vector<paresis_rt_energy> energies(job->energies_host, job->energies_host + job->n_energies);
     for (int p = 0; p < n_positions; ++p) {
@@ -359,12 +341,8 @@ extern "C" int paresis_rt_run_positions(const paresis_rt_job* job, const paresis
         }
         const bool probe_raster = job->probe == 4 && pos.probe_start && pos.probe_end;
         if (probe_raster) cudaEventRecord((cudaEvent_t)pos.probe_start, (cudaStream_t)slot.stream);
-        if (mem->field)
-            rc = paresis_membrane_from_field(mem->field, mem->field_x, mem->field_y, pos.offsets_host, mem->n_layers, mem->margin,
-                                             job->nx, job->ny, pos.thickness, slot.stream);
-        else
-            rc = paresis_raster_spheres(mem->spheres, mem->n_spheres, mem->pix_um, pos.offsets_host, mem->n_layers, job->nx,
-                                        job->ny, mem->margin, pos.thickness, slot.raster_work, slot.raster_work_bytes, slot.stream);
+        rc = membrane_of_position(mem, pos.offsets_host, job->nx, job->ny, pos.thickness, slot.raster_work, slot.raster_work_bytes,
+                                  slot.stream);
         if (probe_raster) cudaEventRecord((cudaEvent_t)pos.probe_end, (cudaStream_t)slot.stream);
         if (rc) return rc;
         // a NULL layer map stands for this position's membrane
@@ -400,9 +378,5 @@ extern "C" int paresis_rt_run_positions(const paresis_rt_job* job, const paresis
                 if (&slots[k] != &slot) PARESIS_CUDA(cudaStreamWaitEvent((cudaStream_t)slots[k].stream, g_events.fork, 0));
         }
     }
-    for (int k = 0; k < used; ++k) {
-        PARESIS_CUDA(cudaEventRecord(g_events.join[k], (cudaStream_t)slots[k].stream));
-        PARESIS_CUDA(cudaStreamWaitEvent(main_stream, g_events.join[k], 0));
-    }
-    return PARESIS_OK;
+    return join_slots(g_events, main_stream, slots, used);
 }

@@ -477,8 +477,9 @@ class ImageFormation:
         self._i_bs_dirty = False
 
     # ------------------------------------------------------------------ many positions, one call
-    def _slots(self, n_slots, raster_bytes):
-        """Scratch sets of paresis_rt_run_positions: slot 0 is this engine's own buffers."""
+    def _slots(self, n_slots, raster_bytes, fresnel=False):
+        """Scratch sets of paresis_rt_run_positions / paresis_fresnel_run_positions: slot 0 is this engine's own buffers.
+        ``fresnel``: each slot also gets a Fresnel plan, two waves and detector work of its own (slots run concurrently)."""
         f32 = dict(device=self.device, dtype=torch.float32)
         cache = self.__dict__.setdefault("_slot_cache", [])
         while len(cache) < n_slots:
@@ -490,7 +491,57 @@ class ImageFormation:
         for c in cache[:n_slots]:
             if c["work"] is None or c["work"].numel() < raster_bytes:
                 c["work"] = torch.empty(raster_bytes, device=self.device, dtype=torch.uint8)
+        if fresnel:
+            self._fresnel_setup()
+            for k, c in enumerate(cache[:n_slots]):
+                if "plan" not in c:
+                    c["plan"] = self._plan if k == 0 else abi.FresnelPlan(self.nx, self.ny, 15)
+                    c["waves"] = self._waves if k == 0 else [torch.empty_like(w) for w in self._waves]
+                    c["detect_work"] = self.work if k == 0 else torch.empty_like(self.work)
         return cache[:n_slots]
+
+    def _positions_buffers(self, n_pos, n_firsts, nbins, n_e):
+        """Outputs of a many-positions call: thickness maps, images [P, 2, nbins, dx, dy], the extra images of position 0,
+        the per-energy sums."""
+        f32 = dict(device=self.device, dtype=torch.float32)
+        return dict(thickness=torch.empty((n_pos, self.nx, self.ny), **f32),
+                    images=torch.empty((n_pos, 2, nbins, self.det_x, self.det_y), **f32),
+                    extra=torch.empty((max(n_firsts, 1), 2, nbins, self.det_x, self.det_y), **f32),
+                    sums=torch.zeros((n_pos, n_e), device=self.device, dtype=torch.float64))
+
+    @staticmethod
+    def _membrane(plan):
+        """paresis_membrane of a geometry.MembranePlan (its sphere field when it has one) -> (struct, field or None)."""
+        field = plan.field()
+        membrane = abi.Membrane(plan.table.data_ptr(), plan.table.shape[0], plan.pix, plan.layers, plan.margin,
+                                field.data_ptr() if field is not None else None,
+                                field.shape[0] if field is not None else 0, field.shape[1] if field is not None else 0)
+        return membrane, field
+
+    def _c_positions(self, buffers, offsets, points, firsts, layers, sequence_base, want_means):
+        """ctypes array of paresis_rt_position, with the offsets array it points to."""
+        n_pos = len(offsets)
+        offs = np.ascontiguousarray(np.asarray(offsets, dtype=np.int64).reshape(n_pos, layers, 2))
+        c_pos = (abi.RtPosition * n_pos)()
+        for p in range(n_pos):
+            cp = c_pos[p]
+            cp.offsets_host = offs[p].ctypes.data_as(abi.ctypes.POINTER(abi.ctypes.c_int64))
+            cp.thickness = buffers["thickness"][p].data_ptr()
+            cp.out_sample, cp.out_ref = buffers["images"][p, 0].data_ptr(), buffers["images"][p, 1].data_ptr()
+            first = points[p] == 0
+            if first:
+                k = firsts.index(p)
+                cp.out_propag, cp.out_white = buffers["extra"][k, 0].data_ptr(), buffers["extra"][k, 1].data_ptr()
+            cp.means = buffers["sums"][p].data_ptr() if want_means else None
+            cp.sequence = self.sequence(points[p], sequence_base)
+            cp.first_point = 1 if first else 0
+        return c_pos, offs
+
+    @staticmethod
+    def _positions_result(buffers, firsts):
+        return dict(thickness=buffers["thickness"], sample=buffers["images"][:, 0], reference=buffers["images"][:, 1],
+                    propag=buffers["extra"][:len(firsts), 0], white=buffers["extra"][:len(firsts), 1], sums=buffers["sums"],
+                    firsts=firsts, buffers=buffers)
 
     @_on_own_device
     def compute_rt_positions(self, scene, plan, offsets, points, sequence_base=0, n_slots=2, probe_label=None,
@@ -519,17 +570,9 @@ class ImageFormation:
         job, keep2 = self._rt_job(s, energies, False, 0)
         job.positions_per_launch = int(per_launch)
         firsts = [p for p in range(n_pos) if points[p] == 0]
-        f32 = dict(device=self.device, dtype=torch.float32)
         if buffers is None:
-            buffers = dict(
-                thickness=torch.empty((n_pos, self.nx, self.ny), **f32),
-                images=torch.empty((n_pos, 2, nbins, self.det_x, self.det_y), **f32),
-                extra=torch.empty((max(len(firsts), 1), 2, nbins, self.det_x, self.det_y), **f32),
-                sums=torch.zeros((n_pos, n_e), device=self.device, dtype=torch.float64))
-        field = plan.field()
-        membrane = abi.Membrane(plan.table.data_ptr(), plan.table.shape[0], plan.pix, plan.layers, plan.margin,
-                                field.data_ptr() if field is not None else None,
-                                field.shape[0] if field is not None else 0, field.shape[1] if field is not None else 0)
+            buffers = self._positions_buffers(n_pos, len(firsts), nbins, n_e)
+        membrane, field = self._membrane(plan)
         raster_bytes = abi.lib.paresis_raster_work_bytes(plan.table.shape[0], plan.layers, self.nx, self.ny)
         slots = self._slots(n_slots, raster_bytes)
         c_slots = (abi.RtSlot * n_slots)()
@@ -545,21 +588,11 @@ class ImageFormation:
                 sl.i_bs_group[kk] = t.data_ptr()
             c["dirty"] = True
         self._i_bs_dirty = True
-        offs = np.ascontiguousarray(np.asarray(offsets, dtype=np.int64).reshape(n_pos, plan.layers, 2))
-        c_pos = (abi.RtPosition * n_pos)()
+        c_pos, offs = self._c_positions(buffers, offsets, points, firsts, plan.layers, sequence_base, want_means)
         launches = 0
         for p in range(n_pos):
             cp = c_pos[p]
-            cp.offsets_host = offs[p].ctypes.data_as(abi.ctypes.POINTER(abi.ctypes.c_int64))
-            cp.thickness = buffers["thickness"][p].data_ptr()
-            cp.out_sample, cp.out_ref = buffers["images"][p, 0].data_ptr(), buffers["images"][p, 1].data_ptr()
             first = points[p] == 0
-            if first:
-                k = firsts.index(p)
-                cp.out_propag, cp.out_white = buffers["extra"][k, 0].data_ptr(), buffers["extra"][k, 1].data_ptr()
-            cp.means = buffers["sums"][p].data_ptr() if want_means else None
-            cp.sequence = self.sequence(points[p], sequence_base)
-            cp.first_point = 1 if first else 0
             if probe_events is not None and probe_events[p] is not None:
                 e0, e1 = probe_events[p]
                 for e in (e0, e1):
@@ -571,10 +604,7 @@ class ImageFormation:
         for c in slots:
             c["dirty"] = False
         self._i_bs_dirty = False
-        out = dict(thickness=buffers["thickness"], sample=buffers["images"][:, 0], reference=buffers["images"][:, 1],
-                   propag=buffers["extra"][:len(firsts), 0], white=buffers["extra"][:len(firsts), 1], sums=buffers["sums"],
-                   firsts=firsts, buffers=buffers)
-        return out
+        return self._positions_result(buffers, firsts)
 
     @_on_own_device
     def accumulate_rt(self, scene, point_num, indices, dark_field=None):
@@ -653,7 +683,9 @@ class ImageFormation:
             en.white = amp * amp
             membrane = (abi.WaveLayer * len(mem_maps))()
             for dst, (t, d, b) in zip(membrane, mem_maps):
-                dst.thickness, dst.atten, dst.phase = t.data_ptr(), k * b, k * d
+                # a NULL map = the membrane of the position at hand (paresis_fresnel_run_positions)
+                dst.thickness = None if t is PER_POSITION else t.data_ptr()
+                dst.atten, dst.phase = k * b, k * d
             en.membrane_host, en.n_membrane = membrane, len(mem_maps)
             for dst, (t, d, b) in zip(en.sample, smp_maps):
                 dst.thickness, dst.atten, dst.phase = t.data_ptr(), k * b, k * d
@@ -666,7 +698,7 @@ class ImageFormation:
                 setattr(en, name, kern._h)
                 setattr(en, "phase_" + name, abi.C32(float(np.real(phase)), float(np.imag(phase))))
             en.close_bin = 1 if ie in closing else 0
-            keep += [membrane] + [t for t, _, _ in mem_maps + smp_maps]
+            keep += [membrane] + [t for t, _, _ in mem_maps + smp_maps if t is not PER_POSITION]
         return energies, keep
 
     def _fresnel_job(self, scene, energies, first, sequence):
@@ -712,6 +744,47 @@ class ImageFormation:
         abi.fresnel_run(job, self._fresnel_launches(n_e, len(closing), first))
         out["mean_energy"] = self._mean_energy([e for e, _ in s.spectrum], sums=self.means[:n_e].cpu().numpy())
         return out
+
+    @_on_own_device
+    def compute_fresnel_positions(self, scene, plan, offsets, points, sequence_base=0, n_slots=2, want_means=True,
+                                  buffers=None):
+        """``len(offsets)`` membrane positions of the Fresnel model in one library call (paresis_fresnel_run_positions): per
+        position the membrane is cut from ``plan`` (geometry.MembranePlan) at ``offsets[p]`` and the Fresnel chain of
+        compute_fresnel runs, positions alternating between ``n_slots`` streams, each with a plan and buffers of its own.
+        No host synchronisation.
+
+        ``scene.membrane`` must hold one ``Layer(PER_POSITION, ...)`` for the position's map.  Arguments and result as
+        compute_rt_positions: thickness [P, N, N], sample / reference [P, nbins, dx, dy], propag / white
+        [P0, nbins, dx, dy] for the positions with ``points[p] == 0`` (in order), sums [P, n_energies] (float64 sums of
+        the reference beam, see paresis_fresnel_job.means), firsts, buffers."""
+        s = scene
+        n_pos = len(offsets)
+        bins = self.bins(s)
+        nbins, n_e = len(s.thresholds), len(s.spectrum)
+        closing = {b[-1] for b in bins[:nbins]}
+        energies, keep = self._fresnel_energies(s, list(range(n_e)), closing)
+        job, keep2 = self._fresnel_job(s, energies, False, 0)
+        firsts = [p for p in range(n_pos) if points[p] == 0]
+        if buffers is None:
+            buffers = self._positions_buffers(n_pos, len(firsts), nbins, n_e)
+        membrane, field = self._membrane(plan)
+        raster_bytes = abi.lib.paresis_raster_work_bytes(plan.table.shape[0], plan.layers, self.nx, self.ny)
+        slots = self._slots(n_slots, raster_bytes, fresnel=True)
+        c_slots = (abi.FresnelSlot * n_slots)()
+        for k, c in enumerate(slots):
+            sl = c_slots[k]
+            sl.plan = c["plan"]._h
+            sl.wave_a, sl.wave_b = c["waves"][0].data_ptr(), c["waves"][1].data_ptr()
+            sl.acc_sample, sl.acc_ref = c["acc"]["sample"].data_ptr(), c["acc"]["reference"].data_ptr()
+            sl.acc_propag, sl.acc_white = c["acc"]["propag"].data_ptr(), c["acc"]["white"].data_ptr()
+            sl.detect_work = c["detect_work"].data_ptr()
+            sl.raster_work, sl.raster_work_bytes = c["work"].data_ptr(), c["work"].numel()
+            sl.stream = c["stream"].cuda_stream
+        c_pos, offs = self._c_positions(buffers, offsets, points, firsts, plan.layers, sequence_base, want_means)
+        cut = 1 if field is not None else 2
+        launches = sum(cut + self._fresnel_launches(n_e, len(closing), points[p] == 0) for p in range(n_pos))
+        abi.fresnel_run_positions(job, membrane, c_pos, c_slots, launches)
+        return self._positions_result(buffers, firsts)
 
     @_on_own_device
     def accumulate_fresnel(self, scene, point_num, indices):
