@@ -585,6 +585,39 @@ typedef struct {
 
 int paresis_df_run(const paresis_df_job* job_host, paresis_stream stream);
 
+/* Many membrane positions of a scattering sample in ONE call, as paresis_rt_run_positions does for a plain sample: for
+ * each position, its membrane map is cut from the sphere field (paresis_membrane_from_field) or, without a field,
+ * rasterised (paresis_raster_spheres) into position.rt.thickness; then the launch sequence of paresis_df_run runs on the
+ * slot's stream with the slot's buffers and the position's outputs, means, sequence and dark-field map.  Position p goes
+ * to slot p mod n_slots, so that consecutive positions overlap on the GPU.  `stream` is the caller's stream: every slot
+ * stream first waits for it, and it waits for every slot stream at the end.  With more than one position the hops use
+ * full-height tiles (paresis_rt_job.throughput = 1), as in paresis_rt_run_positions.
+ *
+ * `job_host` is the template of paresis_df_run: its i_bs, accumulator, detect_work, output, means, sequence, first_point,
+ * scratch and dark_field fields are ignored (they come from the slot and the position).  A hop1 or hop2 layer whose
+ * `thickness` is NULL stands for "the membrane map of this position"; a NULL propag or scattering map is an error.
+ * Positions take no probe events.  Every argument is checked before the first CUDA call (PARESIS_ERR_ARG), including that
+ * no image buffer belongs to two slots; n_positions == 0 does nothing. */
+typedef struct {
+    float* i_bs; float* acc_sample; float* acc_ref; float* acc_propag; float* acc_white;   /* as in paresis_rt_job */
+    float* angle; float* plain; float* scattered; float* clean; float* moved;             /* as in paresis_df_job */
+    float* detect_work;                    /* as paresis_rt_job.detect_work, this slot's own (slots run concurrently); may
+                                              be NULL for ordinary kernel sizes */
+    void* raster_work; size_t raster_work_bytes;   /* needed only when the membrane has no sphere field: at least
+                                                      paresis_raster_work_bytes(n_spheres, n_layers, nx, ny) */
+    paresis_stream stream;
+    int i_bs_dirty;                        /* in/out, as paresis_rt_slot: cleared once the slot has run a position */
+} paresis_df_slot;
+
+typedef struct {
+    paresis_rt_position rt;                /* probe events must be NULL */
+    float* dark_field;                     /* optional [nx][ny], first_point only: += as paresis_df_job.dark_field */
+} paresis_df_position;
+
+int paresis_df_run_positions(const paresis_df_job* job_host, const paresis_membrane* membrane_host,
+                             const paresis_df_position* positions_host, int n_positions,
+                             paresis_df_slot* slots_host, int n_slots, paresis_stream stream);
+
 /* Result transfers (the reference hands back host arrays: Experiment.py:405, :526, main.py:99): an
  * asynchronous device -> pinned-host copy on the library's copy stream, ordered after `producer`.
  * A lane holds the events of one copy in flight; reuse it once paresis_transfer_wait returned. */

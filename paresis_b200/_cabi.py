@@ -26,7 +26,7 @@ EXPORTS = (
     "paresis_version", "paresis_last_error", "paresis_set_tuning", "paresis_trim", "paresis_splat", "paresis_refract_phi", "paresis_refract_layers",
     "paresis_transmit_rt", "paresis_transmit_wave", "paresis_mix_maps", "paresis_fresnel_plan_create", "paresis_fresnel_plan_destroy",
     "paresis_fresnel_plan_bytes", "paresis_fresnel_propagate", "paresis_fresnel_kernel_create", "paresis_fresnel_kernel_destroy",
-    "paresis_fresnel_convolve", "paresis_fresnel_spectrum", "paresis_fresnel_from_spectrum", "paresis_fresnel_run", "paresis_fresnel_run_positions", "paresis_df_run", "paresis_detect_work_floats", "paresis_detect",
+    "paresis_fresnel_convolve", "paresis_fresnel_spectrum", "paresis_fresnel_from_spectrum", "paresis_fresnel_run", "paresis_fresnel_run_positions", "paresis_df_run", "paresis_df_run_positions", "paresis_detect_work_floats", "paresis_detect",
     "paresis_detect_counts", "paresis_detect_counts_multi",
     "paresis_poisson", "paresis_bin_sum", "paresis_raster_work_bytes", "paresis_raster_spheres", "paresis_sphere_map", "paresis_cylinder_map",
     "paresis_fill", "paresis_axpy", "paresis_mean", "paresis_sum_scaled", "paresis_rt_run", "paresis_rt_run_positions",
@@ -96,6 +96,18 @@ class RtSlot(ctypes.Structure):
                 ("acc_propag", ctypes.c_void_p), ("acc_white", ctypes.c_void_p), ("raster_work", ctypes.c_void_p),
                 ("raster_work_bytes", ctypes.c_size_t), ("stream", ctypes.c_void_p), ("i_bs_dirty", ctypes.c_int),
                 ("i_bs_group", ctypes.c_void_p * (MAX_GROUP - 1))]
+
+
+class DfSlot(ctypes.Structure):
+    _fields_ = [("i_bs", ctypes.c_void_p), ("acc_sample", ctypes.c_void_p), ("acc_ref", ctypes.c_void_p),
+                ("acc_propag", ctypes.c_void_p), ("acc_white", ctypes.c_void_p), ("angle", ctypes.c_void_p),
+                ("plain", ctypes.c_void_p), ("scattered", ctypes.c_void_p), ("clean", ctypes.c_void_p), ("moved", ctypes.c_void_p),
+                ("detect_work", ctypes.c_void_p), ("raster_work", ctypes.c_void_p), ("raster_work_bytes", ctypes.c_size_t),
+                ("stream", ctypes.c_void_p), ("i_bs_dirty", ctypes.c_int)]
+
+
+class DfPosition(ctypes.Structure):
+    _fields_ = [("rt", RtPosition), ("dark_field", ctypes.c_void_p)]
 
 
 class Membrane(ctypes.Structure):
@@ -199,6 +211,8 @@ def _load():
         "paresis_sum_scaled": [vp, sz, cd, vp, vp],
         "paresis_rt_run": [ctypes.POINTER(RtJob), vp],
         "paresis_df_run": [ctypes.POINTER(DfJob), vp],
+        "paresis_df_run_positions": [ctypes.POINTER(DfJob), ctypes.POINTER(Membrane), ctypes.POINTER(DfPosition), ci,
+                                     ctypes.POINTER(DfSlot), ci, vp],
         "paresis_two_sphere_phantom": [ci, ci, ci, cd, vp, vp],
         "paresis_df_angle": [vp, cd, vp, sz, vp],
         "paresis_df_split": [vp, cf, vp, cf, vp, vp, vp, sz, vp],
@@ -296,6 +310,13 @@ def fresnel_run_positions(job, membrane, positions, slots, launches_in_job):
 def df_run(job, launches_in_job):
     """paresis_df_run: one membrane position of the ray-tracing model with a scattering sample (a DfJob)."""
     _check(lib.paresis_df_run(ctypes.byref(job), _stream()), "paresis_df_run")
+    _count(launches_in_job)
+
+
+def df_run_positions(job, membrane, positions, slots, launches_in_job):
+    """paresis_df_run_positions: `positions` / `slots` are ctypes arrays of DfPosition / DfSlot."""
+    _check(lib.paresis_df_run_positions(ctypes.byref(job), ctypes.byref(membrane), positions, len(positions), slots,
+                                        len(slots), _stream()), "paresis_df_run_positions")
     _count(launches_in_job)
 
 

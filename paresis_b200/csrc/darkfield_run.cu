@@ -9,7 +9,16 @@
 // The object hop runs as two dual-beam hops, one on the plain rays and one on the scattered rays.  The splat is linear
 // in intensity, so their two reference deposits add up to the reference beam of the whole object-plane image, and each
 // energy's reference sum comes out of the hops (sum_ref) with no reduction pass.
+//
+// paresis_df_run_positions runs the same launch sequence for many membrane positions of a scan (main.py:63-110) in one
+// call, the positions dealt over slots that each own an object-plane buffer, accumulators and dark-field scratch and run
+// on their own stream, so that consecutive positions overlap on the GPU.
+#include <cuda_runtime.h>
+
+#include <vector>
+
 #include "common.cuh"
+#include "positions.cuh"
 
 using namespace paresis;
 
@@ -17,63 +26,70 @@ namespace {
 
 constexpr int kMargin = 15;   // refractionFileNumba2.py:50
 
-int bad(const char* what, int e) {
-    set_last_error("paresis_df_run: energy %d: %s", e, what);
+int bad(const char* who, const char* what, int e) {
+    set_last_error("%s: energy %d: %s", who, e, what);
     return PARESIS_ERR_ARG;
 }
 
-// every check that reads host memory only: nothing is launched before the whole job is known to be well formed
-int check_job(const paresis_df_job* job) {
-    if (!job) { set_last_error("paresis_df_run: null job"); return PARESIS_ERR_ARG; }
+// The per-energy checks of a job (host memory only).  `first`: the sample-only hop runs too (position 0).
+// `position_maps`: a NULL map of the membrane or object hop stands for the membrane of the position at hand
+// (paresis_df_run_positions); a NULL sample-only or scattering map is always an error.
+int check_energies(const char* who, const paresis_df_job* job, bool first, bool position_maps) {
     const paresis_rt_job& r = job->rt;
-    if (!r.energies_host || !job->energies_df_host || r.n_energies < 1) {
-        set_last_error("paresis_df_run: no energies");
-        return PARESIS_ERR_ARG;
-    }
-    if (r.nx < 3 || r.ny < 3) { set_last_error("paresis_df_run: bad frame %d x %d", r.nx, r.ny); return PARESIS_ERR_ARG; }
-    if (!r.i_bs || !r.acc_sample || !r.acc_ref || (r.first_point && !r.acc_propag)) {
-        set_last_error("paresis_df_run: null object-plane buffer or accumulator");
-        return PARESIS_ERR_ARG;
-    }
-    if (!job->angle || !job->plain || !job->scattered || !job->clean || !job->moved) {
-        set_last_error("paresis_df_run: null dark-field scratch buffer");
-        return PARESIS_ERR_ARG;
-    }
-    const bool detect = r.out_sample || r.out_ref || r.out_propag || r.out_white;
-    if (detect && (!r.out_sample || !r.out_ref || (r.first_point && (!r.out_propag || !r.out_white || !r.acc_white)))) {
-        set_last_error("paresis_df_run: incomplete detector outputs (all of them, or none to accumulate only)");
-        return PARESIS_ERR_ARG;
-    }
-    if (detect && (r.oversampling < 1 || r.det_x < 1 || r.det_y < 1)) {
-        set_last_error("paresis_df_run: bad detector geometry");
-        return PARESIS_ERR_ARG;
-    }
-    if (job->dark_field && !r.first_point) {
-        set_last_error("paresis_df_run: the dark-field map belongs to position 0 (first_point)");
-        return PARESIS_ERR_ARG;
-    }
     for (int e = 0; e < r.n_energies; ++e) {
         const paresis_rt_energy& en = r.energies_host[e];
         const paresis_df_energy& df = job->energies_df_host[e];
-        if (en.n_hop1 < 1 || en.n_hop1 > PARESIS_MAX_LAYERS) return bad("need 1 .. PARESIS_MAX_LAYERS membrane maps", e);
+        if (en.n_hop1 < 1 || en.n_hop1 > PARESIS_MAX_LAYERS) return bad(who, "need 1 .. PARESIS_MAX_LAYERS membrane maps", e);
         if (en.n_hop2 < 1 || en.n_hop2 > PARESIS_MAX_LAYERS)
-            return bad("need 1 .. PARESIS_MAX_LAYERS membrane + sample maps in the object hop (mix the sample's maps)", e);
-        if (r.first_point && (en.n_propag < 1 || en.n_propag > PARESIS_MAX_LAYERS))
-            return bad("need 1 .. PARESIS_MAX_LAYERS sample maps in the sample-only hop", e);
-        for (int m = 0; m < en.n_hop1; ++m) if (!en.hop1[m].thickness) return bad("null membrane map", e);
-        for (int m = 0; m < en.n_hop2; ++m) if (!en.hop2[m].thickness) return bad("null object-hop map", e);
-        if (r.first_point)
-            for (int m = 0; m < en.n_propag; ++m) if (!en.propag[m].thickness) return bad("null sample map", e);
-        if (!df.scatter_map) return bad("no scattering map", e);
+            return bad(who, "need 1 .. PARESIS_MAX_LAYERS membrane + sample maps in the object hop (mix the sample's maps)", e);
+        if (first && (en.n_propag < 1 || en.n_propag > PARESIS_MAX_LAYERS))
+            return bad(who, "need 1 .. PARESIS_MAX_LAYERS sample maps in the sample-only hop", e);
+        for (int m = 0; m < en.n_hop1; ++m) if (!en.hop1[m].thickness && !position_maps) return bad(who, "null membrane map", e);
+        for (int m = 0; m < en.n_hop2; ++m) if (!en.hop2[m].thickness && !position_maps) return bad(who, "null object-hop map", e);
+        if (first)
+            for (int m = 0; m < en.n_propag; ++m) if (!en.propag[m].thickness) return bad(who, "null sample map", e);
+        if (!df.scatter_map) return bad(who, "no scattering map", e);
     }
     return PARESIS_OK;
 }
 
-}  // namespace
+// every check that reads host memory only: nothing is launched before the whole job is known to be well formed
+int check_job(const paresis_df_job* job) {
+    const char* who = "paresis_df_run";
+    if (!job) { set_last_error("%s: null job", who); return PARESIS_ERR_ARG; }
+    const paresis_rt_job& r = job->rt;
+    if (!r.energies_host || !job->energies_df_host || r.n_energies < 1) {
+        set_last_error("%s: no energies", who);
+        return PARESIS_ERR_ARG;
+    }
+    if (r.nx < 3 || r.ny < 3) { set_last_error("%s: bad frame %d x %d", who, r.nx, r.ny); return PARESIS_ERR_ARG; }
+    if (!r.i_bs || !r.acc_sample || !r.acc_ref || (r.first_point && !r.acc_propag)) {
+        set_last_error("%s: null object-plane buffer or accumulator", who);
+        return PARESIS_ERR_ARG;
+    }
+    if (!job->angle || !job->plain || !job->scattered || !job->clean || !job->moved) {
+        set_last_error("%s: null dark-field scratch buffer", who);
+        return PARESIS_ERR_ARG;
+    }
+    const bool detect = r.out_sample || r.out_ref || r.out_propag || r.out_white;
+    if (detect && (!r.out_sample || !r.out_ref || (r.first_point && (!r.out_propag || !r.out_white || !r.acc_white)))) {
+        set_last_error("%s: incomplete detector outputs (all of them, or none to accumulate only)", who);
+        return PARESIS_ERR_ARG;
+    }
+    if (detect && (r.oversampling < 1 || r.det_x < 1 || r.det_y < 1)) {
+        set_last_error("%s: bad detector geometry", who);
+        return PARESIS_ERR_ARG;
+    }
+    if (job->dark_field && !r.first_point) {
+        set_last_error("%s: the dark-field map belongs to position 0 (first_point)", who);
+        return PARESIS_ERR_ARG;
+    }
+    return check_energies(who, job, r.first_point != 0, false);
+}
 
-extern "C" int paresis_df_run(const paresis_df_job* job, paresis_stream stream) {
-    int rc = check_job(job);
-    if (rc) return rc;
+// the launch sequence of a checked job
+int run_job(const paresis_df_job* job, paresis_stream stream) {
+    int rc = PARESIS_OK;
     const paresis_rt_job& r = job->rt;
     cudaStream_t s = (cudaStream_t)stream;
     const int nx = r.nx, ny = r.ny;
@@ -165,4 +181,148 @@ extern "C" int paresis_df_run(const paresis_df_job* job, paresis_stream stream) 
         }
     }
     return PARESIS_OK;
+}
+
+}  // namespace
+
+extern "C" int paresis_df_run(const paresis_df_job* job, paresis_stream stream) {
+    const int rc = check_job(job);
+    if (rc) return rc;
+    return run_job(job, stream);
+}
+
+namespace {
+
+int bad_positions(const char* fmt, int i) {
+    set_last_error(fmt, i);
+    return PARESIS_ERR_ARG;
+}
+
+constexpr int kSlotImages = 11;   // i_bs, four accumulators, five dark-field scratch images, detector work
+
+void slot_images(const paresis_df_slot& sl, const void* out[kSlotImages]) {
+    const void* v[kSlotImages] = {sl.i_bs, sl.acc_sample, sl.acc_ref, sl.acc_propag, sl.acc_white, sl.angle, sl.plain,
+                                  sl.scattered, sl.clean, sl.moved, sl.detect_work};
+    for (int i = 0; i < kSlotImages; ++i) out[i] = v[i];
+}
+
+// every argument of paresis_df_run_positions, host memory only
+int check_positions(const paresis_df_job* job, const paresis_membrane* mem, const paresis_df_position* positions,
+                    int n_positions, const paresis_df_slot* slots, int n_slots) {
+    const char* who = "paresis_df_run_positions";
+    if (!job || !mem || !positions || !slots) {
+        set_last_error("%s: null job, membrane, positions or slots", who);
+        return PARESIS_ERR_ARG;
+    }
+    if (n_slots < 1 || n_positions < 0) {
+        set_last_error("%s: need n_slots >= 1 and n_positions >= 0", who);
+        return PARESIS_ERR_ARG;
+    }
+    if (n_positions == 0) return PARESIS_OK;       // nothing to run, nothing else to check
+    const paresis_rt_job& r = job->rt;
+    if (!r.energies_host || !job->energies_df_host || r.n_energies < 1) { set_last_error("%s: no energies", who); return PARESIS_ERR_ARG; }
+    if (r.nx < 3 || r.ny < 3) { set_last_error("%s: bad frame %d x %d", who, r.nx, r.ny); return PARESIS_ERR_ARG; }
+    if (!mem->field && !mem->spheres) { set_last_error("%s: the membrane has neither a sphere field nor spheres", who); return PARESIS_ERR_ARG; }
+    if (r.oversampling < 1 || r.det_x < 1 || r.det_y < 1) {
+        set_last_error("%s: bad detector geometry", who);
+        return PARESIS_ERR_ARG;
+    }
+    bool any_first = false;
+    for (int p = 0; p < n_positions; ++p) {
+        const paresis_rt_position& pos = positions[p].rt;
+        if (!pos.offsets_host || !pos.thickness)
+            return bad_positions("paresis_df_run_positions: position %d lacks offsets or a thickness buffer", p);
+        if (!pos.out_sample || !pos.out_ref || (pos.first_point && (!pos.out_propag || !pos.out_white)))
+            return bad_positions("paresis_df_run_positions: position %d has incomplete detector outputs", p);
+        if (pos.probe_start || pos.probe_end)
+            return bad_positions("paresis_df_run_positions: position %d has probe events (this entry has no probe)", p);
+        if (positions[p].dark_field && !pos.first_point)
+            return bad_positions("paresis_df_run_positions: position %d: the dark-field map belongs to position 0 (first_point)", p);
+        any_first |= pos.first_point != 0;
+    }
+    for (int k = 0; k < n_slots; ++k) {
+        const paresis_df_slot& sl = slots[k];
+        if (!sl.i_bs || !sl.acc_sample || !sl.acc_ref || !sl.acc_propag || !sl.acc_white)
+            return bad_positions("paresis_df_run_positions: slot %d lacks an object-plane buffer or an accumulator", k);
+        if (!sl.angle || !sl.plain || !sl.scattered || !sl.clean || !sl.moved)
+            return bad_positions("paresis_df_run_positions: slot %d lacks a dark-field scratch image", k);
+    }
+    // slots run concurrently: an image two of them write would be a race
+    for (int k = 1; k < n_slots; ++k) {
+        const void* mine[kSlotImages];
+        slot_images(slots[k], mine);
+        for (int j = 0; j < k; ++j) {
+            const void* theirs[kSlotImages];
+            slot_images(slots[j], theirs);
+            for (int a = 0; a < kSlotImages; ++a)
+                for (int b = 0; b < kSlotImages; ++b)
+                    if (mine[a] && mine[a] == theirs[b])
+                        return bad_positions("paresis_df_run_positions: slot %d shares an image buffer with another slot (slots "
+                                             "run concurrently)", k);
+        }
+    }
+    const int rc = check_energies(who, job, any_first, true);
+    if (rc) return rc;
+    if (!mem->field) {
+        const size_t need = paresis_raster_work_bytes(mem->n_spheres, mem->n_layers, r.nx, r.ny);
+        for (int k = 0; k < n_slots; ++k)
+            if (!slots[k].raster_work || slots[k].raster_work_bytes < need)
+                return bad_positions("paresis_df_run_positions: slot %d: the membrane has no sphere field and the raster "
+                                     "work is smaller than paresis_raster_work_bytes", k);
+    }
+    return PARESIS_OK;
+}
+
+}  // namespace
+
+// Each position: its membrane map (cut from the sphere field, or rasterised), then the launch sequence of paresis_df_run
+// on its slot's stream with the slot's buffers.  Position p goes to slot p mod n_slots.
+extern "C" int paresis_df_run_positions(const paresis_df_job* job, const paresis_membrane* mem,
+                                        const paresis_df_position* positions, int n_positions, paresis_df_slot* slots,
+                                        int n_slots, paresis_stream stream) {
+    int rc = check_positions(job, mem, positions, n_positions, slots, n_slots);
+    if (rc) return rc;
+    if (n_positions == 0) return PARESIS_OK;
+    const paresis_rt_job& r = job->rt;
+    SlotEvents* events = nullptr;
+    rc = slot_events(n_slots, &events);
+    if (rc) return rc;
+    cudaStream_t main_stream = (cudaStream_t)stream;
+    const int used = n_slots < n_positions ? n_slots : n_positions;
+    rc = fork_slots(*events, main_stream, slots, used);
+    if (rc) return rc;
+
+    std::vector<paresis_rt_energy> energies(r.energies_host, r.energies_host + r.n_energies);
+    for (int p = 0; p < n_positions; ++p) {
+        const paresis_rt_position& pos = positions[p].rt;
+        paresis_df_slot& slot = slots[p % n_slots];
+        rc = membrane_of_position(mem, pos.offsets_host, r.nx, r.ny, pos.thickness, slot.raster_work, slot.raster_work_bytes,
+                                  slot.stream);
+        if (rc) return rc;
+        // a NULL map of the membrane or object hop stands for this position's membrane
+        for (int e = 0; e < r.n_energies; ++e) {
+            const paresis_rt_energy& src = r.energies_host[e];
+            paresis_rt_energy& dst = energies[e];
+            for (int m = 0; m < src.n_hop1; ++m) dst.hop1[m].thickness = src.hop1[m].thickness ? src.hop1[m].thickness : pos.thickness;
+            for (int m = 0; m < src.n_hop2; ++m) dst.hop2[m].thickness = src.hop2[m].thickness ? src.hop2[m].thickness : pos.thickness;
+        }
+        paresis_df_job j = *job;
+        paresis_rt_job& jr = j.rt;
+        jr.energies_host = energies.data();
+        jr.first_point = pos.first_point;
+        jr.i_bs = slot.i_bs; jr.acc_sample = slot.acc_sample; jr.acc_ref = slot.acc_ref;
+        jr.acc_propag = slot.acc_propag; jr.acc_white = slot.acc_white;
+        jr.i_bs_dirty = slot.i_bs_dirty;
+        jr.detect_work = slot.detect_work;
+        jr.means = pos.means;
+        jr.out_sample = pos.out_sample; jr.out_ref = pos.out_ref; jr.out_propag = pos.out_propag; jr.out_white = pos.out_white;
+        jr.sequence = pos.sequence;
+        if (n_positions > 1) jr.throughput = 1;       // launches of neighbouring positions overlap: least work per pixel wins
+        j.angle = slot.angle; j.plain = slot.plain; j.scattered = slot.scattered; j.clean = slot.clean; j.moved = slot.moved;
+        j.dark_field = positions[p].dark_field;
+        rc = run_job(&j, slot.stream);
+        if (rc) return rc;
+        slot.i_bs_dirty = 0;
+    }
+    return join_slots(*events, main_stream, slots, used);
 }

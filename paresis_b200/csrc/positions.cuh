@@ -1,5 +1,5 @@
-// What the many-positions entries (paresis_rt_run_positions, paresis_fresnel_run_positions) share: the fork / join of
-// their slot streams and the membrane map of one position.
+// What the many-positions entries (paresis_rt_run_positions, paresis_fresnel_run_positions, paresis_df_run_positions)
+// share: the fork / join of their slot streams and the membrane map of one position.
 #pragma once
 #include <vector>
 

@@ -18,6 +18,7 @@ from . import _cabi as abi
 from . import hostmath as hm
 
 IMAGES = ("sample", "reference", "propag", "white")
+DF_SCRATCH = ("angle", "plain", "scattered", "clean", "moved")    # scratch images of paresis_df_run
 
 
 class _PerPosition:
@@ -364,9 +365,11 @@ class ImageFormation:
     def _df_scratch(self):
         """The scratch images of paresis_df_run: angle, plain, scattered, clean, moved (any content between jobs)."""
         if self._df is None:
-            self._df = {k: torch.empty((self.nx, self.ny), device=self.device, dtype=torch.float32)
-                        for k in ("angle", "plain", "scattered", "clean", "moved")}
+            self._df = self._new_df_scratch()
         return self._df
+
+    def _new_df_scratch(self):
+        return {k: torch.empty((self.nx, self.ny), device=self.device, dtype=torch.float32) for k in DF_SCRATCH}
 
     def _df_job(self, scene, job, indices, dark_field=None):
         """Wrap a paresis_rt_job (``job``) into a paresis_df_job for the spectrum entries ``indices``."""
@@ -375,7 +378,7 @@ class ImageFormation:
         dj = abi.DfJob()
         dj.rt = job
         dj.energies_df_host = df_energies
-        for k in ("angle", "plain", "scattered", "clean", "moved"):
+        for k in DF_SCRATCH:
             setattr(dj, k, scratch[k].data_ptr())
         dj.dark_field = dark_field.data_ptr() if dark_field is not None else None
         return dj, (df_energies, keep)
@@ -477,9 +480,10 @@ class ImageFormation:
         self._i_bs_dirty = False
 
     # ------------------------------------------------------------------ many positions, one call
-    def _slots(self, n_slots, raster_bytes, fresnel=False):
-        """Scratch sets of paresis_rt_run_positions / paresis_fresnel_run_positions: slot 0 is this engine's own buffers.
-        ``fresnel``: each slot also gets a Fresnel plan, two waves and detector work of its own (slots run concurrently)."""
+    def _slots(self, n_slots, raster_bytes, fresnel=False, darkfield=False):
+        """Scratch sets of paresis_rt_run_positions / paresis_fresnel_run_positions / paresis_df_run_positions: slot 0 is
+        this engine's own buffers.  ``fresnel``: each slot also gets a Fresnel plan, two waves and detector work of its own
+        (slots run concurrently); ``darkfield``: the five scratch images of paresis_df_run and detector work of its own."""
         f32 = dict(device=self.device, dtype=torch.float32)
         cache = self.__dict__.setdefault("_slot_cache", [])
         while len(cache) < n_slots:
@@ -497,6 +501,13 @@ class ImageFormation:
                 if "plan" not in c:
                     c["plan"] = self._plan if k == 0 else abi.FresnelPlan(self.nx, self.ny, 15)
                     c["waves"] = self._waves if k == 0 else [torch.empty_like(w) for w in self._waves]
+        if darkfield:
+            for k, c in enumerate(cache[:n_slots]):
+                if "df" not in c:
+                    c["df"] = self._df_scratch() if k == 0 else self._new_df_scratch()
+        if fresnel or darkfield:
+            for k, c in enumerate(cache[:n_slots]):
+                if "detect_work" not in c:
                     c["detect_work"] = self.work if k == 0 else torch.empty_like(self.work)
         return cache[:n_slots]
 
@@ -560,8 +571,8 @@ class ImageFormation:
         sums [P, n_energies] (float64 sums of the reference beam, see paresis_rt_job.means)."""
         s = scene
         if self.scatters(s):
-            raise NotImplementedError("scattering (dark-field) samples run position by position: compute_rt, or the "
-                                      "energy-sharded call")
+            raise NotImplementedError("scattering (dark-field) samples run many positions per call through "
+                                      "compute_df_positions")
         n_pos = len(offsets)
         bins = self.bins(s)
         nbins, n_e = len(s.thresholds), len(s.spectrum)
@@ -605,6 +616,65 @@ class ImageFormation:
             c["dirty"] = False
         self._i_bs_dirty = False
         return self._positions_result(buffers, firsts)
+
+    @_on_own_device
+    def compute_df_positions(self, scene, plan, offsets, points, sequence_base=0, n_slots=2, want_means=True, buffers=None):
+        """``len(offsets)`` membrane positions of a scattering sample in one library call (paresis_df_run_positions): per
+        position the membrane is cut from ``plan`` (geometry.MembranePlan) at ``offsets[p]`` and the dark-field chain of
+        compute_rt runs, positions alternating between ``n_slots`` streams, each with buffers of its own.  No host
+        synchronisation.
+
+        ``scene.membrane`` must hold one ``Layer(PER_POSITION, ...)`` for the position's map, and a sample material must
+        scatter (Layer.scatter).  Arguments and result as compute_rt_positions, plus dark_field [P0, nx, ny] (radians, as
+        compute_rt's) for the positions with ``points[p] == 0`` (in order)."""
+        s = scene
+        if not self.scatters(s):
+            raise NotImplementedError("no material of the sample scatters: compute_rt_positions runs such a scene")
+        n_pos = len(offsets)
+        bins = self.bins(s)
+        nbins, n_e = len(s.thresholds), len(s.spectrum)
+        closing = {b[-1] for b in bins[:nbins]}
+        energies, keep = self._rt_energies(s, list(range(n_e)), closing)
+        job, keep2 = self._rt_job(s, energies, False, 0, group=False)
+        dj, keep3 = self._df_job(s, job, list(range(n_e)))
+        firsts = [p for p in range(n_pos) if points[p] == 0]
+        if buffers is None:
+            buffers = self._positions_buffers(n_pos, len(firsts), nbins, n_e)
+        if "dark_field" not in buffers:
+            buffers["dark_field"] = torch.empty((max(len(firsts), 1), self.nx, self.ny), device=self.device, dtype=torch.float32)
+        buffers["dark_field"].zero_()         # paresis_df_run_positions adds to it
+        membrane, field = self._membrane(plan)
+        raster_bytes = abi.lib.paresis_raster_work_bytes(plan.table.shape[0], plan.layers, self.nx, self.ny)
+        slots = self._slots(n_slots, raster_bytes, darkfield=True)
+        c_slots = (abi.DfSlot * n_slots)()
+        for k, c in enumerate(slots):
+            sl = c_slots[k]
+            sl.i_bs = c["i_bs"].data_ptr()
+            sl.acc_sample, sl.acc_ref = c["acc"]["sample"].data_ptr(), c["acc"]["reference"].data_ptr()
+            sl.acc_propag, sl.acc_white = c["acc"]["propag"].data_ptr(), c["acc"]["white"].data_ptr()
+            for name in DF_SCRATCH:
+                setattr(sl, name, c["df"][name].data_ptr())
+            sl.detect_work = c["detect_work"].data_ptr()
+            sl.raster_work, sl.raster_work_bytes = c["work"].data_ptr(), c["work"].numel()
+            sl.stream = c["stream"].cuda_stream
+            sl.i_bs_dirty = 1 if (c["dirty"] or (k == 0 and self._i_bs_dirty)) else 0
+            c["dirty"] = True
+        self._i_bs_dirty = True
+        rt_pos, offs = self._c_positions(buffers, offsets, points, firsts, plan.layers, sequence_base, want_means)
+        c_pos = (abi.DfPosition * n_pos)()
+        for p in range(n_pos):
+            c_pos[p].rt = rt_pos[p]
+            if points[p] == 0:
+                c_pos[p].dark_field = buffers["dark_field"][firsts.index(p)].data_ptr()
+        cut = 1 if field is not None else 2
+        launches = sum(cut + self._df_launches(n_e, len(closing), points[p] == 0) for p in range(n_pos))
+        abi.df_run_positions(dj, membrane, c_pos, c_slots, launches)
+        for c in slots:
+            c["dirty"] = False
+        self._i_bs_dirty = False
+        res = self._positions_result(buffers, firsts)
+        res["dark_field"] = buffers["dark_field"][:len(firsts)]
+        return res
 
     @_on_own_device
     def accumulate_rt(self, scene, point_num, indices, dark_field=None):
