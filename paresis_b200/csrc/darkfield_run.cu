@@ -93,7 +93,7 @@ int run_job(const paresis_df_job* job, paresis_stream stream) {
     const paresis_rt_job& r = job->rt;
     cudaStream_t s = (cudaStream_t)stream;
     const int nx = r.nx, ny = r.ny;
-    const size_t n = (size_t)nx * ny, nd = (size_t)r.det_x * r.det_y;
+    const size_t n = (size_t)nx * ny;
     const float limit = nx / 4.f;                         // refractionFileNumba2.py:130
     const bool detect = r.out_sample != nullptr;
     if (r.i_bs_dirty) PARESIS_CUDA(cudaMemsetAsync(r.i_bs, 0, sizeof(float) * n, s));
@@ -162,19 +162,7 @@ int run_job(const paresis_df_job* job, paresis_stream stream) {
             white += en.intensity_propag;
         }
         if (detect && en.close_bin) {   // :501-521, all images of the bin in one launch
-            const int count = r.first_point ? 4 : 2;
-            if (r.first_point) {
-                rc = paresis_fill(r.acc_white, white, n, stream);
-                if (rc) return rc;
-            }
-            const uint64_t seq = r.sequence + (uint64_t)ibin * 4;
-            const float* in_k[4] = {r.acc_sample, r.acc_ref, r.acc_propag, r.acc_white};
-            float* out_k[4] = {r.out_sample + (size_t)ibin * nd, r.out_ref + (size_t)ibin * nd,
-                               r.first_point ? r.out_propag + (size_t)ibin * nd : nullptr,
-                               r.first_point ? r.out_white + (size_t)ibin * nd : nullptr};
-            const uint64_t seq_k[4] = {seq, seq + 1, seq + 2, seq + 3};
-            rc = paresis_detect_counts_multi(in_k, out_k, seq_k, count, nx, ny, r.oversampling, r.det_x, r.det_y, r.src_kernel,
-                                             r.src_half, r.psf_kernel, r.psf_half, r.detect_work, r.noise, r.seed, stream);
+            rc = close_bin(r, nx, ny, ibin, white, stream);
             if (rc) return rc;
             ++ibin;
             fresh_bin = true;
@@ -210,32 +198,18 @@ void slot_images(const paresis_df_slot& sl, const void* out[kSlotImages]) {
 int check_positions(const paresis_df_job* job, const paresis_membrane* mem, const paresis_df_position* positions,
                     int n_positions, const paresis_df_slot* slots, int n_slots) {
     const char* who = "paresis_df_run_positions";
-    if (!job || !mem || !positions || !slots) {
-        set_last_error("%s: null job, membrane, positions or slots", who);
-        return PARESIS_ERR_ARG;
-    }
-    if (n_slots < 1 || n_positions < 0) {
-        set_last_error("%s: need n_slots >= 1 and n_positions >= 0", who);
-        return PARESIS_ERR_ARG;
-    }
-    if (n_positions == 0) return PARESIS_OK;       // nothing to run, nothing else to check
+    int rc = check_call(who, job, mem, positions, slots, n_positions, n_slots);
+    if (rc || n_positions == 0) return rc;       // nothing to run, nothing else to check
     const paresis_rt_job& r = job->rt;
     if (!r.energies_host || !job->energies_df_host || r.n_energies < 1) { set_last_error("%s: no energies", who); return PARESIS_ERR_ARG; }
     if (r.nx < 3 || r.ny < 3) { set_last_error("%s: bad frame %d x %d", who, r.nx, r.ny); return PARESIS_ERR_ARG; }
-    if (!mem->field && !mem->spheres) { set_last_error("%s: the membrane has neither a sphere field nor spheres", who); return PARESIS_ERR_ARG; }
-    if (r.oversampling < 1 || r.det_x < 1 || r.det_y < 1) {
-        set_last_error("%s: bad detector geometry", who);
-        return PARESIS_ERR_ARG;
-    }
+    rc = check_membrane_detector(who, mem, r.oversampling, r.det_x, r.det_y);
+    if (rc) return rc;
     bool any_first = false;
     for (int p = 0; p < n_positions; ++p) {
         const paresis_rt_position& pos = positions[p].rt;
-        if (!pos.offsets_host || !pos.thickness)
-            return bad_positions("paresis_df_run_positions: position %d lacks offsets or a thickness buffer", p);
-        if (!pos.out_sample || !pos.out_ref || (pos.first_point && (!pos.out_propag || !pos.out_white)))
-            return bad_positions("paresis_df_run_positions: position %d has incomplete detector outputs", p);
-        if (pos.probe_start || pos.probe_end)
-            return bad_positions("paresis_df_run_positions: position %d has probe events (this entry has no probe)", p);
+        rc = check_position(who, pos, p);
+        if (rc) return rc;
         if (positions[p].dark_field && !pos.first_point)
             return bad_positions("paresis_df_run_positions: position %d: the dark-field map belongs to position 0 (first_point)", p);
         any_first |= pos.first_point != 0;
@@ -261,16 +235,9 @@ int check_positions(const paresis_df_job* job, const paresis_membrane* mem, cons
                                              "run concurrently)", k);
         }
     }
-    const int rc = check_energies(who, job, any_first, true);
+    rc = check_energies(who, job, any_first, true);
     if (rc) return rc;
-    if (!mem->field) {
-        const size_t need = paresis_raster_work_bytes(mem->n_spheres, mem->n_layers, r.nx, r.ny);
-        for (int k = 0; k < n_slots; ++k)
-            if (!slots[k].raster_work || slots[k].raster_work_bytes < need)
-                return bad_positions("paresis_df_run_positions: slot %d: the membrane has no sphere field and the raster "
-                                     "work is smaller than paresis_raster_work_bytes", k);
-    }
-    return PARESIS_OK;
+    return check_raster_work(who, mem, r.nx, r.ny, slots, n_slots);
 }
 
 }  // namespace
@@ -284,45 +251,27 @@ extern "C" int paresis_df_run_positions(const paresis_df_job* job, const paresis
     if (rc) return rc;
     if (n_positions == 0) return PARESIS_OK;
     const paresis_rt_job& r = job->rt;
-    SlotEvents* events = nullptr;
-    rc = slot_events(n_slots, &events);
-    if (rc) return rc;
-    cudaStream_t main_stream = (cudaStream_t)stream;
-    const int used = n_slots < n_positions ? n_slots : n_positions;
-    rc = fork_slots(*events, main_stream, slots, used);
-    if (rc) return rc;
-
     std::vector<paresis_rt_energy> energies(r.energies_host, r.energies_host + r.n_energies);
-    for (int p = 0; p < n_positions; ++p) {
+    return run_on_slots(slots, n_slots, n_positions, stream, [&](int p, paresis_df_slot& slot) -> int {
         const paresis_rt_position& pos = positions[p].rt;
-        paresis_df_slot& slot = slots[p % n_slots];
-        rc = membrane_of_position(mem, pos.offsets_host, r.nx, r.ny, pos.thickness, slot.raster_work, slot.raster_work_bytes,
-                                  slot.stream);
+        int rc = membrane_of_position(mem, pos.offsets_host, r.nx, r.ny, pos.thickness, slot.raster_work, slot.raster_work_bytes,
+                                      slot.stream);
         if (rc) return rc;
-        // a NULL map of the membrane or object hop stands for this position's membrane
-        for (int e = 0; e < r.n_energies; ++e) {
-            const paresis_rt_energy& src = r.energies_host[e];
-            paresis_rt_energy& dst = energies[e];
-            for (int m = 0; m < src.n_hop1; ++m) dst.hop1[m].thickness = src.hop1[m].thickness ? src.hop1[m].thickness : pos.thickness;
-            for (int m = 0; m < src.n_hop2; ++m) dst.hop2[m].thickness = src.hop2[m].thickness ? src.hop2[m].thickness : pos.thickness;
-        }
+        bind_position_maps(r.energies_host, r.n_energies, pos.thickness, energies.data());
         paresis_df_job j = *job;
         paresis_rt_job& jr = j.rt;
         jr.energies_host = energies.data();
-        jr.first_point = pos.first_point;
+        bind_position(jr, pos);
         jr.i_bs = slot.i_bs; jr.acc_sample = slot.acc_sample; jr.acc_ref = slot.acc_ref;
         jr.acc_propag = slot.acc_propag; jr.acc_white = slot.acc_white;
         jr.i_bs_dirty = slot.i_bs_dirty;
         jr.detect_work = slot.detect_work;
-        jr.means = pos.means;
-        jr.out_sample = pos.out_sample; jr.out_ref = pos.out_ref; jr.out_propag = pos.out_propag; jr.out_white = pos.out_white;
-        jr.sequence = pos.sequence;
         if (n_positions > 1) jr.throughput = 1;       // launches of neighbouring positions overlap: least work per pixel wins
         j.angle = slot.angle; j.plain = slot.plain; j.scattered = slot.scattered; j.clean = slot.clean; j.moved = slot.moved;
         j.dark_field = positions[p].dark_field;
         rc = run_job(&j, slot.stream);
         if (rc) return rc;
         slot.i_bs_dirty = 0;
-    }
-    return join_slots(*events, main_stream, slots, used);
+        return PARESIS_OK;
+    });
 }

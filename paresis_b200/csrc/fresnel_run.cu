@@ -104,7 +104,7 @@ int run_job(const paresis_fresnel_job* job, paresis_stream stream) {
     cudaStream_t s = (cudaStream_t)stream;
     int nx = 0, ny = 0;
     fresnel_plan_dims(job->plan, &nx, &ny);
-    const size_t n = (size_t)nx * ny, nd = (size_t)job->det_x * job->det_y;
+    const size_t n = (size_t)nx * ny;
     const bool detect = job->out_sample != nullptr;
     float2* wa = reinterpret_cast<float2*>(job->wave_a);
     float2* wb = reinterpret_cast<float2*>(job->wave_b);
@@ -144,20 +144,7 @@ int run_job(const paresis_fresnel_job* job, paresis_stream stream) {
             white += en.white;
         }
         if (detect && en.close_bin) {   // :378-398, all images of the bin in one launch
-            const int count = job->first_point ? 4 : 2;
-            if (job->first_point) {
-                rc = paresis_fill(job->acc_white, (float)white, n, stream);
-                if (rc) return rc;
-            }
-            const uint64_t seq = job->sequence + (uint64_t)ibin * 4;
-            const float* in_k[4] = {job->acc_sample, job->acc_ref, job->acc_propag, job->acc_white};
-            float* out_k[4] = {job->out_sample + (size_t)ibin * nd, job->out_ref + (size_t)ibin * nd,
-                               job->first_point ? job->out_propag + (size_t)ibin * nd : nullptr,
-                               job->first_point ? job->out_white + (size_t)ibin * nd : nullptr};
-            const uint64_t seq_k[4] = {seq, seq + 1, seq + 2, seq + 3};
-            rc = paresis_detect_counts_multi(in_k, out_k, seq_k, count, nx, ny, job->oversampling, job->det_x, job->det_y,
-                                             job->src_kernel, job->src_half, job->psf_kernel, job->psf_half, job->detect_work,
-                                             job->noise, job->seed, stream);
+            rc = close_bin(*job, nx, ny, ibin, (float)white, stream);
             if (rc) return rc;
             ++ibin;
             fresh_bin = true;
@@ -185,31 +172,15 @@ int bad_positions(const char* fmt, int i) {
 int check_positions(const paresis_fresnel_job* job, const paresis_membrane* mem, const paresis_rt_position* positions,
                     int n_positions, const paresis_fresnel_slot* slots, int n_slots) {
     const char* who = "paresis_fresnel_run_positions";
-    if (!job || !mem || !positions || !slots) {
-        set_last_error("%s: null job, membrane, positions or slots", who);
-        return PARESIS_ERR_ARG;
-    }
-    if (n_slots < 1 || n_positions < 0) {
-        set_last_error("%s: need n_slots >= 1 and n_positions >= 0", who);
-        return PARESIS_ERR_ARG;
-    }
-    if (n_positions == 0) return PARESIS_OK;       // nothing to run, nothing else to check
+    int rc = check_call(who, job, mem, positions, slots, n_positions, n_slots);
+    if (rc || n_positions == 0) return rc;       // nothing to run, nothing else to check
     if (!job->energies_host || job->n_energies < 1) { set_last_error("%s: no energies", who); return PARESIS_ERR_ARG; }
-    if (!mem->field && !mem->spheres) { set_last_error("%s: the membrane has neither a sphere field nor spheres", who); return PARESIS_ERR_ARG; }
-    if (job->oversampling < 1 || job->det_x < 1 || job->det_y < 1) {
-        set_last_error("%s: bad detector geometry", who);
-        return PARESIS_ERR_ARG;
-    }
+    rc = check_membrane_detector(who, mem, job->oversampling, job->det_x, job->det_y);
+    if (rc) return rc;
     for (int p = 0; p < n_positions; ++p) {
-        const paresis_rt_position& pos = positions[p];
-        if (!pos.offsets_host || !pos.thickness)
-            return bad_positions("paresis_fresnel_run_positions: position %d lacks offsets or a thickness buffer", p);
-        if (!pos.out_sample || !pos.out_ref || (pos.first_point && (!pos.out_propag || !pos.out_white)))
-            return bad_positions("paresis_fresnel_run_positions: position %d has incomplete detector outputs", p);
-        if (pos.probe_start || pos.probe_end)
-            return bad_positions("paresis_fresnel_run_positions: position %d has probe events (this entry has no probe)", p);
+        rc = check_position(who, positions[p], p);
+        if (rc) return rc;
     }
-    int nx = 0, ny = 0;
     for (int k = 0; k < n_slots; ++k) {
         const paresis_fresnel_slot& sl = slots[k];
         if (!sl.plan) return bad_positions("paresis_fresnel_run_positions: slot %d has no plan", k);
@@ -220,21 +191,15 @@ int check_positions(const paresis_fresnel_job* job, const paresis_membrane* mem,
                 return bad_positions("paresis_fresnel_run_positions: slot %d shares its plan with another slot (a plan owns its "
                                      "work buffers)", k);
     }
-    int rc = check_energies(who, job, true);
+    rc = check_energies(who, job, true);
     if (rc) return rc;
     for (int k = 0; k < n_slots; ++k) {
         rc = check_kernels(who, job, slots[k].plan);
         if (rc) return rc;
     }
+    int nx = 0, ny = 0;
     fresnel_plan_dims(slots[0].plan, &nx, &ny);
-    if (!mem->field) {
-        const size_t need = paresis_raster_work_bytes(mem->n_spheres, mem->n_layers, nx, ny);
-        for (int k = 0; k < n_slots; ++k)
-            if (!slots[k].raster_work || slots[k].raster_work_bytes < need)
-                return bad_positions("paresis_fresnel_run_positions: slot %d: the membrane has no sphere field and the raster "
-                                     "work is smaller than paresis_raster_work_bytes", k);
-    }
-    return PARESIS_OK;
+    return check_raster_work(who, mem, nx, ny, slots, n_slots);
 }
 
 }  // namespace
@@ -249,14 +214,6 @@ extern "C" int paresis_fresnel_run_positions(const paresis_fresnel_job* job, con
     if (n_positions == 0) return PARESIS_OK;
     int nx = 0, ny = 0;
     fresnel_plan_dims(slots[0].plan, &nx, &ny);
-    SlotEvents* events = nullptr;
-    rc = slot_events(n_slots, &events);
-    if (rc) return rc;
-    cudaStream_t main_stream = (cudaStream_t)stream;
-    const int used = n_slots < n_positions ? n_slots : n_positions;
-    rc = fork_slots(*events, main_stream, slots, used);
-    if (rc) return rc;
-
     // the template's energies with a NULL membrane map replaced by the position's: membrane layers of energy e start at
     // first[e] of `layers`
     std::vector<paresis_fresnel_energy> energies(job->energies_host, job->energies_host + job->n_energies);
@@ -265,10 +222,10 @@ extern "C" int paresis_fresnel_run_positions(const paresis_fresnel_job* job, con
     for (int e = 0; e < job->n_energies; ++e) { first[e] = n_layers; n_layers += job->energies_host[e].n_membrane; }
     std::vector<paresis_wave_layer> layers(n_layers);
     for (int e = 0; e < job->n_energies; ++e) energies[e].membrane_host = layers.data() + first[e];
-    for (int p = 0; p < n_positions; ++p) {
+    return run_on_slots(slots, n_slots, n_positions, stream, [&](int p, const paresis_fresnel_slot& slot) -> int {
         const paresis_rt_position& pos = positions[p];
-        const paresis_fresnel_slot& slot = slots[p % n_slots];
-        rc = membrane_of_position(mem, pos.offsets_host, nx, ny, pos.thickness, slot.raster_work, slot.raster_work_bytes, slot.stream);
+        int rc = membrane_of_position(mem, pos.offsets_host, nx, ny, pos.thickness, slot.raster_work, slot.raster_work_bytes,
+                                      slot.stream);
         if (rc) return rc;
         for (int e = 0; e < job->n_energies; ++e) {
             const paresis_fresnel_energy& src = job->energies_host[e];
@@ -281,15 +238,10 @@ extern "C" int paresis_fresnel_run_positions(const paresis_fresnel_job* job, con
         paresis_fresnel_job j = *job;
         j.plan = slot.plan;
         j.energies_host = energies.data();
-        j.first_point = pos.first_point;
+        bind_position(j, pos);
         j.wave_a = slot.wave_a; j.wave_b = slot.wave_b;
         j.acc_sample = slot.acc_sample; j.acc_ref = slot.acc_ref; j.acc_propag = slot.acc_propag; j.acc_white = slot.acc_white;
         j.detect_work = slot.detect_work;
-        j.means = pos.means;
-        j.out_sample = pos.out_sample; j.out_ref = pos.out_ref; j.out_propag = pos.out_propag; j.out_white = pos.out_white;
-        j.sequence = pos.sequence;
-        rc = run_job(&j, slot.stream);
-        if (rc) return rc;
-    }
-    return join_slots(*events, main_stream, slots, used);
+        return run_job(&j, slot.stream);
+    });
 }

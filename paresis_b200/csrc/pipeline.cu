@@ -25,7 +25,7 @@ extern "C" int paresis_rt_run(const paresis_rt_job* job, paresis_stream stream) 
         return PARESIS_ERR_ARG;
     }
     cudaStream_t s = (cudaStream_t)stream;
-    const size_t n = (size_t)job->nx * job->ny, nd = (size_t)job->det_x * job->det_y;
+    const size_t n = (size_t)job->nx * job->ny;
     const int margin = 15;   // refractionFileNumba2.py:50
     // object-plane intensity buffers: one per energy of a group (all zero between jobs)
     float* ibs[PARESIS_MAX_GROUP] = {job->i_bs};
@@ -76,28 +76,6 @@ extern "C" int paresis_rt_run(const paresis_rt_job* job, paresis_stream stream) 
                                                  want_d ? job->dx_pad : nullptr, want_d ? job->dy_pad : nullptr, job->nx, job->ny,
                                                  margin, job->flag, &x3, stream);
         white += en.intensity_propag;
-        return rc;
-    };
-    // all images of the bin in one launch (Detector.detection is called once per image, :501-521)
-    auto close_bin = [&]() -> int {
-        const uint64_t seq = job->sequence + (uint64_t)ibin * 4;
-        float* const imgs[4] = {job->acc_sample, job->acc_ref, job->acc_propag, job->acc_white};
-        float* const outs[4] = {job->out_sample, job->out_ref, job->out_propag, job->out_white};
-        const int count = job->first_point ? 4 : 2;
-        int rc = PARESIS_OK;
-        if (job->first_point) {
-            rc = paresis_fill(job->acc_white, white, n, stream);
-            if (rc) return rc;
-        }
-        const float* in_k[4]; float* out_k[4]; uint64_t seq_k[4];
-        for (int k = 0; k < count; ++k) { in_k[k] = imgs[k]; out_k[k] = outs[k] + (size_t)ibin * nd; seq_k[k] = seq + k; }
-        if (ibin == 0) probe(3, true);
-        rc = paresis_detect_counts_multi(in_k, out_k, seq_k, count, job->nx, job->ny, job->oversampling, job->det_x,
-                                         job->det_y, job->src_kernel, job->src_half, job->psf_kernel, job->psf_half,
-                                         job->detect_work, job->noise, job->seed, stream);
-        if (ibin == 0) probe(3, false);
-        ++ibin;
-        fresh_bin = true;
         return rc;
     };
     auto same_maps = [&](const paresis_rt_energy& p, const paresis_rt_energy& q) {
@@ -157,8 +135,12 @@ extern "C" int paresis_rt_run(const paresis_rt_job* job, paresis_stream stream) 
             }
         }
         if (job->energies_host[e + group - 1].close_bin) {   // :501-521
-            rc = close_bin();
+            const bool probed = ibin == 0 && job->probe == 3 && job->probe_start && job->probe_end;
+            rc = close_bin(*job, job->nx, job->ny, ibin, white, stream, probed ? job->probe_start : nullptr,
+                           probed ? job->probe_end : nullptr);
             if (rc) return rc;
+            ++ibin;
+            fresh_bin = true;
         }
         e += group;
     }
@@ -275,15 +257,7 @@ static int run_positions_batched(const paresis_rt_job* job, const paresis_membra
         int rc = paresis_membrane_from_field(mem->field, mem->field_x, mem->field_y, pos.offsets_host, mem->n_layers, mem->margin,
                                              job->nx, job->ny, pos.thickness, stream);
         if (rc) return rc;
-        for (int e = 0; e < job->n_energies; ++e) {
-            const paresis_rt_energy& src = job->energies_host[e];
-            paresis_rt_energy& dst = energies[e];
-            for (int m = 0; m < PARESIS_MAX_LAYERS; ++m) {
-                dst.hop1[m].thickness = src.hop1[m].thickness ? src.hop1[m].thickness : pos.thickness;
-                dst.hop2[m].thickness = src.hop2[m].thickness ? src.hop2[m].thickness : pos.thickness;
-                dst.propag[m].thickness = src.propag[m].thickness ? src.propag[m].thickness : pos.thickness;
-            }
-        }
+        bind_position_maps(job->energies_host, job->n_energies, pos.thickness, energies.data());
         paresis_rt_job j = *job;
         j.energies_host = energies.data();
         j.first_point = 1;
@@ -312,59 +286,30 @@ extern "C" int paresis_rt_run_positions(const paresis_rt_job* job, const paresis
     if (n_positions == 0) return PARESIS_OK;
     if (job->positions_per_launch > 1 && mem->field && !job->i_bs_group[0] && single_energy_bins(job))
         return run_positions_batched(job, mem, positions, n_positions, slots, n_slots, stream);
-    SlotEvents* events = nullptr;
-    int rc = slot_events(n_slots, &events);
-    if (rc) return rc;
-    SlotEvents& g_events = *events;
-    cudaStream_t main_stream = (cudaStream_t)stream;
-    const int used = n_slots < n_positions ? n_slots : n_positions;
-    rc = fork_slots(g_events, main_stream, slots, used);
-    if (rc) return rc;
-
     std::vector<paresis_rt_energy> energies(job->energies_host, job->energies_host + job->n_energies);
-    for (int p = 0; p < n_positions; ++p) {
+    // A probed position runs alone on the GPU, so that the CUDA events around its kernel time that kernel and not its
+    // neighbours on the other streams.
+    auto probed = [&](int p) { return job->probe != 0 && positions[p].probe_start && positions[p].probe_end && n_slots > 1; };
+    auto run = [&](int p, paresis_rt_slot& slot) -> int {
         const paresis_rt_position& pos = positions[p];
-        paresis_rt_slot& slot = slots[p % n_slots];
         if (!pos.offsets_host || !pos.thickness) {
             set_last_error("paresis_rt_run_positions: position %d lacks offsets or a thickness buffer", p);
             return PARESIS_ERR_ARG;
         }
-        // A probed position runs alone on the GPU (the other slots drain first and wait for it), so that the
-        // CUDA events around its kernel time that kernel and not its neighbours on the other streams.
-        const bool probed = job->probe != 0 && pos.probe_start && pos.probe_end && n_slots > 1;
-        if (probed) {
-            for (int k = 0; k < used; ++k) {
-                if (&slots[k] == &slot) continue;
-                PARESIS_CUDA(cudaEventRecord(g_events.join[k], (cudaStream_t)slots[k].stream));
-                PARESIS_CUDA(cudaStreamWaitEvent((cudaStream_t)slot.stream, g_events.join[k], 0));
-            }
-        }
         const bool probe_raster = job->probe == 4 && pos.probe_start && pos.probe_end;
         if (probe_raster) cudaEventRecord((cudaEvent_t)pos.probe_start, (cudaStream_t)slot.stream);
-        rc = membrane_of_position(mem, pos.offsets_host, job->nx, job->ny, pos.thickness, slot.raster_work, slot.raster_work_bytes,
-                                  slot.stream);
+        int rc = membrane_of_position(mem, pos.offsets_host, job->nx, job->ny, pos.thickness, slot.raster_work,
+                                      slot.raster_work_bytes, slot.stream);
         if (probe_raster) cudaEventRecord((cudaEvent_t)pos.probe_end, (cudaStream_t)slot.stream);
         if (rc) return rc;
-        // a NULL layer map stands for this position's membrane
-        for (int e = 0; e < job->n_energies; ++e) {
-            const paresis_rt_energy& src = job->energies_host[e];
-            paresis_rt_energy& dst = energies[e];
-            for (int m = 0; m < PARESIS_MAX_LAYERS; ++m) {
-                dst.hop1[m].thickness = src.hop1[m].thickness ? src.hop1[m].thickness : pos.thickness;
-                dst.hop2[m].thickness = src.hop2[m].thickness ? src.hop2[m].thickness : pos.thickness;
-                dst.propag[m].thickness = src.propag[m].thickness ? src.propag[m].thickness : pos.thickness;
-            }
-        }
+        bind_position_maps(job->energies_host, job->n_energies, pos.thickness, energies.data());
         paresis_rt_job j = *job;
         j.energies_host = energies.data();
-        j.first_point = pos.first_point;
+        bind_position(j, pos);
         j.i_bs = slot.i_bs; j.acc_sample = slot.acc_sample; j.acc_ref = slot.acc_ref;
         for (int k = 0; k < PARESIS_MAX_GROUP - 1; ++k) j.i_bs_group[k] = slot.i_bs_group[k];
         j.acc_propag = slot.acc_propag; j.acc_white = slot.acc_white;
         j.i_bs_dirty = slot.i_bs_dirty;
-        j.means = pos.means;
-        j.out_sample = pos.out_sample; j.out_ref = pos.out_ref; j.out_propag = pos.out_propag; j.out_white = pos.out_white;
-        j.sequence = pos.sequence;
         j.probe_start = pos.probe_start; j.probe_end = pos.probe_end;
         if (!pos.probe_start || !pos.probe_end) j.probe = 0;
         j.dx_pad = j.dy_pad = nullptr;
@@ -372,11 +317,7 @@ extern "C" int paresis_rt_run_positions(const paresis_rt_job* job, const paresis
         rc = paresis_rt_run(&j, slot.stream);
         if (rc) return rc;
         slot.i_bs_dirty = 0;
-        if (probed) {
-            PARESIS_CUDA(cudaEventRecord(g_events.fork, (cudaStream_t)slot.stream));
-            for (int k = 0; k < used; ++k)
-                if (&slots[k] != &slot) PARESIS_CUDA(cudaStreamWaitEvent((cudaStream_t)slots[k].stream, g_events.fork, 0));
-        }
-    }
-    return join_slots(g_events, main_stream, slots, used);
+        return PARESIS_OK;
+    };
+    return run_on_slots(slots, n_slots, n_positions, stream, run, probed);
 }

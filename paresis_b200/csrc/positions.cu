@@ -1,4 +1,4 @@
-// Shared parts of the many-positions entries (positions.cuh).
+// Shared parts of the run entries (positions.cuh).
 #include "positions.cuh"
 
 namespace paresis {
@@ -15,6 +15,11 @@ int SlotEvents::ensure(int n) {
 
 namespace {
 SlotEvents g_events_of[32];     // CUDA events belong to a device
+
+int bad(const char* fmt, const char* who, int i = 0) {
+    set_last_error(fmt, who, i);
+    return PARESIS_ERR_ARG;
+}
 }  // namespace
 
 int slot_events(int n, SlotEvents** out) {
@@ -34,6 +39,39 @@ int membrane_of_position(const paresis_membrane* mem, const int64_t* offsets_hos
                                            ny, thickness, stream);
     return paresis_raster_spheres(mem->spheres, mem->n_spheres, mem->pix_um, offsets_host, mem->n_layers, nx, ny, mem->margin,
                                   thickness, raster_work, raster_work_bytes, stream);
+}
+
+void bind_position_maps(const paresis_rt_energy* energies, int n_energies, const float* thickness, paresis_rt_energy* out) {
+    auto bind = [&](const paresis_layer* src, int n, paresis_layer* dst) {
+        for (int m = 0; m < n && m < PARESIS_MAX_LAYERS; ++m) dst[m].thickness = src[m].thickness ? src[m].thickness : thickness;
+    };
+    for (int e = 0; e < n_energies; ++e) {
+        const paresis_rt_energy& src = energies[e];
+        bind(src.hop1, src.n_hop1, out[e].hop1);
+        bind(src.hop2, src.n_hop2, out[e].hop2);
+        bind(src.propag, src.n_propag, out[e].propag);
+    }
+}
+
+int check_call(const char* who, const void* job, const paresis_membrane* mem, const void* positions, const void* slots,
+               int n_positions, int n_slots) {
+    if (!job || !mem || !positions || !slots) return bad("%s: null job, membrane, positions or slots", who);
+    if (n_slots < 1 || n_positions < 0) return bad("%s: need n_slots >= 1 and n_positions >= 0", who);
+    return PARESIS_OK;
+}
+
+int check_membrane_detector(const char* who, const paresis_membrane* mem, int oversampling, int det_x, int det_y) {
+    if (!mem->field && !mem->spheres) return bad("%s: the membrane has neither a sphere field nor spheres", who);
+    if (oversampling < 1 || det_x < 1 || det_y < 1) return bad("%s: bad detector geometry", who);
+    return PARESIS_OK;
+}
+
+int check_position(const char* who, const paresis_rt_position& pos, int p) {
+    if (!pos.offsets_host || !pos.thickness) return bad("%s: position %d lacks offsets or a thickness buffer", who, p);
+    if (!pos.out_sample || !pos.out_ref || (pos.first_point && (!pos.out_propag || !pos.out_white)))
+        return bad("%s: position %d has incomplete detector outputs", who, p);
+    if (pos.probe_start || pos.probe_end) return bad("%s: position %d has probe events (this entry has no probe)", who, p);
+    return PARESIS_OK;
 }
 
 }  // namespace paresis

@@ -10,6 +10,7 @@ The host shim (``paresis_b200/CodePython/Experiment.py``) builds a :class:`Scene
 XML-derived objects and calls :meth:`ImageFormation.compute_rt` / ``compute_fresnel``.
 """
 import time
+from types import SimpleNamespace
 
 import numpy as np
 import torch
@@ -315,27 +316,34 @@ class ImageFormation:
             en.close_bin = 1 if ie in closing else 0
         return energies, keep
 
-    def _rt_job(self, scene, energies, first, sequence, group=True):
+    def _detector_fields(self, job, scene, sequence):
+        """The fields paresis_rt_job and paresis_fresnel_job share: detector geometry and kernels, noise, the per-energy
+        sums (self.means, grown to ``job.n_energies``) and the detector work.  Returns the kernels the job points to."""
         fwhm = scene.effective_source_fwhm()
         src = self._gauss(fwhm / 2.355) if fwhm != 0 else None
         psf = self._gauss(scene.psf_sigma) if scene.psf_sigma != 0 else None
-        if len(energies) > self.means.numel():
-            self.means = torch.zeros(len(energies), device=self.device, dtype=torch.float64)
+        if job.n_energies > self.means.numel():
+            self.means = torch.zeros(job.n_energies, device=self.device, dtype=torch.float64)
+        job.oversampling, job.det_x, job.det_y = self.os, self.det_x, self.det_y
+        job.means, job.detect_work = self.means.data_ptr(), self.work.data_ptr()
+        job.src_kernel, job.src_half = (src.data_ptr(), (src.numel() - 1) // 2) if src is not None else (None, 0)
+        job.psf_kernel, job.psf_half = (psf.data_ptr(), (psf.numel() - 1) // 2) if psf is not None else (None, 0)
+        job.noise, job.seed, job.sequence = int(self.poisson), self.seed, sequence
+        return src, psf
+
+    def _rt_job(self, scene, energies, first, sequence, group=True):
         job = abi.RtJob()
-        job.nx, job.ny, job.oversampling, job.det_x, job.det_y = self.nx, self.ny, self.os, self.det_x, self.det_y
+        job.nx, job.ny = self.nx, self.ny
         job.first_point, job.n_energies, job.energies_host = int(first), len(energies), energies
+        kernels = self._detector_fields(job, scene, sequence)
         job.i_bs = self.i_bs.data_ptr()
         job.i_bs_dirty = 1 if self._i_bs_dirty else 0
         for k, t in enumerate(self._group_buffers(scene) if group else ()):
             job.i_bs_group[k] = t.data_ptr()
         job.acc_sample, job.acc_ref = self.acc["sample"].data_ptr(), self.acc["reference"].data_ptr()
         job.acc_propag, job.acc_white = self.acc["propag"].data_ptr(), self.acc["white"].data_ptr()
-        job.means, job.detect_work = self.means.data_ptr(), self.work.data_ptr()
-        job.src_kernel, job.src_half = (src.data_ptr(), (src.numel() - 1) // 2) if src is not None else (None, 0)
-        job.psf_kernel, job.psf_half = (psf.data_ptr(), (psf.numel() - 1) // 2) if psf is not None else (None, 0)
-        job.noise, job.seed, job.sequence = int(self.poisson), self.seed, sequence
         job.flag = self.flag.data_ptr()
-        return job, (src, psf)
+        return job, kernels
 
     def _group_buffers(self, scene, owner=None):
         """Extra object-plane buffers so that up to MAX_GROUP energies of a detector bin share one object hop."""
@@ -382,6 +390,12 @@ class ImageFormation:
             setattr(dj, k, scratch[k].data_ptr())
         dj.dark_field = dark_field.data_ptr() if dark_field is not None else None
         return dj, (df_energies, keep)
+
+    @staticmethod
+    def _rt_launches(n_energies, n_bins, first):
+        # per energy: membrane hop, object hop (+ the sample-only hop at position 0); per bin: the detector (+ the white
+        # fill)
+        return n_energies * (3 if first else 2) + n_bins * (2 if first else 1)
 
     @staticmethod
     def _df_launches(n_energies, n_bins, first):
@@ -447,8 +461,7 @@ class ImageFormation:
         else:
             if wd:
                 job.dx_pad, job.dy_pad = self.dx_pad.data_ptr(), self.dy_pad.data_ptr()
-            launches = n_e * (3 if first else 2) + len(closing) * (2 if first else 1)
-            self._run(job, launches, probe)
+            self._run(job, self._rt_launches(n_e, len(closing), first), probe)
         if want_mean and defer:
             # no host synchronisation here: the per-energy sums and the status flag travel with the images
             # (one small device buffer); the caller finishes with finish_deferred() once they are on the host
@@ -554,6 +567,34 @@ class ImageFormation:
                     propag=buffers["extra"][:len(firsts), 0], white=buffers["extra"][:len(firsts), 1], sums=buffers["sums"],
                     firsts=firsts, buffers=buffers)
 
+    def _positions_call(self, scene, plan, offsets, points, n_slots, buffers, sequence_base, want_means, slot_type, **kind):
+        """What compute_rt_positions, compute_df_positions and compute_fresnel_positions set up alike: the energies that
+        close a detector bin, the output buffers, the membrane, a ctypes array of ``slot_type`` with the fields every slot
+        struct has (``kind``: see _slots), the positions, and the launches of one position's membrane (``cut``)."""
+        n_pos = len(offsets)
+        nbins, n_e = len(scene.thresholds), len(scene.spectrum)
+        closing = {b[-1] for b in self.bins(scene)[:nbins]}
+        firsts = [p for p in range(n_pos) if points[p] == 0]
+        if buffers is None:
+            buffers = self._positions_buffers(n_pos, len(firsts), nbins, n_e)
+        membrane, field = self._membrane(plan)
+        raster_bytes = abi.lib.paresis_raster_work_bytes(plan.table.shape[0], plan.layers, self.nx, self.ny)
+        slots = self._slots(n_slots, raster_bytes, **kind)
+        c_slots = (slot_type * n_slots)()
+        for k, (sl, c) in enumerate(zip(c_slots, slots)):
+            sl.acc_sample, sl.acc_ref = c["acc"]["sample"].data_ptr(), c["acc"]["reference"].data_ptr()
+            sl.acc_propag, sl.acc_white = c["acc"]["propag"].data_ptr(), c["acc"]["white"].data_ptr()
+            sl.raster_work, sl.raster_work_bytes = c["work"].data_ptr(), c["work"].numel()
+            sl.stream = c["stream"].cuda_stream
+            if hasattr(sl, "i_bs"):
+                sl.i_bs = c["i_bs"].data_ptr()
+                sl.i_bs_dirty = 1 if (c["dirty"] or (k == 0 and self._i_bs_dirty)) else 0
+            if hasattr(sl, "detect_work"):
+                sl.detect_work = c["detect_work"].data_ptr()
+        c_pos, offs = self._c_positions(buffers, offsets, points, firsts, plan.layers, sequence_base, want_means)
+        return SimpleNamespace(n_e=n_e, closing=closing, firsts=firsts, buffers=buffers, membrane=membrane, field=field,
+                               cut=1 if field is not None else 2, slots=slots, c_slots=c_slots, c_pos=c_pos, offs=offs)
+
     @_on_own_device
     def compute_rt_positions(self, scene, plan, offsets, points, sequence_base=0, n_slots=2, probe_label=None,
                              probe_events=None, want_means=True, buffers=None, per_launch=0):
@@ -573,49 +614,30 @@ class ImageFormation:
         if self.scatters(s):
             raise NotImplementedError("scattering (dark-field) samples run many positions per call through "
                                       "compute_df_positions")
-        n_pos = len(offsets)
-        bins = self.bins(s)
-        nbins, n_e = len(s.thresholds), len(s.spectrum)
-        closing = {b[-1] for b in bins[:nbins]}
-        energies, keep = self._rt_energies(s, list(range(n_e)), closing)
+        call = self._positions_call(s, plan, offsets, points, n_slots, buffers, sequence_base, want_means, abi.RtSlot)
+        energies, keep = self._rt_energies(s, list(range(call.n_e)), call.closing)
         job, keep2 = self._rt_job(s, energies, False, 0)
         job.positions_per_launch = int(per_launch)
-        firsts = [p for p in range(n_pos) if points[p] == 0]
-        if buffers is None:
-            buffers = self._positions_buffers(n_pos, len(firsts), nbins, n_e)
-        membrane, field = self._membrane(plan)
-        raster_bytes = abi.lib.paresis_raster_work_bytes(plan.table.shape[0], plan.layers, self.nx, self.ny)
-        slots = self._slots(n_slots, raster_bytes)
-        c_slots = (abi.RtSlot * n_slots)()
-        for k, c in enumerate(slots):
-            sl = c_slots[k]
-            sl.i_bs = c["i_bs"].data_ptr()
-            sl.acc_sample, sl.acc_ref = c["acc"]["sample"].data_ptr(), c["acc"]["reference"].data_ptr()
-            sl.acc_propag, sl.acc_white = c["acc"]["propag"].data_ptr(), c["acc"]["white"].data_ptr()
-            sl.raster_work, sl.raster_work_bytes = c["work"].data_ptr(), c["work"].numel()
-            sl.stream = c["stream"].cuda_stream
-            sl.i_bs_dirty = 1 if (c["dirty"] or (k == 0 and self._i_bs_dirty)) else 0
+        for k, (sl, c) in enumerate(zip(call.c_slots, call.slots)):
             for kk, t in enumerate(self._group_buffers(s, owner=None if k == 0 else c)):
                 sl.i_bs_group[kk] = t.data_ptr()
             c["dirty"] = True
         self._i_bs_dirty = True
-        c_pos, offs = self._c_positions(buffers, offsets, points, firsts, plan.layers, sequence_base, want_means)
         launches = 0
-        for p in range(n_pos):
-            cp = c_pos[p]
-            first = points[p] == 0
+        for p in range(len(offsets)):
             if probe_events is not None and probe_events[p] is not None:
                 e0, e1 = probe_events[p]
                 for e in (e0, e1):
                     if not e.cuda_event:
                         e.record()
-                cp.probe_start, cp.probe_end = e0.cuda_event, e1.cuda_event
-            launches += (1 if field is not None else 2) + n_e * (3 if first else 2) + len(closing) * (2 if first else 1)
-        abi.rt_run_positions(job, membrane, c_pos, c_slots, launches, probe_label if probe_events is not None else None)
-        for c in slots:
+                call.c_pos[p].probe_start, call.c_pos[p].probe_end = e0.cuda_event, e1.cuda_event
+            launches += call.cut + self._rt_launches(call.n_e, len(call.closing), points[p] == 0)
+        abi.rt_run_positions(job, call.membrane, call.c_pos, call.c_slots, launches,
+                             probe_label if probe_events is not None else None)
+        for c in call.slots:
             c["dirty"] = False
         self._i_bs_dirty = False
-        return self._positions_result(buffers, firsts)
+        return self._positions_result(call.buffers, call.firsts)
 
     @_on_own_device
     def compute_df_positions(self, scene, plan, offsets, points, sequence_base=0, n_slots=2, want_means=True, buffers=None):
@@ -631,45 +653,28 @@ class ImageFormation:
         if not self.scatters(s):
             raise NotImplementedError("no material of the sample scatters: compute_rt_positions runs such a scene")
         n_pos = len(offsets)
-        bins = self.bins(s)
-        nbins, n_e = len(s.thresholds), len(s.spectrum)
-        closing = {b[-1] for b in bins[:nbins]}
-        energies, keep = self._rt_energies(s, list(range(n_e)), closing)
+        call = self._positions_call(s, plan, offsets, points, n_slots, buffers, sequence_base, want_means, abi.DfSlot,
+                                    darkfield=True)
+        energies, keep = self._rt_energies(s, list(range(call.n_e)), call.closing)
         job, keep2 = self._rt_job(s, energies, False, 0, group=False)
-        dj, keep3 = self._df_job(s, job, list(range(n_e)))
-        firsts = [p for p in range(n_pos) if points[p] == 0]
-        if buffers is None:
-            buffers = self._positions_buffers(n_pos, len(firsts), nbins, n_e)
+        dj, keep3 = self._df_job(s, job, list(range(call.n_e)))
+        buffers, firsts = call.buffers, call.firsts
         if "dark_field" not in buffers:
             buffers["dark_field"] = torch.empty((max(len(firsts), 1), self.nx, self.ny), device=self.device, dtype=torch.float32)
         buffers["dark_field"].zero_()         # paresis_df_run_positions adds to it
-        membrane, field = self._membrane(plan)
-        raster_bytes = abi.lib.paresis_raster_work_bytes(plan.table.shape[0], plan.layers, self.nx, self.ny)
-        slots = self._slots(n_slots, raster_bytes, darkfield=True)
-        c_slots = (abi.DfSlot * n_slots)()
-        for k, c in enumerate(slots):
-            sl = c_slots[k]
-            sl.i_bs = c["i_bs"].data_ptr()
-            sl.acc_sample, sl.acc_ref = c["acc"]["sample"].data_ptr(), c["acc"]["reference"].data_ptr()
-            sl.acc_propag, sl.acc_white = c["acc"]["propag"].data_ptr(), c["acc"]["white"].data_ptr()
+        for sl, c in zip(call.c_slots, call.slots):
             for name in DF_SCRATCH:
                 setattr(sl, name, c["df"][name].data_ptr())
-            sl.detect_work = c["detect_work"].data_ptr()
-            sl.raster_work, sl.raster_work_bytes = c["work"].data_ptr(), c["work"].numel()
-            sl.stream = c["stream"].cuda_stream
-            sl.i_bs_dirty = 1 if (c["dirty"] or (k == 0 and self._i_bs_dirty)) else 0
             c["dirty"] = True
         self._i_bs_dirty = True
-        rt_pos, offs = self._c_positions(buffers, offsets, points, firsts, plan.layers, sequence_base, want_means)
         c_pos = (abi.DfPosition * n_pos)()
         for p in range(n_pos):
-            c_pos[p].rt = rt_pos[p]
+            c_pos[p].rt = call.c_pos[p]
             if points[p] == 0:
                 c_pos[p].dark_field = buffers["dark_field"][firsts.index(p)].data_ptr()
-        cut = 1 if field is not None else 2
-        launches = sum(cut + self._df_launches(n_e, len(closing), points[p] == 0) for p in range(n_pos))
-        abi.df_run_positions(dj, membrane, c_pos, c_slots, launches)
-        for c in slots:
+        launches = sum(call.cut + self._df_launches(call.n_e, len(call.closing), points[p] == 0) for p in range(n_pos))
+        abi.df_run_positions(dj, call.membrane, c_pos, call.c_slots, launches)
+        for c in call.slots:
             c["dirty"] = False
         self._i_bs_dirty = False
         res = self._positions_result(buffers, firsts)
@@ -693,7 +698,7 @@ class ImageFormation:
         job, keep2 = self._rt_job(scene, energies, first, 0)
         dummy = torch.empty(1, device=self.device, dtype=torch.float32)
         job.out_sample = job.out_ref = job.out_propag = job.out_white = dummy.data_ptr()
-        self._run(job, len(indices) * (3 if first else 2))
+        self._run(job, self._rt_launches(len(indices), 0, first))
         return self.means[:len(indices)] / float(self.nx * self.ny)
 
     # ------------------------------------------------------------------ Fresnel
@@ -772,23 +777,14 @@ class ImageFormation:
         return energies, keep
 
     def _fresnel_job(self, scene, energies, first, sequence):
-        fwhm = scene.effective_source_fwhm()
-        src = self._gauss(fwhm / 2.355) if fwhm != 0 else None
-        psf = self._gauss(scene.psf_sigma) if scene.psf_sigma != 0 else None
-        if len(energies) > self.means.numel():
-            self.means = torch.zeros(len(energies), device=self.device, dtype=torch.float64)
         job = abi.FresnelJob()
         job.plan = self._plan._h
-        job.oversampling, job.det_x, job.det_y = self.os, self.det_x, self.det_y
         job.first_point, job.n_energies, job.energies_host = int(first), len(energies), energies
+        kernels = self._detector_fields(job, scene, sequence)
         job.wave_a, job.wave_b = self._waves[0].data_ptr(), self._waves[1].data_ptr()
         job.acc_sample, job.acc_ref = self.acc["sample"].data_ptr(), self.acc["reference"].data_ptr()
         job.acc_propag, job.acc_white = self.acc["propag"].data_ptr(), self.acc["white"].data_ptr()
-        job.means, job.detect_work = self.means.data_ptr(), self.work.data_ptr()
-        job.src_kernel, job.src_half = (src.data_ptr(), (src.numel() - 1) // 2) if src is not None else (None, 0)
-        job.psf_kernel, job.psf_half = (psf.data_ptr(), (psf.numel() - 1) // 2) if psf is not None else (None, 0)
-        job.noise, job.seed, job.sequence = int(self.poisson), self.seed, sequence
-        return job, (src, psf)
+        return job, kernels
 
     @staticmethod
     def _fresnel_launches(n_energies, n_bins, first):
@@ -828,33 +824,17 @@ class ImageFormation:
         [P0, nbins, dx, dy] for the positions with ``points[p] == 0`` (in order), sums [P, n_energies] (float64 sums of
         the reference beam, see paresis_fresnel_job.means), firsts, buffers."""
         s = scene
-        n_pos = len(offsets)
-        bins = self.bins(s)
-        nbins, n_e = len(s.thresholds), len(s.spectrum)
-        closing = {b[-1] for b in bins[:nbins]}
-        energies, keep = self._fresnel_energies(s, list(range(n_e)), closing)
+        call = self._positions_call(s, plan, offsets, points, n_slots, buffers, sequence_base, want_means, abi.FresnelSlot,
+                                    fresnel=True)
+        energies, keep = self._fresnel_energies(s, list(range(call.n_e)), call.closing)
         job, keep2 = self._fresnel_job(s, energies, False, 0)
-        firsts = [p for p in range(n_pos) if points[p] == 0]
-        if buffers is None:
-            buffers = self._positions_buffers(n_pos, len(firsts), nbins, n_e)
-        membrane, field = self._membrane(plan)
-        raster_bytes = abi.lib.paresis_raster_work_bytes(plan.table.shape[0], plan.layers, self.nx, self.ny)
-        slots = self._slots(n_slots, raster_bytes, fresnel=True)
-        c_slots = (abi.FresnelSlot * n_slots)()
-        for k, c in enumerate(slots):
-            sl = c_slots[k]
+        for sl, c in zip(call.c_slots, call.slots):
             sl.plan = c["plan"]._h
             sl.wave_a, sl.wave_b = c["waves"][0].data_ptr(), c["waves"][1].data_ptr()
-            sl.acc_sample, sl.acc_ref = c["acc"]["sample"].data_ptr(), c["acc"]["reference"].data_ptr()
-            sl.acc_propag, sl.acc_white = c["acc"]["propag"].data_ptr(), c["acc"]["white"].data_ptr()
-            sl.detect_work = c["detect_work"].data_ptr()
-            sl.raster_work, sl.raster_work_bytes = c["work"].data_ptr(), c["work"].numel()
-            sl.stream = c["stream"].cuda_stream
-        c_pos, offs = self._c_positions(buffers, offsets, points, firsts, plan.layers, sequence_base, want_means)
-        cut = 1 if field is not None else 2
-        launches = sum(cut + self._fresnel_launches(n_e, len(closing), points[p] == 0) for p in range(n_pos))
-        abi.fresnel_run_positions(job, membrane, c_pos, c_slots, launches)
-        return self._positions_result(buffers, firsts)
+        launches = sum(call.cut + self._fresnel_launches(call.n_e, len(call.closing), points[p] == 0)
+                       for p in range(len(offsets)))
+        abi.fresnel_run_positions(job, call.membrane, call.c_pos, call.c_slots, launches)
+        return self._positions_result(call.buffers, call.firsts)
 
     @_on_own_device
     def accumulate_fresnel(self, scene, point_num, indices):
