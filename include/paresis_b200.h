@@ -238,8 +238,11 @@ typedef struct {
     const float* src_kernel; int src_half;
     const float* psf_kernel; int psf_half;
     int noise; uint64_t seed; uint64_t sequence;   /* Poisson stream: image k of bin b uses sequence + 4b + k */
-    float* out_sample; float* out_ref; float* out_propag; float* out_white;   /* [n_bins][det_x][det_y] */
-    float* dx_pad; float* dy_pad;   /* optional [(nx+30)][(ny+30)]: Dx, Dy of the sample-only beam, last energy (:492) */
+    float* out_sample; float* out_ref; float* out_propag; float* out_white;   /* [n_bins][det_x][det_y].  All NULL: the
+                                  energies are accumulated only and close_bin is ignored (the caller runs the detector,
+                                  as the energy-sharded path does); acc_white is needed with outputs at position 0 only */
+    float* dx_pad; float* dy_pad;   /* optional [(nx+30)][(ny+30)], both or neither: Dx, Dy of the sample-only beam, last
+                                       energy (:492) */
     int* flag;
     /* optional timing probe: cudaEvent_t pair recorded around one kernel of the first energy / bin
      * (1 = membrane hop, 2 = sample+reference hop, 3 = detector launch of the first bin); 0 = off */
@@ -247,7 +250,8 @@ typedef struct {
     int i_bs_dirty;            /* i_bs (and i_bs_group) hold garbage: zero them first (extra memsets) */
     float* i_bs_group[PARESIS_MAX_GROUP - 1];   /* optional: further [nx][ny] buffers like i_bs (same all-zero contract).
                                   With k of them, up to k+1 energies of a detector bin share one object hop
-                                  (paresis_refract_group); NULL entries end the list. */
+                                  (paresis_refract_group); the first NULL entry ends the list, and no entry may
+                                  follow it. */
     int positions_per_launch;  /* paresis_rt_run_positions only: > 1 = membrane cut, hops and detector of up to this many
                                   positions (<= n_slots, <= PARESIS_MAX_HOP_BATCH) share ONE launch each (blockIdx.z =
                                   position) on the caller's stream, instead of one launch per position on per-slot
@@ -258,6 +262,10 @@ typedef struct {
                                   what the caller put here. */
 } paresis_rt_job;
 
+/* Per energy: the membrane hop into i_bs, the object hop into acc_sample / acc_ref (+ means[e]), at position 0 the
+ * sample-only hop into acc_propag; at a bin close the detector on 2 or 4 images.  Accumulators start from zero and are
+ * zeroed again after each detector run.  Each hop takes 1 .. PARESIS_MAX_LAYERS maps, none of them NULL.  Every argument
+ * is checked before the first CUDA call (PARESIS_ERR_ARG). */
 int paresis_rt_run(const paresis_rt_job* job_host, paresis_stream stream);
 
 /* Many membrane positions in ONE call: for each position, rasterise its membrane
@@ -266,9 +274,11 @@ int paresis_rt_run(const paresis_rt_job* job_host, paresis_stream stream);
  * overlap on the GPU (positions are independent: main.py:63-110).  `stream` is the caller's
  * stream: every slot stream first waits for it, and it waits for every slot stream at the end.
  *
- * `job_host` is the template of paresis_rt_run: its scratch / output / sequence / first_point /
- * probe fields are ignored (they come from the slot and the position); a hop layer whose
- * `thickness` is NULL stands for "the membrane map of this position". */
+ * `job_host` is the template of paresis_rt_run: its scratch / detect_work / output / means / sequence / first_point /
+ * probe event fields are ignored (they come from the slot and the position; with positions_per_launch the template's
+ * detect_work serves every position).  A hop1 or hop2 layer whose `thickness` is NULL stands for "the membrane map of
+ * this position"; a NULL propag map is an error.  Every argument is checked before the first CUDA call
+ * (PARESIS_ERR_ARG), including that no image buffer belongs to two slots; n_positions == 0 does nothing. */
 typedef struct {
     const int64_t* offsets_host;   /* [n_layers][2]: the np.random.randint draws of this position (x, y) */
     float* thickness;              /* [nx][ny] out: membrane grain map, metres */
@@ -282,10 +292,13 @@ typedef struct {
 
 typedef struct {
     float* i_bs; float* acc_sample; float* acc_ref; float* acc_propag; float* acc_white;   /* as in paresis_rt_job */
-    void* raster_work; size_t raster_work_bytes;
+    void* raster_work; size_t raster_work_bytes;   /* needed only when the membrane has no sphere field: at least
+                                                      paresis_raster_work_bytes(n_spheres, n_layers, nx, ny) */
     paresis_stream stream;
     int i_bs_dirty;                /* in/out: cleared once the slot has run a position */
     float* i_bs_group[PARESIS_MAX_GROUP - 1];   /* as in paresis_rt_job */
+    float* detect_work;            /* as paresis_rt_job.detect_work, this slot's own (slots run concurrently); may be NULL
+                                      for ordinary kernel sizes */
 } paresis_rt_slot;
 
 typedef struct {
@@ -569,10 +582,8 @@ typedef struct {
 } paresis_df_energy;
 
 typedef struct {
-    paresis_rt_job rt;         /* as for paresis_rt_run, with these differences: i_bs_group, positions_per_launch, dx_pad,
-                                  dy_pad and probe are ignored; out_* may all be NULL, then the energies are accumulated
-                                  only and close_bin is ignored (the energy-sharded path runs the detector itself);
-                                  acc_white is needed with outputs at position 0 only.  i_bs keeps paresis_rt_run's
+    paresis_rt_job rt;         /* as for paresis_rt_run (out_* all NULL: accumulate only), except that i_bs_group,
+                                  positions_per_launch, dx_pad, dy_pad and probe are ignored.  i_bs keeps paresis_rt_run's
                                   contract: all zero on entry unless i_bs_dirty is set, all zero on exit.  The object
                                   hops of each energy must fit in PARESIS_MAX_LAYERS maps (mix the sample's maps
                                   otherwise). */

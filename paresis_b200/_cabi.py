@@ -95,7 +95,7 @@ class RtSlot(ctypes.Structure):
     _fields_ = [("i_bs", ctypes.c_void_p), ("acc_sample", ctypes.c_void_p), ("acc_ref", ctypes.c_void_p),
                 ("acc_propag", ctypes.c_void_p), ("acc_white", ctypes.c_void_p), ("raster_work", ctypes.c_void_p),
                 ("raster_work_bytes", ctypes.c_size_t), ("stream", ctypes.c_void_p), ("i_bs_dirty", ctypes.c_int),
-                ("i_bs_group", ctypes.c_void_p * (MAX_GROUP - 1))]
+                ("i_bs_group", ctypes.c_void_p * (MAX_GROUP - 1)), ("detect_work", ctypes.c_void_p)]
 
 
 class DfSlot(ctypes.Structure):

@@ -15,6 +15,7 @@
 // on their own stream, so that consecutive positions overlap on the GPU.
 #include <cuda_runtime.h>
 
+#include <array>
 #include <vector>
 
 #include "common.cuh"
@@ -26,30 +27,13 @@ namespace {
 
 constexpr int kMargin = 15;   // refractionFileNumba2.py:50
 
-int bad(const char* who, const char* what, int e) {
-    set_last_error("%s: energy %d: %s", who, e, what);
-    return PARESIS_ERR_ARG;
-}
-
-// The per-energy checks of a job (host memory only).  `first`: the sample-only hop runs too (position 0).
-// `position_maps`: a NULL map of the membrane or object hop stands for the membrane of the position at hand
-// (paresis_df_run_positions); a NULL sample-only or scattering map is always an error.
-int check_energies(const char* who, const paresis_df_job* job, bool first, bool position_maps) {
-    const paresis_rt_job& r = job->rt;
-    for (int e = 0; e < r.n_energies; ++e) {
-        const paresis_rt_energy& en = r.energies_host[e];
-        const paresis_df_energy& df = job->energies_df_host[e];
-        if (en.n_hop1 < 1 || en.n_hop1 > PARESIS_MAX_LAYERS) return bad(who, "need 1 .. PARESIS_MAX_LAYERS membrane maps", e);
-        if (en.n_hop2 < 1 || en.n_hop2 > PARESIS_MAX_LAYERS)
-            return bad(who, "need 1 .. PARESIS_MAX_LAYERS membrane + sample maps in the object hop (mix the sample's maps)", e);
-        if (first && (en.n_propag < 1 || en.n_propag > PARESIS_MAX_LAYERS))
-            return bad(who, "need 1 .. PARESIS_MAX_LAYERS sample maps in the sample-only hop", e);
-        for (int m = 0; m < en.n_hop1; ++m) if (!en.hop1[m].thickness && !position_maps) return bad(who, "null membrane map", e);
-        for (int m = 0; m < en.n_hop2; ++m) if (!en.hop2[m].thickness && !position_maps) return bad(who, "null object-hop map", e);
-        if (first)
-            for (int m = 0; m < en.n_propag; ++m) if (!en.propag[m].thickness) return bad(who, "null sample map", e);
-        if (!df.scatter_map) return bad(who, "no scattering map", e);
-    }
+// every energy has a scattering map (host memory only)
+int check_scatter_maps(const char* who, const paresis_df_job* job) {
+    for (int e = 0; e < job->rt.n_energies; ++e)
+        if (!job->energies_df_host[e].scatter_map) {
+            set_last_error("%s: energy %d: no scattering map", who, e);
+            return PARESIS_ERR_ARG;
+        }
     return PARESIS_OK;
 }
 
@@ -57,34 +41,19 @@ int check_energies(const char* who, const paresis_df_job* job, bool first, bool 
 int check_job(const paresis_df_job* job) {
     const char* who = "paresis_df_run";
     if (!job) { set_last_error("%s: null job", who); return PARESIS_ERR_ARG; }
+    if (!job->energies_df_host) { set_last_error("%s: no energies", who); return PARESIS_ERR_ARG; }
     const paresis_rt_job& r = job->rt;
-    if (!r.energies_host || !job->energies_df_host || r.n_energies < 1) {
-        set_last_error("%s: no energies", who);
-        return PARESIS_ERR_ARG;
-    }
-    if (r.nx < 3 || r.ny < 3) { set_last_error("%s: bad frame %d x %d", who, r.nx, r.ny); return PARESIS_ERR_ARG; }
-    if (!r.i_bs || !r.acc_sample || !r.acc_ref || (r.first_point && !r.acc_propag)) {
-        set_last_error("%s: null object-plane buffer or accumulator", who);
-        return PARESIS_ERR_ARG;
-    }
+    int rc = check_rt_job(who, r);
+    if (rc) return rc;
     if (!job->angle || !job->plain || !job->scattered || !job->clean || !job->moved) {
         set_last_error("%s: null dark-field scratch buffer", who);
-        return PARESIS_ERR_ARG;
-    }
-    const bool detect = r.out_sample || r.out_ref || r.out_propag || r.out_white;
-    if (detect && (!r.out_sample || !r.out_ref || (r.first_point && (!r.out_propag || !r.out_white || !r.acc_white)))) {
-        set_last_error("%s: incomplete detector outputs (all of them, or none to accumulate only)", who);
-        return PARESIS_ERR_ARG;
-    }
-    if (detect && (r.oversampling < 1 || r.det_x < 1 || r.det_y < 1)) {
-        set_last_error("%s: bad detector geometry", who);
         return PARESIS_ERR_ARG;
     }
     if (job->dark_field && !r.first_point) {
         set_last_error("%s: the dark-field map belongs to position 0 (first_point)", who);
         return PARESIS_ERR_ARG;
     }
-    return check_energies(who, job, r.first_point != 0, false);
+    return check_scatter_maps(who, job);
 }
 
 // the launch sequence of a checked job
@@ -186,14 +155,6 @@ int bad_positions(const char* fmt, int i) {
     return PARESIS_ERR_ARG;
 }
 
-constexpr int kSlotImages = 11;   // i_bs, four accumulators, five dark-field scratch images, detector work
-
-void slot_images(const paresis_df_slot& sl, const void* out[kSlotImages]) {
-    const void* v[kSlotImages] = {sl.i_bs, sl.acc_sample, sl.acc_ref, sl.acc_propag, sl.acc_white, sl.angle, sl.plain,
-                                  sl.scattered, sl.clean, sl.moved, sl.detect_work};
-    for (int i = 0; i < kSlotImages; ++i) out[i] = v[i];
-}
-
 // every argument of paresis_df_run_positions, host memory only
 int check_positions(const paresis_df_job* job, const paresis_membrane* mem, const paresis_df_position* positions,
                     int n_positions, const paresis_df_slot* slots, int n_slots) {
@@ -201,14 +162,17 @@ int check_positions(const paresis_df_job* job, const paresis_membrane* mem, cons
     int rc = check_call(who, job, mem, positions, slots, n_positions, n_slots);
     if (rc || n_positions == 0) return rc;       // nothing to run, nothing else to check
     const paresis_rt_job& r = job->rt;
-    if (!r.energies_host || !job->energies_df_host || r.n_energies < 1) { set_last_error("%s: no energies", who); return PARESIS_ERR_ARG; }
-    if (r.nx < 3 || r.ny < 3) { set_last_error("%s: bad frame %d x %d", who, r.nx, r.ny); return PARESIS_ERR_ARG; }
+    if (!job->energies_df_host) { set_last_error("%s: no energies", who); return PARESIS_ERR_ARG; }
+    rc = check_rt_frame(who, r);
+    if (rc) return rc;
     rc = check_membrane_detector(who, mem, r.oversampling, r.det_x, r.det_y);
     if (rc) return rc;
     bool any_first = false;
     for (int p = 0; p < n_positions; ++p) {
         const paresis_rt_position& pos = positions[p].rt;
         rc = check_position(who, pos, p);
+        if (rc) return rc;
+        rc = check_no_probe(who, pos, p);
         if (rc) return rc;
         if (positions[p].dark_field && !pos.first_point)
             return bad_positions("paresis_df_run_positions: position %d: the dark-field map belongs to position 0 (first_point)", p);
@@ -221,21 +185,14 @@ int check_positions(const paresis_df_job* job, const paresis_membrane* mem, cons
         if (!sl.angle || !sl.plain || !sl.scattered || !sl.clean || !sl.moved)
             return bad_positions("paresis_df_run_positions: slot %d lacks a dark-field scratch image", k);
     }
-    // slots run concurrently: an image two of them write would be a race
-    for (int k = 1; k < n_slots; ++k) {
-        const void* mine[kSlotImages];
-        slot_images(slots[k], mine);
-        for (int j = 0; j < k; ++j) {
-            const void* theirs[kSlotImages];
-            slot_images(slots[j], theirs);
-            for (int a = 0; a < kSlotImages; ++a)
-                for (int b = 0; b < kSlotImages; ++b)
-                    if (mine[a] && mine[a] == theirs[b])
-                        return bad_positions("paresis_df_run_positions: slot %d shares an image buffer with another slot (slots "
-                                             "run concurrently)", k);
-        }
-    }
-    rc = check_energies(who, job, any_first, true);
+    rc = check_slots_apart(who, slots, n_slots, [](const paresis_df_slot& sl) {
+        return std::array<const void*, 11>{sl.i_bs, sl.acc_sample, sl.acc_ref, sl.acc_propag, sl.acc_white, sl.angle,
+                                           sl.plain, sl.scattered, sl.clean, sl.moved, sl.detect_work};
+    });
+    if (rc) return rc;
+    rc = check_rt_energies(who, r, any_first, true);
+    if (rc) return rc;
+    rc = check_scatter_maps(who, job);
     if (rc) return rc;
     return check_raster_work(who, mem, r.nx, r.ny, slots, n_slots);
 }

@@ -180,6 +180,8 @@ int check_positions(const paresis_fresnel_job* job, const paresis_membrane* mem,
     for (int p = 0; p < n_positions; ++p) {
         rc = check_position(who, positions[p], p);
         if (rc) return rc;
+        rc = check_no_probe(who, positions[p], p);
+        if (rc) return rc;
     }
     for (int k = 0; k < n_slots; ++k) {
         const paresis_fresnel_slot& sl = slots[k];

@@ -10,6 +10,7 @@
 // reference hop, detector = 5 kernels and one 16 KB memset.  There are no zero-fill or reduction
 // passes: each hop zero-fills what the next one scatters into, the object hop clears I_bs behind
 // itself and sums the reference beam while it deposits it (paresis_refract_extras).
+#include <array>
 #include <vector>
 
 #include "common.cuh"
@@ -17,16 +18,38 @@
 
 using namespace paresis;
 
-extern "C" int paresis_rt_run(const paresis_rt_job* job, paresis_stream stream) {
-    if (!job || !job->energies_host || job->n_energies < 1 || !job->i_bs || !job->acc_sample || !job->acc_ref ||
-        !job->out_sample || !job->out_ref ||
-        (job->first_point && (!job->acc_propag || !job->acc_white || !job->out_propag || !job->out_white))) {
-        set_last_error("paresis_rt_run: incomplete job description");
+namespace {
+
+// i_bs_group is a list that ends at its first NULL entry: no entry may follow a NULL one
+bool group_list_ok(float* const* group) {
+    for (int k = 1; k < PARESIS_MAX_GROUP - 1; ++k)
+        if (group[k] && !group[k - 1]) return false;
+    return true;
+}
+
+// every check that reads host memory only: nothing is launched before the whole job is known to be well formed
+int check_job(const paresis_rt_job* job) {
+    const char* who = "paresis_rt_run";
+    if (!job) { set_last_error("%s: null job", who); return PARESIS_ERR_ARG; }
+    const int rc = check_rt_job(who, *job);
+    if (rc) return rc;
+    if ((job->dx_pad == nullptr) != (job->dy_pad == nullptr)) {
+        set_last_error("%s: dx_pad and dy_pad come together", who);
         return PARESIS_ERR_ARG;
     }
+    if (!group_list_ok(job->i_bs_group)) {
+        set_last_error("%s: an i_bs_group entry follows a NULL one (the list ends at its first NULL)", who);
+        return PARESIS_ERR_ARG;
+    }
+    return PARESIS_OK;
+}
+
+// the launch sequence of a checked job
+int run_job(const paresis_rt_job* job, paresis_stream stream) {
     cudaStream_t s = (cudaStream_t)stream;
     const size_t n = (size_t)job->nx * job->ny;
     const int margin = 15;   // refractionFileNumba2.py:50
+    const bool detect = job->out_sample != nullptr;
     // object-plane intensity buffers: one per energy of a group (all zero between jobs)
     float* ibs[PARESIS_MAX_GROUP] = {job->i_bs};
     int n_ibs = 1;
@@ -86,14 +109,10 @@ extern "C" int paresis_rt_run(const paresis_rt_job* job, paresis_stream stream) 
     };
     for (int e = 0; e < job->n_energies;) {
         const paresis_rt_energy& en = job->energies_host[e];
-        if (en.n_hop1 < 1 || en.n_hop2 < 1 || (job->first_point && en.n_propag < 1)) {
-            set_last_error("paresis_rt_run: energy %d has an empty hop", e);
-            return PARESIS_ERR_ARG;
-        }
         // energies of the same detector bin that share their maps go through the object hop together
         int group = 1;
         while (group < n_ibs && e + group < job->n_energies && !job->energies_host[e + group - 1].close_bin &&
-               job->energies_host[e + group].n_hop1 >= 1 && same_maps(en, job->energies_host[e + group]))
+               same_maps(en, job->energies_host[e + group]))
             ++group;
         int rc;
         if (group == 1) {
@@ -134,7 +153,7 @@ extern "C" int paresis_rt_run(const paresis_rt_job* job, paresis_stream stream) 
                 if (rc) return rc;
             }
         }
-        if (job->energies_host[e + group - 1].close_bin) {   // :501-521
+        if (detect && job->energies_host[e + group - 1].close_bin) {   // :501-521
             const bool probed = ibin == 0 && job->probe == 3 && job->probe_start && job->probe_end;
             rc = close_bin(*job, job->nx, job->ny, ibin, white, stream, probed ? job->probe_start : nullptr,
                            probed ? job->probe_end : nullptr);
@@ -145,6 +164,14 @@ extern "C" int paresis_rt_run(const paresis_rt_job* job, paresis_stream stream) 
         e += group;
     }
     return PARESIS_OK;
+}
+
+}  // namespace
+
+extern "C" int paresis_rt_run(const paresis_rt_job* job, paresis_stream stream) {
+    const int rc = check_job(job);
+    if (rc) return rc;
+    return run_job(job, stream);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -176,10 +203,6 @@ static int run_positions_batched(const paresis_rt_job* job, const paresis_membra
         void *ev0 = nullptr, *ev1 = nullptr;              // probe events of the first probed position of the group
         for (int z = 0; z < g; ++z) {
             pos[z] = &positions[idx[z]];
-            if (!pos[z]->offsets_host || !pos[z]->thickness) {
-                set_last_error("paresis_rt_run_positions: position %d lacks offsets or a thickness buffer", idx[z]);
-                return PARESIS_ERR_ARG;
-            }
             offs[z] = pos[z]->offsets_host; thick[z] = pos[z]->thickness;
             if (!ev0 && pos[z]->probe_start && pos[z]->probe_end) { ev0 = pos[z]->probe_start; ev1 = pos[z]->probe_end; }
         }
@@ -194,7 +217,6 @@ static int run_positions_batched(const paresis_rt_job* job, const paresis_membra
         int ibin = 0;
         for (int e = 0; e < job->n_energies; ++e) {
             const paresis_rt_energy& en = job->energies_host[e];
-            if (en.n_hop1 < 1 || en.n_hop2 < 1) { set_last_error("paresis_rt_run_positions: energy %d has an empty hop", e); return PARESIS_ERR_ARG; }
             paresis_tile_hop_item h1[PARESIS_MAX_HOP_BATCH] = {}, h2[PARESIS_MAX_HOP_BATCH] = {};
             for (int z = 0; z < g; ++z) {
                 const paresis_rt_slot& sl = slots[z];
@@ -250,10 +272,6 @@ static int run_positions_batched(const paresis_rt_job* job, const paresis_membra
         }
         // position 0: on its own, through the per-position pipeline, after what is pending (it shares slot 0)
         if (g) { int rc = run_group(group, g); if (rc) return rc; g = 0; }
-        if (!pos.offsets_host || !pos.thickness) {
-            set_last_error("paresis_rt_run_positions: position %d lacks offsets or a thickness buffer", p);
-            return PARESIS_ERR_ARG;
-        }
         int rc = paresis_membrane_from_field(mem->field, mem->field_x, mem->field_y, pos.offsets_host, mem->n_layers, mem->margin,
                                              job->nx, job->ny, pos.thickness, stream);
         if (rc) return rc;
@@ -269,20 +287,59 @@ static int run_positions_batched(const paresis_rt_job* job, const paresis_membra
         j.sequence = pos.sequence;
         j.probe = 0;
         j.dx_pad = j.dy_pad = nullptr;
-        rc = paresis_rt_run(&j, stream);
+        rc = run_job(&j, stream);
         if (rc) return rc;
     }
     if (g) { int rc = run_group(group, g); if (rc) return rc; }
     return PARESIS_OK;
 }
 
+// every argument of paresis_rt_run_positions, host memory only
+static int check_positions(const paresis_rt_job* job, const paresis_membrane* mem, const paresis_rt_position* positions,
+                           int n_positions, const paresis_rt_slot* slots, int n_slots) {
+    const char* who = "paresis_rt_run_positions";
+    int rc = check_call(who, job, mem, positions, slots, n_positions, n_slots);
+    if (rc || n_positions == 0) return rc;       // nothing to run, nothing else to check
+    rc = check_rt_frame(who, *job);
+    if (rc) return rc;
+    rc = check_membrane_detector(who, mem, job->oversampling, job->det_x, job->det_y);
+    if (rc) return rc;
+    bool any_first = false;
+    for (int p = 0; p < n_positions; ++p) {
+        rc = check_position(who, positions[p], p);
+        if (rc) return rc;
+        any_first |= positions[p].first_point != 0;
+    }
+    for (int k = 0; k < n_slots; ++k) {
+        const paresis_rt_slot& sl = slots[k];
+        if (!sl.i_bs || !sl.acc_sample || !sl.acc_ref || !sl.acc_propag || !sl.acc_white) {
+            set_last_error("%s: slot %d lacks an object-plane buffer or an accumulator", who, k);
+            return PARESIS_ERR_ARG;
+        }
+        if (!group_list_ok(sl.i_bs_group)) {
+            set_last_error("%s: slot %d: an i_bs_group entry follows a NULL one (the list ends at its first NULL)", who, k);
+            return PARESIS_ERR_ARG;
+        }
+    }
+    rc = check_slots_apart(who, slots, n_slots, [](const paresis_rt_slot& sl) {
+        std::array<const void*, 6 + PARESIS_MAX_GROUP - 1> images{sl.i_bs, sl.acc_sample, sl.acc_ref, sl.acc_propag,
+                                                                  sl.acc_white, sl.detect_work};
+        for (int k = 0; k < PARESIS_MAX_GROUP - 1; ++k) images[6 + k] = sl.i_bs_group[k];
+        return images;
+    });
+    if (rc) return rc;
+    rc = check_rt_energies(who, *job, any_first, true);
+    if (rc) return rc;
+    return check_raster_work(who, mem, job->nx, job->ny, slots, n_slots);
+}
+
+// Each position: its membrane map (cut from the sphere field, or rasterised), then the launch sequence of paresis_rt_run
+// on its slot's stream with the slot's buffers -- or, with positions_per_launch, several positions per launch.
 extern "C" int paresis_rt_run_positions(const paresis_rt_job* job, const paresis_membrane* mem,
                                         const paresis_rt_position* positions, int n_positions,
                                         paresis_rt_slot* slots, int n_slots, paresis_stream stream) {
-    if (!job || !mem || !positions || !slots || n_positions < 0 || n_slots < 1 || !job->energies_host || job->n_energies < 1) {
-        set_last_error("paresis_rt_run_positions: bad arguments");
-        return PARESIS_ERR_ARG;
-    }
+    const int rc = check_positions(job, mem, positions, n_positions, slots, n_slots);
+    if (rc) return rc;
     if (n_positions == 0) return PARESIS_OK;
     if (job->positions_per_launch > 1 && mem->field && !job->i_bs_group[0] && single_energy_bins(job))
         return run_positions_batched(job, mem, positions, n_positions, slots, n_slots, stream);
@@ -292,10 +349,6 @@ extern "C" int paresis_rt_run_positions(const paresis_rt_job* job, const paresis
     auto probed = [&](int p) { return job->probe != 0 && positions[p].probe_start && positions[p].probe_end && n_slots > 1; };
     auto run = [&](int p, paresis_rt_slot& slot) -> int {
         const paresis_rt_position& pos = positions[p];
-        if (!pos.offsets_host || !pos.thickness) {
-            set_last_error("paresis_rt_run_positions: position %d lacks offsets or a thickness buffer", p);
-            return PARESIS_ERR_ARG;
-        }
         const bool probe_raster = job->probe == 4 && pos.probe_start && pos.probe_end;
         if (probe_raster) cudaEventRecord((cudaEvent_t)pos.probe_start, (cudaStream_t)slot.stream);
         int rc = membrane_of_position(mem, pos.offsets_host, job->nx, job->ny, pos.thickness, slot.raster_work,
@@ -310,11 +363,12 @@ extern "C" int paresis_rt_run_positions(const paresis_rt_job* job, const paresis
         for (int k = 0; k < PARESIS_MAX_GROUP - 1; ++k) j.i_bs_group[k] = slot.i_bs_group[k];
         j.acc_propag = slot.acc_propag; j.acc_white = slot.acc_white;
         j.i_bs_dirty = slot.i_bs_dirty;
+        j.detect_work = slot.detect_work;
         j.probe_start = pos.probe_start; j.probe_end = pos.probe_end;
         if (!pos.probe_start || !pos.probe_end) j.probe = 0;
         j.dx_pad = j.dy_pad = nullptr;
         if (n_positions > 1) j.throughput = 1;        // launches of neighbouring positions overlap: least work per pixel wins
-        rc = paresis_rt_run(&j, slot.stream);
+        rc = run_job(&j, slot.stream);
         if (rc) return rc;
         slot.i_bs_dirty = 0;
         return PARESIS_OK;

@@ -1,6 +1,6 @@
 // What the run entries (paresis_rt_run, paresis_fresnel_run, paresis_df_run and their _positions forms) share: the
 // detector-bin close of one position, the slot driver of the many-positions entries with the membrane map and the layer
-// maps of one position, and the argument checks of the Fresnel and dark-field many-positions entries.
+// maps of one position, the checks of a ray-tracing job, and the argument checks of the many-positions entries.
 #pragma once
 #include <vector>
 
@@ -102,19 +102,46 @@ void bind_position(Job& j, const paresis_rt_position& pos) {
     j.sequence = pos.sequence;
 }
 
-// out[e] = energies[e] for e < n_energies, except that a NULL hop1 / hop2 / propag map stands for `thickness`, the
-// membrane map of the position at hand.  Only the layers below n_hop1 / n_hop2 / n_propag are read or written.
+// out[e] = energies[e] for e < n_energies, except that a NULL hop1 / hop2 map stands for `thickness`, the membrane map
+// of the position at hand.  Only the layers below n_hop1 / n_hop2 are read or written.
 void bind_position_maps(const paresis_rt_energy* energies, int n_energies, const float* thickness, paresis_rt_energy* out);
 
-// The argument checks of paresis_fresnel_run_positions and paresis_df_run_positions that do not depend on the model
-// (host memory only); `who` prefixes the message.
-// The pointers and counts of the call:
+// The argument checks of the run entries (host memory only); `who` prefixes the message.
+// A ray-tracing job (paresis_rt_run, paresis_df_run's job->rt): energies and a frame of at least 3 x 3 ...
+int check_rt_frame(const char* who, const paresis_rt_job& r);
+// ... and everything of a single-position job: the frame, i_bs and the accumulators, the detector outputs (all of them,
+// or none to accumulate only), acc_white and the detector geometry with outputs, and the energies (check_rt_energies):
+int check_rt_job(const char* who, const paresis_rt_job& r);
+// per energy, 1 .. PARESIS_MAX_LAYERS layers in each hop (the sample-only hop when `first`) and no NULL map; with
+// `position_maps`, a NULL hop1 / hop2 map stands for the position's membrane map (a NULL propag map never does):
+int check_rt_energies(const char* who, const paresis_rt_job& r, bool first, bool position_maps);
+// The pointers and counts of a many-positions call:
 int check_call(const char* who, const void* job, const paresis_membrane* mem, const void* positions, const void* slots,
                int n_positions, int n_slots);
 // the membrane has a sphere field or spheres, and the detector geometry:
 int check_membrane_detector(const char* who, const paresis_membrane* mem, int oversampling, int det_x, int det_y);
-// position p has offsets, a thickness buffer and all its detector outputs, and no probe events:
+// position p has offsets, a thickness buffer and all its detector outputs:
 int check_position(const char* who, const paresis_rt_position& pos, int p);
+// position p has no probe events (an entry that records none):
+int check_no_probe(const char* who, const paresis_rt_position& pos, int p);
+// Slots run concurrently, so no image may belong to two of them.  images(slot): a std::array of the slot's image
+// pointers, NULL for none.
+template <class Slot, class Images>
+int check_slots_apart(const char* who, const Slot* slots, int n_slots, Images&& images) {
+    for (int k = 1; k < n_slots; ++k) {
+        const auto mine = images(slots[k]);
+        for (int j = 0; j < k; ++j) {
+            const auto theirs = images(slots[j]);
+            for (const void* a : mine)
+                for (const void* b : theirs)
+                    if (a && a == b) {
+                        set_last_error("%s: slot %d shares an image buffer with another slot (slots run concurrently)", who, k);
+                        return PARESIS_ERR_ARG;
+                    }
+        }
+    }
+    return PARESIS_OK;
+}
 // without a sphere field, every slot has raster work of at least paresis_raster_work_bytes:
 template <class Slot>
 int check_raster_work(const char* who, const paresis_membrane* mem, int nx, int ny, const Slot* slots, int n_slots) {

@@ -495,8 +495,8 @@ class ImageFormation:
     # ------------------------------------------------------------------ many positions, one call
     def _slots(self, n_slots, raster_bytes, fresnel=False, darkfield=False):
         """Scratch sets of paresis_rt_run_positions / paresis_fresnel_run_positions / paresis_df_run_positions: slot 0 is
-        this engine's own buffers.  ``fresnel``: each slot also gets a Fresnel plan, two waves and detector work of its own
-        (slots run concurrently); ``darkfield``: the five scratch images of paresis_df_run and detector work of its own."""
+        this engine's own buffers.  Each slot has detector work of its own (slots run concurrently).  ``fresnel``: each
+        slot also gets a Fresnel plan and two waves of its own; ``darkfield``: the five scratch images of paresis_df_run."""
         f32 = dict(device=self.device, dtype=torch.float32)
         cache = self.__dict__.setdefault("_slot_cache", [])
         while len(cache) < n_slots:
@@ -504,6 +504,7 @@ class ImageFormation:
             cache.append(dict(
                 i_bs=self.i_bs if k == 0 else torch.zeros((self.nx, self.ny), **f32),
                 acc={name: (self.acc[name] if k == 0 else torch.empty((self.nx, self.ny), **f32)) for name in IMAGES},
+                detect_work=self.work if k == 0 else torch.empty_like(self.work),
                 work=None, stream=torch.cuda.Stream(device=self.device), dirty=False))
         for c in cache[:n_slots]:
             if c["work"] is None or c["work"].numel() < raster_bytes:
@@ -518,10 +519,6 @@ class ImageFormation:
             for k, c in enumerate(cache[:n_slots]):
                 if "df" not in c:
                     c["df"] = self._df_scratch() if k == 0 else self._new_df_scratch()
-        if fresnel or darkfield:
-            for k, c in enumerate(cache[:n_slots]):
-                if "detect_work" not in c:
-                    c["detect_work"] = self.work if k == 0 else torch.empty_like(self.work)
         return cache[:n_slots]
 
     def _positions_buffers(self, n_pos, n_firsts, nbins, n_e):
@@ -586,11 +583,10 @@ class ImageFormation:
             sl.acc_propag, sl.acc_white = c["acc"]["propag"].data_ptr(), c["acc"]["white"].data_ptr()
             sl.raster_work, sl.raster_work_bytes = c["work"].data_ptr(), c["work"].numel()
             sl.stream = c["stream"].cuda_stream
+            sl.detect_work = c["detect_work"].data_ptr()
             if hasattr(sl, "i_bs"):
                 sl.i_bs = c["i_bs"].data_ptr()
                 sl.i_bs_dirty = 1 if (c["dirty"] or (k == 0 and self._i_bs_dirty)) else 0
-            if hasattr(sl, "detect_work"):
-                sl.detect_work = c["detect_work"].data_ptr()
         c_pos, offs = self._c_positions(buffers, offsets, points, firsts, plan.layers, sequence_base, want_means)
         return SimpleNamespace(n_e=n_e, closing=closing, firsts=firsts, buffers=buffers, membrane=membrane, field=field,
                                cut=1 if field is not None else 2, slots=slots, c_slots=c_slots, c_pos=c_pos, offs=offs)
@@ -689,16 +685,15 @@ class ImageFormation:
         several GPUs (shard.py).  ``dark_field``: [nx, ny] float32 tensor that a scattering sample at
         position 0 adds these energies' share of compute_rt's ``dark_field`` to."""
         first = point_num == 0
+        scatters = self.scatters(scene)
         energies, keep = self._rt_energies(scene, list(indices), closing=set())
-        if self.scatters(scene):
-            job, keep2 = self._rt_job(scene, energies, first, 0, group=False)
+        # no detector outputs: the library accumulates only
+        job, keep2 = self._rt_job(scene, energies, first, 0, group=not scatters)
+        if scatters:
             dj, keep3 = self._df_job(scene, job, list(indices), dark_field if first else None)
             self._run_df(dj, self._df_launches(len(indices), 0, first))
-            return self.means[:len(indices)] / float(self.nx * self.ny)
-        job, keep2 = self._rt_job(scene, energies, first, 0)
-        dummy = torch.empty(1, device=self.device, dtype=torch.float32)
-        job.out_sample = job.out_ref = job.out_propag = job.out_white = dummy.data_ptr()
-        self._run(job, self._rt_launches(len(indices), 0, first))
+        else:
+            self._run(job, self._rt_launches(len(indices), 0, first))
         return self.means[:len(indices)] / float(self.nx * self.ny)
 
     # ------------------------------------------------------------------ Fresnel
